@@ -1,6 +1,7 @@
 """bench.py — HGTConv forward edges/s on synthetic heterographs shaped like BASELINE.json's configs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c5|c4]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 --config (default c2 = the configuration BASELINE.json's metric is quoted on):
@@ -179,6 +180,47 @@ def edge_algorithmic_bytes(n_edges, n_dst, d, use_rte=False):
     return n_edges * per_edge + n_dst * (2 * d * 4 + 4)
 
 
+DUMP_MAX_BYTES = 64 * 2 ** 20
+DUMP_SAMPLE_ROWS = 16384
+
+
+def dump_rows(n_rows, row_bytes, budget):
+    """Row ids --dump-outputs writes of an [n_rows, d] output: all of them when they fit `budget` bytes, else a fixed
+    seeded sample of DUMP_SAMPLE_ROWS rows in ascending order (the same rows in every run with the same arguments)."""
+    import torch
+    if n_rows * row_bytes <= budget:
+        return torch.arange(n_rows)
+    pick = torch.randperm(n_rows, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE_ROWS]
+    return pick.sort().values
+
+
+def gather_rows(out, rows, n_rows, row_global, world):
+    """Rows `rows` of an [n_rows, d] output, on the host.  Sharded runs: `out` holds this rank's rows, global ids
+    `row_global`; each sampled row is filled in by its owner and summed over ranks (every other rank adds zeros)."""
+    import torch
+    if world == 1:
+        return out.index_select(0, rows.to(out.device)).cpu()
+    import torch.distributed as dist
+    pos = torch.full((n_rows,), -1, dtype=torch.int64)
+    pos[row_global.cpu()] = torch.arange(row_global.numel())
+    local = pos[rows]
+    mine = local >= 0
+    buf = torch.zeros((rows.numel(), out.shape[1]), dtype=out.dtype, device=out.device)
+    buf[mine.to(out.device)] = out.index_select(0, local[mine].to(out.device))
+    dist.all_reduce(buf)
+    return buf.cpu()
+
+
+def write_outputs(path, arrays):
+    """--dump-outputs: every array as <path>/<name>.npy (float32 values, float64 row ids)."""
+    import numpy as np
+    total = sum(a.numel() * a.element_size() for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, "dump of %d bytes exceeds %d" % (total, DUMP_MAX_BYTES)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.numpy())
+
+
 def _median(v):
     s = sorted(v)
     n = len(s)
@@ -301,7 +343,7 @@ def run_cpu_port(config, steps, warmup, edges_m=64.0):
 def main_reference(args, rank, world):
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     warmup = 1
     cfg = CONFIGS[args.config]
     ups, info, ms, g, scale = run_cpu_port(args.config, steps, warmup, args.edges_m)
@@ -454,6 +496,11 @@ def main_ours(args, rank, local_rank, world):
         if sampler is not None:
             sampler.mark_end()
         launches = _lib.kernel_launches() - launches0
+        if args.dump_outputs:                                         # `out` is the last timed step's result
+            rows = dump_rows(N, D * 4 + 8, DUMP_MAX_BYTES)
+            sample = gather_rows(out, rows, N, None if world == 1 else shard.owned_global, world)
+            if rank == 0:
+                write_outputs(args.dump_outputs, {"out": sample, "out_rows": rows.double()})
         per_step = torch.tensor([evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)], device=dev,
                                 dtype=torch.float64)
         if world > 1:
@@ -599,7 +646,7 @@ def main_ours(args, rank, local_rank, world):
 
         run_pipeline(2)
         barrier()
-        k2 = max(4, args.steps)
+        k2 = args.steps
         a, b_ev = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         trace.clear()
         done.clear()
@@ -616,15 +663,17 @@ def main_ours(args, rank, local_rank, world):
         t2 = torch.tensor([a.elapsed_time(b_ev) / k2], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(t2, op=dist.ReduceOp.MAX)
-            dist.all_reduce(gaps, op=dist.ReduceOp.MAX)
-        e2e_ms = _median(gaps.tolist())
+            if k2 > 1:
+                dist.all_reduce(gaps, op=dist.ReduceOp.MAX)
+        e2e_ms = _median(gaps.tolist()) if k2 > 1 else t2.item()     # one step has no interval: its whole time
         h2d_all = torch.tensor([float(h2d), float(d2h)], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(h2d_all)
         e2e = {"value": E / (e2e_ms * 1e-3), "unit": UNIT, "h2d_bytes_per_step": int(h2d_all[0].item()),
                "d2h_bytes_per_step": int(h2d_all[1].item()), "ms_per_step": e2e_ms,
-               "ms_per_step_stat": "median interval between consecutive results landing in host memory "
-                                   "(%d steps, max over ranks)" % k2,
+               "ms_per_step_stat": ("median interval between consecutive results landing in host memory "
+                                    "(%d steps, max over ranks)" % k2) if k2 > 1 else
+                                   "time of the single step, H2D to D2H (max over ranks)",
                "ms_per_step_mean": t2.item(),
                "stream_busy_ms_per_step_rank0": {k: round(v, 2) for k, v in busy.items()},
                "includes": ("per step%s: H2D of node_inp/node_type/edge_index/edge_type%s from pinned host memory, plan "
@@ -736,13 +785,19 @@ def main_train(args, rank, local_rank, world, dev, sampler, numa, affinity0):
         sampler.mark_begin()
     evs[0].record()
     for i in range(args.steps):
-        step()
-        layers.zero_grad(set_to_none=True)
+        layers.zero_grad(set_to_none=True)           # at the start, so the last step's gradients outlive the loop
+        h = step()
         evs[i + 1].record()
     barrier()
     if sampler is not None:
         sampler.mark_end()
     launches = _lib.kernel_launches() - launches0
+    if args.dump_outputs:                            # the last step's output rows and parameter gradients
+        grads = {"grad." + n: p.grad.cpu() for n, p in layers.named_parameters() if p.grad is not None}
+        rows = dump_rows(N, D * 4 + 8, DUMP_MAX_BYTES - sum(g.numel() * 4 for g in grads.values()))
+        sample = gather_rows(h.detach(), rows, N, None if world == 1 else shard.owned_global, world)
+        if rank == 0:
+            write_outputs(args.dump_outputs, dict(out=sample, out_rows=rows.double(), **grads))
     per_step = torch.tensor([evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(per_step, op=dist.ReduceOp.MAX)
@@ -791,7 +846,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--halo", default=None, choices=["nccl", "p2p", "push"],
                     help="multi-GPU halo exchange: one NCCL all_to_all or the fused peer-memory pull kernel (default auto)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (at most 64 MB: "
+                         "a fixed seeded sample of the output rows, ids in out_rows.npy; c4 adds grad.<param>.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm times a smaller CPU sample")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -126,9 +126,7 @@ def synthetic_sampled_subgraph(seed, n_per_type=(40, 25, 10), n_edges=300):
     """A sampled sub-graph in the format sample_subgraph() returns (data.py:210): feature / times per type and
     edge_list[target_type][source_type][relation] = [[target_ser, source_ser], ...], plus a reference Graph object that
     defines the type order and the meta graph."""
-    import numpy as np
     data = pyg_shim.load_reference_data()
-    rng = np.random.RandomState(seed)
     g = data.Graph()
     names = ["paper", "author", "venue"]
     rels = [("author", "paper", "AP_write"), ("paper", "paper", "PP_cite"), ("paper", "venue", "PV_Journal")]
@@ -136,19 +134,27 @@ def synthetic_sampled_subgraph(seed, n_per_type=(40, 25, 10), n_edges=300):
         g.add_edge({"type": s_t, "id": "s0"}, {"type": t_t, "id": "t0"}, time=2000, relation_type=r)
     for t in names:
         g.node_feature[t] = []                                  # get_types() = list(node_feature.keys())
-    feature = {t: rng.randn(n, 7).astype(np.float32) for t, n in zip(names, n_per_type)}
-    times = {t: rng.randint(1990, 2020, size=n) for t, n in zip(names, n_per_type)}
-    sizes = dict(zip(names, n_per_type))
+    feature, times, edge_list = sampled_subgraph_inputs(seed, g.get_types(), g.get_meta_graph(), n_per_type, n_edges)
+    return data, g, feature, times, edge_list
+
+
+def sampled_subgraph_inputs(seed, types, metas, n_per_type, n_edges):
+    """The seeded part of synthetic_sampled_subgraph: needs only the type order and the meta graph (both stored in
+    tests/golden/to_torch.pt), not the reference."""
+    import numpy as np
     from collections import defaultdict
+    rng = np.random.RandomState(seed)
+    feature = {t: rng.randn(n, 7).astype(np.float32) for t, n in zip(types, n_per_type)}
+    times = {t: rng.randint(1990, 2020, size=n) for t, n in zip(types, n_per_type)}
+    sizes = dict(zip(types, n_per_type))
     edge_list = defaultdict(lambda: defaultdict(lambda: defaultdict(lambda: [])))
-    metas = g.get_meta_graph()
     for _ in range(n_edges):
         t_t, s_t, r = metas[rng.randint(len(metas))]
         edge_list[t_t][s_t][r] += [[int(rng.randint(sizes[t_t])), int(rng.randint(sizes[s_t]))]]
-    for t in names:                                             # 'self' loops as in data.py:183-186
+    for t in types:                                             # 'self' loops as in data.py:183-186
         for i in range(sizes[t]):
             edge_list[t][t]['self'] += [[i, i]]
-    return data, g, feature, times, edge_list
+    return feature, times, edge_list
 
 
 def to_torch_case(name, seed):
@@ -238,6 +244,111 @@ def sampler_case(name, seed):
     print("%-28s %d sampled cases  %.0f KB" % (name, len(cases), os.path.getsize(path) / 1024))
 
 
+def sampler_edge_list(seed, n_paper, n_author, n_venue, n_field, e_ap, e_pp, e_pf):
+    """An OAG-like graph straight in the reference's adjacency layout (data.py:35-38), without the reference:
+    edge_list[target_type][source_type][relation][target_id][source_id] = time, each edge also stored the other way
+    round under 'rev_' + relation.  Node ids are the drawn ids.  Returns (edge_list, paper years)."""
+    import numpy as np
+    rng = np.random.RandomState(seed)
+    years = rng.randint(2000, 2020, size=n_paper)
+    edge_list = {}
+
+    def link(s_t, s, t_t, t, time, r):
+        for a_t, a, b_t, b, rel in ((t_t, t, s_t, s, r), (s_t, s, t_t, t, "rev_" + r)):
+            edge_list.setdefault(a_t, {}).setdefault(b_t, {}).setdefault(rel, {}).setdefault(a, {})[b] = time
+    for i in range(n_paper):
+        link("paper", i, "venue", int(rng.randint(n_venue)), int(years[i]), "PV_Journal")
+    for _ in range(e_ap):
+        p = int(rng.randint(n_paper))
+        link("author", int(rng.randint(n_author)), "paper", p, int(years[p]), "AP_write")
+    for _ in range(e_pp):
+        p, q = int(rng.randint(n_paper)), int(rng.randint(n_paper))
+        link("paper", p, "paper", q, int(years[q]), "PP_cite")
+    for _ in range(e_pf):
+        p = int(rng.randint(n_paper))
+        link("paper", p, "field", int(rng.randint(n_field)), None if rng.rand() < 0.3 else int(years[p]), "PF_in_L2")
+    return edge_list, years
+
+
+# The larger cases of tests/test_data_ingest.py and tests/test_sampler.py.  Their outputs are too large to store, so
+# the record keeps SHA-256 digests of them; the inputs are regenerated from these arguments.
+TO_TORCH_LARGE = dict(seed=5, n_per_type=[3000, 2000, 300], n_edges=60000)
+SAMPLER_LARGE = dict(graph=dict(seed=11, n_paper=6000, n_author=4000, n_venue=20, n_field=200, e_ap=24000,
+                                e_pp=30000, e_pf=18000),
+                     seeds=dict(seed=5, count=128), np_seed=3, depth=5, number=64)
+
+
+def sampler_large_inputs():
+    """(edge_list, time_range, inp) of SAMPLER_LARGE."""
+    import numpy as np
+    edge_list, years = sampler_edge_list(**SAMPLER_LARGE["graph"])
+    time_range = {int(y): True for y in range(2000, 2016)}
+    pids = np.random.RandomState(SAMPLER_LARGE["seeds"]["seed"]).choice(SAMPLER_LARGE["graph"]["n_paper"],
+                                                                       SAMPLER_LARGE["seeds"]["count"], replace=False)
+    inp = {"paper": np.array([[int(p), int(years[p])] for p in pids])}
+    return edge_list, time_range, inp
+
+
+def digest(a):
+    """SHA-256 over an array's dtype, shape and bytes (numpy array or CPU tensor)."""
+    import hashlib
+    import numpy as np
+    a = np.ascontiguousarray(a.numpy() if isinstance(a, torch.Tensor) else a)
+    h = hashlib.sha256(("%s %s " % (a.dtype.str, a.shape)).encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def sampler_digests(edge_list, indxs, rng_state):
+    """What tests/test_sampler.py compares of one sample_subgraph result: the sampled blocks in order, the sampled ids
+    per type and numpy's RNG state afterwards."""
+    import numpy as np
+    blocks = [[t, s, r, digest(np.asarray(edge_list[t][s][r], dtype=np.int64).reshape(-1, 2))]
+              for t in edge_list for s in edge_list[t] for r in edge_list[t][s]]
+    return {"blocks": blocks, "indxs": {k: digest(np.asarray(v, dtype=np.int64)) for k, v in indxs.items()},
+            "rng_after": digest(np.asarray(rng_state, dtype=np.uint32))}
+
+
+def _inventory(module):
+    return [[n, list(p.shape)] for n, p in module.named_parameters()]
+
+
+def reference_record(name):
+    """Facts about the reference that tests check without it: parameter inventories (names and shapes) and digests of
+    the reference's outputs on TO_TORCH_LARGE and SAMPLER_LARGE."""
+    import json
+    import types
+    import warnings
+    import numpy as np
+    conv, model = pyg_shim.load_reference()
+    data = pyg_shim.load_reference_data()
+    rec = {"hgtconv_32_3_4_4_params": _inventory(conv.HGTConv(32, 32, 3, 4, 4, 0.2, True, True)),
+           "mag_gnn_params": _inventory(model.GNN(in_dim=129, n_hid=512, num_types=4, num_relations=9, n_heads=8,
+                                                  n_layers=4, prev_norm=True, last_norm=True, use_RTE=True)),
+           "mag_classifier_params": _inventory(model.Classifier(512, 349))}
+
+    _, g, feature, times, edge_list = synthetic_sampled_subgraph(**TO_TORCH_LARGE)
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        ref = data.to_torch(feature, times, edge_list, g)
+    keys = ("node_feature", "node_type", "edge_time", "edge_index", "edge_type")
+    rec["to_torch_large"] = dict(TO_TORCH_LARGE, **{k: digest(v) for k, v in zip(keys, ref[:5])},
+                                 node_dict={k: [int(x) for x in v] for k, v in ref[5].items()},
+                                 edge_dict={k: int(v) for k, v in ref[6].items()})
+
+    edge_list, time_range, inp = sampler_large_inputs()
+    np.random.seed(SAMPLER_LARGE["np_seed"])
+    _, _, s_edges, s_indxs, _ = data.sample_subgraph(types.SimpleNamespace(edge_list=edge_list), time_range,
+                                                     SAMPLER_LARGE["depth"], SAMPLER_LARGE["number"], inp,
+                                                     sampler_extractor)
+    rec["sampler_large"] = dict(SAMPLER_LARGE, **sampler_digests(s_edges, s_indxs, np.random.get_state()[1]))
+    path = os.path.join(OUT_DIR, name + ".json")
+    with open(path, "w") as f:
+        json.dump(rec, f, indent=1)
+        f.write("\n")
+    print("%-28s %.0f KB" % (name, os.path.getsize(path) / 1024))
+
+
 def main():
     os.makedirs(OUT_DIR, exist_ok=True)
     to_torch_case("to_torch", seed=31)
@@ -271,6 +382,7 @@ def main():
     # DenseHGTConv variant (unsorted types, isolated destinations), d=64 so the FFN runs on the tensor-core GEMM
     g = synth.make_random(300, 2400, 3, 3, seed=27, isolated_frac=0.2, self_loops=30)
     dense_case("dense_hgt", g, 64, 4, True, True, seed=18)
+    reference_record("reference_record")
 
 
 if __name__ == "__main__":

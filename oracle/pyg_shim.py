@@ -1,10 +1,9 @@
 """Stand-ins for the three PyTorch-Geometric primitives pyHGT's conv.py imports,
 plus a loader that imports the UNMODIFIED reference modules from /root/reference.
 
-TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).  Works only in the dev container:
-/root/reference does not exist on the GPU box, so this module is used solely by
-``oracle/make_golden.py`` (fixture generation) and by CPU tests that skip when the
-reference tree is absent.
+TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).  Used solely by ``oracle/make_golden.py``
+to generate the fixtures under tests/golden, which needs a checkout of the reference
+(PYHGT_REFERENCE_ROOT); the tests themselves read only the fixtures.
 
 Third-party arithmetic restated here (not vendored under /root/reference):
 torch-geometric==1.3.2 / torch-scatter==1.3.2 (requirements.txt:5,9).  Call sites in

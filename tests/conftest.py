@@ -20,6 +20,13 @@ def load_golden(name):
     return torch.load(os.path.join(GOLDEN_DIR, name + ".pt"), map_location="cpu", weights_only=False)
 
 
+def load_record():
+    """tests/golden/reference_record.json: parameter inventories of the reference and digests of its larger outputs."""
+    import json
+    with open(os.path.join(GOLDEN_DIR, "reference_record.json")) as f:
+        return json.load(f)
+
+
 @pytest.fixture(params=CONV_FIXTURES)
 def conv_fixture(request):
     fx = load_golden(request.param)

@@ -6,8 +6,7 @@ import pytest
 import torch
 
 import pyhgt_b200
-from oracle import pyg_shim
-from tests.conftest import load_golden
+from tests.conftest import load_golden, load_record
 
 
 def test_param_count_known_answer():
@@ -46,13 +45,10 @@ def test_rte_table_matches_oracle_formula():
     assert m.emb.weight.requires_grad          # the reference leaves the table trainable (SURVEY §8 a8)
 
 
-@pytest.mark.skipif(not pyg_shim.reference_available(), reason="reference tree only exists in the dev container")
 def test_parameter_names_equal_reference_module():
-    conv, _ = pyg_shim.load_reference()
-    ref = conv.HGTConv(32, 32, 3, 4, 4, 0.2, True, True)
+    ref = load_record()["hgtconv_32_3_4_4_params"]          # the reference's HGTConv(32, 32, 3, 4, 4, 0.2, True, True)
     mine = pyhgt_b200.HGTConv(32, 32, 3, 4, 4, 0.2, True, True)
-    assert [(n, tuple(p.shape)) for n, p in ref.named_parameters()] == \
-           [(n, tuple(p.shape)) for n, p in mine.named_parameters()]
+    assert [(n, tuple(s)) for n, s in ref] == [(n, tuple(p.shape)) for n, p in mine.named_parameters()]
 
 
 def test_general_conv_dispatch():
@@ -103,32 +99,3 @@ def test_module_pickles_and_deep_copies_with_launch_caches():
         for (k, a), (k2, b) in zip(m.state_dict().items(), other.state_dict().items()):
             assert k == k2 and torch.equal(a, b)
     assert "_args_cache" in m.__dict__                                            # the live module keeps its caches
-
-
-def test_reference_model_py_runs_on_the_integration_rebind():
-    """INTEGRATION.md §1: rebinding the name `HGTConv` in the reference's pyHGT/conv.py is the whole change — the
-    UNMODIFIED pyHGT/model.py (`from .conv import *`, model.py:1) then builds its GNN out of pyhgt_b200 layers, with
-    the reference's parameter names (reference checkpoints load strict).  Dev container only (needs /root/reference)."""
-    import pytest
-    from oracle import pyg_shim
-    if not pyg_shim.reference_available():
-        pytest.skip("reference tree not present")
-    import pyhgt_b200
-    from pyhgt_b200 import _lib
-    conv, model = pyg_shim.load_reference()
-    original = conv.HGTConv
-    try:
-        conv.HGTConv = pyhgt_b200.HGTConv                      # the rebind of INTEGRATION.md §1
-        fx = load_golden("gnn_2layer")
-        c = fx["cfg"]
-        torch.manual_seed(0)
-        m = model.GNN(c["in_dim"], c["n_hid"], c["num_types"], c["num_relations"], c["n_heads"], c["n_layers"], 0.2,
-                      "hgt", c["prev_norm"], c["last_norm"], c["use_RTE"])
-        assert all(type(gc.base_conv) is pyhgt_b200.HGTConv for gc in m.gcs)
-        assert list(m.state_dict().keys()) == list(fx["state_dict"].keys())
-        m.load_state_dict(fx["state_dict"], strict=True)
-        # GeneralConv.forward (conv.py:317) passes the five tensors positionally; on CPU the CUDA layer refuses loudly
-        with pytest.raises(_lib.HgtError):
-            m(fx["node_feature"], fx["node_type"], fx["edge_time"], fx["edge_index"], fx["edge_type"])
-    finally:
-        conv.HGTConv = original

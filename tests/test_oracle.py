@@ -1,9 +1,12 @@
 """Pin the CPU oracle (oracle/hgt_oracle.py) against outputs of the reference itself:
 tests/golden/*.pt were produced by /root/reference/pyHGT/conv.py (oracle/make_golden.py)."""
+import math
+
 import pytest
 import torch
 
-from oracle import hgt_oracle, pyg_shim
+from oracle import hgt_oracle
+from tests.conftest import load_record
 
 
 def _kw(fx):
@@ -46,30 +49,16 @@ def test_init_params_inventory_matches_reference_count():
     assert sum(v.numel() for v in p.values()) == 5182028
 
 
-@pytest.mark.skipif(not pyg_shim.reference_available(), reason="reference tree only exists in the dev container")
 def test_reference_model_param_count_known_answer():
-    conv, model = pyg_shim.load_reference()
-    g = model.GNN(in_dim=129, n_hid=512, num_types=4, num_relations=9, n_heads=8, n_layers=4,
-                  prev_norm=True, last_norm=True, use_RTE=True)
-    c = model.Classifier(512, 349)
-    assert sum(p.numel() for p in g.parameters()) + sum(p.numel() for p in c.parameters()) == 21173389
-
-
-@pytest.mark.skipif(not pyg_shim.reference_available(), reason="reference tree only exists in the dev container")
-def test_golden_reproducible_from_reference():
-    """The committed c1 fixture is what the reference computes today."""
-    from tests.conftest import load_golden
-    fx = load_golden("c1_rte")
-    conv, _ = pyg_shim.load_reference()
-    c = fx["cfg"]
-    m = conv.HGTConv(c["in_dim"], c["out_dim"], c["num_types"], c["num_relations"], c["n_heads"], 0.2,
-                     c["use_norm"], c["use_RTE"])
-    m.load_state_dict(fx["state_dict"])
-    m.eval()
-    with torch.no_grad():
-        out = m(fx["node_inp"], fx["node_type"], fx["edge_index"], fx["edge_type"], fx["edge_time"])
-    assert torch.allclose(out, fx["out"], rtol=1e-6, atol=1e-6)
-    assert torch.allclose(m.att, fx["att"], rtol=1e-6, atol=1e-7)
+    """The reference's MAG model (GNN + Classifier, inventories in tests/golden/reference_record.json) has 21,173,389
+    parameters, and pyhgt_b200's GNN of the same shape has the reference GNN's parameter names and shapes."""
+    from pyhgt_b200.model import GNN
+    rec = load_record()
+    g, c = rec["mag_gnn_params"], rec["mag_classifier_params"]
+    assert sum(math.prod(s) for _, s in g) + sum(math.prod(s) for _, s in c) == 21173389
+    mine = GNN(in_dim=129, n_hid=512, num_types=4, num_relations=9, n_heads=8, n_layers=4,
+               prev_norm=True, last_norm=True, use_RTE=True)
+    assert [(n, tuple(p.shape)) for n, p in mine.named_parameters()] == [(n, tuple(s)) for n, s in g]
 
 
 def _random_case(seed, n=120, e=900, T=3, R=4, d=16, H=4, rte=True):
