@@ -1,5 +1,6 @@
 // Error channel + small utilities shared by every translation unit of libhgt_b200.so.
 #include "common.cuh"
+#include "tc_ptx.cuh"
 
 #include <string.h>
 
@@ -21,6 +22,38 @@ int hgt_sm_count() {
     n = HGT_SM_COUNT_FALLBACK;
   cached = n;
   return n;
+}
+
+// The driver entry point is looked up through the runtime, so the library does not link libcuda.
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+static EncodeTiledFn encode_fn() {
+  static EncodeTiledFn fn = nullptr;
+  if (fn) return fn;
+  void* p = nullptr;
+  cudaDriverEntryPointQueryResult q;
+  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
+      q != cudaDriverEntryPointSuccess)
+    return nullptr;
+  fn = reinterpret_cast<EncodeTiledFn>(p);
+  return fn;
+}
+
+int hgt_make_tma_map_bf16(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
+  EncodeTiledFn fn = encode_fn();
+  HGT_REQUIRE(fn != nullptr, "cuTensorMapEncodeTiled not available from the driver");
+  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)(rows > 0 ? rows : 1)};
+  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
+  cuuint32_t box[2] = {64u, (cuuint32_t)box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  HGT_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (%d) rows=%lld cols=%lld ld=%lld box_rows=%d", (int)r,
+              (long long)rows, (long long)cols, (long long)ld, box_rows);
+  return 0;
 }
 
 unsigned long long g_hgt_launches = 0;

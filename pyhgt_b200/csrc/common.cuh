@@ -1,6 +1,7 @@
 // Shared helpers for libhgt_b200.so (sm_100a only).
 #pragma once
 #include <cuda_runtime.h>
+#include <cuda_bf16.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdarg.h>
@@ -41,4 +42,19 @@ static inline size_t hgt_align_up(size_t x, size_t a) { return (x + a - 1) / a *
 __device__ __forceinline__ float hgt_gelu_erf(float x) {
   // F.gelu default (exact erf form), conv.py:119
   return 0.5f * x * (1.0f + erff(x * 0.70710678118654752440f));
+}
+
+// The operand format of every tcgen05 GEMM: x = hi + lo with hi = rn(x), lo = rn(x - hi), both bf16.  Every producer
+// splits through these two helpers, so pre-split operands (and sharded runs) round exactly like the GEMM's own split.
+__device__ __forceinline__ void hgt_split_bf16(float x, __nv_bfloat16& hi, __nv_bfloat16& lo) {
+  hi = __float2bfloat16_rn(x);
+  lo = __float2bfloat16_rn(x - __bfloat162float(hi));
+}
+// Four consecutive values, stored as one 8-byte word into each of hi and lo.
+__device__ __forceinline__ void hgt_split_bf16x4(const float (&v)[4], uint2* hi, uint2* lo) {
+  __nv_bfloat16 h[4], l[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) hgt_split_bf16(v[j], h[j], l[j]);
+  *hi = *reinterpret_cast<uint2*>(h);
+  *lo = *reinterpret_cast<uint2*>(l);
 }

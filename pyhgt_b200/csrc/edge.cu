@@ -19,8 +19,11 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "tc_ptx.cuh"
 
 namespace {
+
+using namespace tcp;
 
 constexpr int kWarpsPerCta = 16;
 constexpr int kCtaThreads = kWarpsPerCta * 32;
@@ -97,10 +100,7 @@ template <int VEC>
 __device__ __forceinline__ void store_split_bf16(__nv_bfloat16* hi, __nv_bfloat16* lo, const float (&src)[VEC]) {
   __nv_bfloat16 h[VEC], l[VEC];
 #pragma unroll
-  for (int i = 0; i < VEC; ++i) {
-    h[i] = __float2bfloat16_rn(src[i]);
-    l[i] = __float2bfloat16_rn(src[i] - __bfloat162float(h[i]));
-  }
+  for (int i = 0; i < VEC; ++i) hgt_split_bf16(src[i], h[i], l[i]);
   if constexpr (VEC == 4) {
     *reinterpret_cast<uint2*>(hi) = *reinterpret_cast<uint2*>(h);
     *reinterpret_cast<uint2*>(lo) = *reinterpret_cast<uint2*>(l);
@@ -327,35 +327,6 @@ k_edge_fwd_ldg(EdgeParams p) {
 // ------------------------------------------------------------------------------------------------
 // variant 2: bulk async copy (TMA engine) -> per-warp shared-memory ring
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return static_cast<uint32_t>(__cvta_generic_to_shared(p));
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t"
-      "}"
-      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  while (!mbar_try_wait(bar, parity)) {}
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src_gmem, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   dst_smem), "l"(src_gmem), "r"(bytes), "r"(bar)
-               : "memory");
-}
-
 template <int VEC, int NCH>
 __global__ void __launch_bounds__(kCtaThreads, (VEC * NCH <= 4) ? 2 : 1)   // narrow rows (d_k <= 16): two CTAs per SM
 k_edge_fwd_tma(EdgeParams p) {
@@ -372,8 +343,8 @@ k_edge_fwd_tma(EdgeParams p) {
   unsigned char* ring = smem_raw + (size_t)warp * S * slot_bytes;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + (size_t)kWarpsPerCta * S * slot_bytes) + warp * S;
   if (lane == 0) {
-    for (int s = 0; s < S; ++s) mbar_init(smem_u32(&bars[s]), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < S; ++s) mbar_init(s_u32(&bars[s]), 1);
+    fence_mbar_init();
   }
   __syncwarp();
   int offs[NCH];
@@ -418,8 +389,8 @@ k_edge_fwd_tma(EdgeParams p) {
       const int rrow = rte ? __shfl_sync(0xffffffffu, ridxA, c - ibase) : 0;
       const uint32_t slot = issue_it % S;
       if (lane == 0) {
-        const uint32_t bar = smem_u32(&bars[slot]);
-        const uint32_t dst = smem_u32(ring + (size_t)slot * slot_bytes);
+        const uint32_t bar = s_u32(&bars[slot]);
+        const uint32_t dst = s_u32(ring + (size_t)slot * slot_bytes);
         mbar_expect_tx(bar, slot_bytes);
         bulk_g2s(dst, p.kv + (int64_t)row * row_stride, row_bytes, bar);
         if (rte) bulk_g2s(dst + row_bytes, p.kvr + (int64_t)rrow * row_stride, row_bytes, bar);
@@ -448,7 +419,7 @@ k_edge_fwd_tma(EdgeParams p) {
         }
         for (int c = seg_begin; c < seg_end; ++c) {
           const uint32_t slot = it % S;
-          mbar_wait(smem_u32(&bars[slot]), (it / S) & 1u);
+          mbar_wait(s_u32(&bars[slot]), (it / S) & 1u);
           const float* srow = reinterpret_cast<const float*>(ring + (size_t)slot * slot_bytes);
           float kk[NCH][VEC], vv[NCH][VEC];
           float part = 0.f;
@@ -545,11 +516,7 @@ k_merge_partials(EdgeParams p, const int32_t* __restrict__ hubs, int n_hubs_host
         t *= s_inv[c / p.DK];
         t = p.apply_gelu ? hgt_gelu_erf(t) : t;
         if (p.agg_out) p.agg_out[(int64_t)dst * p.d + c] = t;
-        if (p.g_hi) {
-          const __nv_bfloat16 h = __float2bfloat16_rn(t);
-          p.g_hi[(int64_t)dst * p.d + c] = h;
-          p.g_lo[(int64_t)dst * p.d + c] = __float2bfloat16_rn(t - __bfloat162float(h));
-        }
+        if (p.g_hi) hgt_split_bf16(t, p.g_hi[(int64_t)dst * p.d + c], p.g_lo[(int64_t)dst * p.d + c]);
       }
       __syncthreads();
     }

@@ -22,7 +22,6 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 
-#include <stdlib.h>
 #include <algorithm>
 #include <utility>
 #include <vector>
@@ -48,17 +47,6 @@ __device__ __forceinline__ void map_acquire(const CUtensorMap* m) {
 __device__ __forceinline__ float gelu_grad(float x) {
   // d/dx [0.5 x (1 + erf(x / sqrt 2))]
   return 0.5f * (1.0f + erff(x * 0.70710678118654752440f)) + x * 0.39894228040143267794f * __expf(-0.5f * x * x);
-}
-
-__device__ __forceinline__ void split4(const float (&v)[4], uint2* hi, uint2* lo) {
-  __nv_bfloat16 h[4], l[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    h[j] = __float2bfloat16_rn(v[j]);
-    l[j] = __float2bfloat16_rn(v[j] - __bfloat162float(h[j]));
-  }
-  *hi = *reinterpret_cast<uint2*>(h);
-  *lo = *reinterpret_cast<uint2*>(l);
 }
 
 // ---- fp32 [rows, K] (row stride ld) -> act(x) as fp32 and/or the bf16 hi/lo split [rows, Kp] -------------------------
@@ -87,7 +75,7 @@ __global__ void k_act_split(const float* __restrict__ in, int64_t ld, int64_t ro
     for (int j = 0; j < 4; ++j)
       if (c + j < K) out_f32[r * K + c + j] = v[j];
   }
-  if (hi) split4(v, reinterpret_cast<uint2*>(hi + r * Kp + c), reinterpret_cast<uint2*>(lo + r * Kp + c));
+  if (hi) hgt_split_bf16x4(v, reinterpret_cast<uint2*>(hi + r * Kp + c), reinterpret_cast<uint2*>(lo + r * Kp + c));
 }
 
 // ---- W [w_rows, K] -> W^T split, block-padded:  WT[k, blk*wpad + n] = W[blk*width + n, k], zero for n >= width ----------
@@ -102,9 +90,7 @@ __global__ void k_wt_split(const float* __restrict__ W, int64_t w_rows, int K, i
   float v = 0.f;
   const int64_t wr = blk * width + n;
   if (n < width && wr < w_rows) v = W[wr * K + k];
-  const __nv_bfloat16 h = __float2bfloat16_rn(v);
-  hi[i] = h;
-  lo[i] = __float2bfloat16_rn(v - __bfloat162float(h));
+  hgt_split_bf16(v, hi[i], lo[i]);
 }
 
 // ---- dOut split pass + bias gradient ---------------------------------------------------------------------------------
@@ -143,7 +129,7 @@ k_split_colsum(const float* __restrict__ dout, const GcTask* __restrict__ tasks,
         const int64_t off = tk.out_off + r * tk.ld + c0 * 4;
         const float4 v4 = *reinterpret_cast<const float4*>(dout + off);
         const float v[4] = {v4.x, v4.y, v4.z, v4.w};
-        split4(v, reinterpret_cast<uint2*>(hi + off), reinterpret_cast<uint2*>(lo + off));
+        hgt_split_bf16x4(v, reinterpret_cast<uint2*>(hi + off), reinterpret_cast<uint2*>(lo + off));
 #pragma unroll
         for (int j = 0; j < 4; ++j) s[j] += v[j];
       }
@@ -206,12 +192,10 @@ k_lin_dx_tc(const CUtensorMap* __restrict__ maps, int map_wt, const GcTask* __re
       mbar_init(s_u32(&empty_bar[s]), 1);
     }
     mbar_init(s_u32(tmem_full_bar), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_ptr_smem)),
-                 "r"(256u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(s_u32(tmem_ptr_smem), 256u);
   }
   tc_fence_before();
   __syncthreads();
@@ -303,7 +287,7 @@ k_lin_dx_tc(const CUtensorMap* __restrict__ maps, int map_wt, const GcTask* __re
   tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256u) : "memory");
+    tmem_dealloc<1>(tmem_base, 256u);
   }
 }
 
@@ -344,12 +328,10 @@ k_lin_dw_tc(const CUtensorMap* __restrict__ maps, const GcTask* __restrict__ tas
       mbar_init(s_u32(&empty_bar[s]), 1);
     }
     mbar_init(s_u32(tmem_full_bar), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_ptr_smem)),
-                 "r"(256u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(s_u32(tmem_ptr_smem), 256u);
   }
   tc_fence_before();
   __syncthreads();
@@ -431,7 +413,7 @@ k_lin_dw_tc(const CUtensorMap* __restrict__ maps, const GcTask* __restrict__ tas
   tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256u) : "memory");
+    tmem_dealloc<1>(tmem_base, 256u);
   }
 }
 
@@ -515,38 +497,6 @@ k_lin_dw_simt(const float* __restrict__ dout, const float* __restrict__ A, int64
 }
 
 // ---- host helpers ---------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn) return fn;
-  void* p = nullptr;
-  cudaDriverEntryPointQueryResult q;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-      q != cudaDriverEntryPointSuccess)
-    return nullptr;
-  fn = reinterpret_cast<EncodeTiledFn>(p);
-  return fn;
-}
-
-// 2-D bf16 map over [rows, cols] with row stride `ld` elements, box {64 columns, box_rows}, SWIZZLE_128B, OOB -> 0.
-int make_map2(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
-  EncodeTiledFn fn = encode_fn();
-  HGT_REQUIRE(fn != nullptr, "hgt_typed_linear_bwd: cuTensorMapEncodeTiled not available from the driver");
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)(rows > 0 ? rows : 1)};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {64u, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  HGT_REQUIRE(r == CUDA_SUCCESS, "hgt_typed_linear_bwd: cuTensorMapEncodeTiled failed (%d) rows=%lld cols=%lld ld=%lld",
-              (int)r, (long long)rows, (long long)cols, (long long)ld);
-  return 0;
-}
-
 struct BwdLayout {
   bool tc;
   int Kp, wpad;
@@ -565,8 +515,6 @@ bool groups_overlap(const hgt_lin_group* h, int n) {
 }
 
 bool bwd_tc_ok(const hgt_lin_group* h_groups, int n_groups, const hgt_lin_cblock* h_cb, int K, int width, int64_t lda) {
-  static const bool off = [] { const char* e = getenv("HGT_BWD_SIMT"); return e && e[0] == '1'; }();
-  if (off) return false;
   if (width % 8 || K % 16 || K < 64 || width < 16 || lda != K) return false;
   if (groups_overlap(h_groups, n_groups)) return false;
   int64_t rows = 0;
@@ -615,18 +563,23 @@ BwdLayout bwd_layout(const hgt_lin_group* h_groups, int n_groups, const hgt_lin_
 
 }  // namespace
 
+// k_act_split over [rows, K] into split rows of pitch Kp (a multiple of 4, >= K); also the forward GEMM's operand split.
+int hgt_act_split_launch(const float* in, int64_t ld, int64_t rows, int K, int Kp, int act, float* out_f32,
+                         __nv_bfloat16* hi, __nv_bfloat16* lo, cudaStream_t st) {
+  if (rows == 0) return 0;
+  const int64_t n = rows * (Kp / 4);
+  k_act_split<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(in, ld, rows, K, Kp, act, out_f32, hi, lo);
+  HGT_LAUNCH_CHECK();
+  return 0;
+}
+
 extern "C" int hgt_act_split(const float* in, int64_t ld, int64_t rows, int32_t K, int32_t act, float* out_f32,
                              void* hi, void* lo, void* stream_) {
   HGT_REQUIRE(in && (out_f32 || (hi && lo)), "hgt_act_split: NULL argument");
   HGT_REQUIRE(act == 0 || act == 1, "hgt_act_split: act=%d (0 = identity, 1 = gelu)", act);
   HGT_REQUIRE(!hi || K % 8 == 0, "hgt_act_split: the bf16 split needs K %% 8 == 0 (K=%d)", K);
-  if (rows == 0) return 0;
-  const int Kp = (K + 3) / 4 * 4;
-  const int64_t n = rows * (Kp / 4);
-  k_act_split<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream_>>>(
-      in, ld, rows, K, Kp, act, out_f32, reinterpret_cast<__nv_bfloat16*>(hi), reinterpret_cast<__nv_bfloat16*>(lo));
-  HGT_LAUNCH_CHECK();
-  return 0;
+  return hgt_act_split_launch(in, ld, rows, K, (K + 3) / 4 * 4, act, out_f32, reinterpret_cast<__nv_bfloat16*>(hi),
+                              reinterpret_cast<__nv_bfloat16*>(lo), (cudaStream_t)stream_);
 }
 
 extern "C" int hgt_typed_linear_bwd_workspace_bytes(const hgt_lin_group* h_groups, int32_t n_groups,
@@ -767,9 +720,7 @@ extern "C" int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, cons
   // 2. A split (dW needs it) unless saved by the forward
   if (dW && !have_asplit && L.a_rows > 0) {
     HGT_REQUIRE(A, "hgt_typed_linear_bwd: dW needs A or its bf16 split");
-    const int64_t n = L.a_rows * (K / 4);
-    k_act_split<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(A, lda, L.a_rows, K, K, 0, nullptr, a_hi, a_lo);
-    HGT_LAUNCH_CHECK();
+    if ((rc = hgt_act_split_launch(A, lda, L.a_rows, K, K, 0, nullptr, a_hi, a_lo, st))) return rc;
   }
   // 3. W^T split (dX)
   if (dA) {
@@ -780,17 +731,19 @@ extern "C" int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, cons
   // 4. tensor maps: per task dOut hi/lo {cols = width, rows = m}; per group A hi/lo {cols = K, rows = m}; W^T hi/lo
   std::vector<CUtensorMap> maps(2 * nt + 2 * n_groups + 2);
   for (int t = 0; t < nt; ++t) {
-    if ((rc = make_map2(&maps[2 * t], d_hi + tasks[t].out_off, tasks[t].rows, cb_width, tasks[t].ld, 64))) return rc;
-    if ((rc = make_map2(&maps[2 * t + 1], d_lo + tasks[t].out_off, tasks[t].rows, cb_width, tasks[t].ld, 64))) return rc;
+    const int64_t off = tasks[t].out_off, rows = tasks[t].rows, ld = tasks[t].ld;
+    if ((rc = hgt_make_tma_map_bf16(&maps[2 * t], d_hi + off, rows, cb_width, ld, 64))) return rc;
+    if ((rc = hgt_make_tma_map_bf16(&maps[2 * t + 1], d_lo + off, rows, cb_width, ld, 64))) return rc;
   }
   for (int g = 0; g < n_groups; ++g) {
-    if ((rc = make_map2(&maps[2 * nt + 2 * g], a_hi + h_groups[g].a_row0 * K, h_groups[g].m, K, K, 64))) return rc;
-    if ((rc = make_map2(&maps[2 * nt + 2 * g + 1], a_lo + h_groups[g].a_row0 * K, h_groups[g].m, K, K, 64))) return rc;
+    const int64_t off = h_groups[g].a_row0 * K, rows = h_groups[g].m;
+    if ((rc = hgt_make_tma_map_bf16(&maps[2 * nt + 2 * g], a_hi + off, rows, K, K, 64))) return rc;
+    if ((rc = hgt_make_tma_map_bf16(&maps[2 * nt + 2 * g + 1], a_lo + off, rows, K, K, 64))) return rc;
   }
   const int map_wt = 2 * nt + 2 * n_groups;
   const int bn_box = K >= 256 ? 256 : K;
-  if ((rc = make_map2(&maps[map_wt], wt_hi, K, L.wt_cols, L.wt_cols, bn_box))) return rc;
-  if ((rc = make_map2(&maps[map_wt + 1], wt_lo, K, L.wt_cols, L.wt_cols, bn_box))) return rc;
+  if ((rc = hgt_make_tma_map_bf16(&maps[map_wt], wt_hi, K, L.wt_cols, L.wt_cols, bn_box))) return rc;
+  if ((rc = hgt_make_tma_map_bf16(&maps[map_wt + 1], wt_lo, K, L.wt_cols, L.wt_cols, bn_box))) return rc;
   CUtensorMap* d_maps = reinterpret_cast<CUtensorMap*>(base + L.off_maps);
   HGT_CHECK_CUDA(cudaMemcpyAsync(d_maps, maps.data(), maps.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice, st));
 

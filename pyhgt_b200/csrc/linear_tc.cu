@@ -15,11 +15,15 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 
-#include <stdlib.h>
-
 #include "common.cuh"
+#include "tc_ptx.cuh"
+
+int hgt_act_split_launch(const float* in, int64_t ld, int64_t rows, int K, int Kp, int act, float* out_f32,
+                         __nv_bfloat16* hi, __nv_bfloat16* lo, cudaStream_t st);
 
 namespace {
+
+using namespace tcp;
 
 constexpr int kMaxGroups = 64;
 constexpr int TC_BM = 128;
@@ -31,96 +35,6 @@ struct TcTilePrefix {
   int32_t first_tile[kMaxGroups + 1];
   int32_t n_tiles_n;
 };
-
-// ---- PTX wrappers ------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t s_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t"
-      "}"
-      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  while (!mbar_try_wait(bar, parity)) {}
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t smem_dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_dst), "l"(map), "r"(bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void umma_bf16_ss(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                             uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-
-// K-major, SWIZZLE_128B shared-memory matrix descriptor (sm_100 UMMA format): rows of 128 bytes,
-// 8-row swizzle atoms 1024 bytes apart (SBO), version 1, layout type 2.
-__device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3FFFF) >> 4);          // start address, bits [0,14)
-  d |= (uint64_t)1 << 16;                               // leading byte offset (ignored for swizzled K-major)
-  d |= (uint64_t)(1024 >> 4) << 32;                     // stride byte offset, bits [32,46)
-  d |= (uint64_t)1 << 46;                               // descriptor version (Blackwell)
-  d |= (uint64_t)2 << 61;                               // SWIZZLE_128B
-  return d;
-}
-
-// ---- fp32 -> (bf16 hi, bf16 lo) split ------------------------------------------------------------
-__global__ void k_split_bf16(const float* __restrict__ in, int64_t ld_in, int64_t rows, int K, int Kp,
-                             __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo) {
-  const int vec_per_row = Kp / 4;
-  int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (i >= rows * vec_per_row) return;
-  int64_t r = i / vec_per_row;
-  int c = (int)(i - r * vec_per_row) * 4;
-  float v[4];
-  const float* src = in + r * ld_in + c;
-  if (c + 3 < K && ((reinterpret_cast<uintptr_t>(src) & 15) == 0)) {
-    float4 t = *reinterpret_cast<const float4*>(src);
-    v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
-  } else {
-#pragma unroll
-    for (int j = 0; j < 4; ++j) v[j] = (c + j < K) ? src[j] : 0.f;
-  }
-  __nv_bfloat16 h[4], l[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    h[j] = __float2bfloat16_rn(v[j]);
-    l[j] = __float2bfloat16_rn(v[j] - __bfloat162float(h[j]));
-  }
-  *reinterpret_cast<uint2*>(hi + r * Kp + c) = *reinterpret_cast<uint2*>(h);
-  *reinterpret_cast<uint2*>(lo + r * Kp + c) = *reinterpret_cast<uint2*>(l);
-}
 
 // ---- the GEMM -------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(TC_THREADS, 2)
@@ -167,30 +81,27 @@ k_typed_linear_tc(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
   const int total_iters = 3 * k_blocks;
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a_hi) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a_lo) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w_hi) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w_lo) : "memory");
+    prefetch_map(&map_a_hi);
+    prefetch_map(&map_a_lo);
+    prefetch_map(&map_w_hi);
+    prefetch_map(&map_w_lo);
     for (int s = 0; s < stages; ++s) {
       mbar_init(s_u32(&full_bar[s]), 1);
       mbar_init(s_u32(&empty_bar[s]), 1);
     }
     mbar_init(s_u32(tmem_full_bar), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_ptr_smem)),
-                 "r"((uint32_t)tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(s_u32(tmem_ptr_smem), (uint32_t)tmem_cols);
   }
   if (warp >= 2) {
     for (int c = threadIdx.x - 64; c < BN; c += TC_THREADS - 64)
       s_bias[c] = (grp.has_bias && bias) ? bias[w_row + c] : 0.f;
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
 
   if (warp == 0) {
@@ -214,18 +125,15 @@ k_typed_linear_tc(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
   } else if (warp == 1) {
     if (lane == 0) {
       // ===== MMA issuer =====
-      // instruction descriptor: D=f32 (bits 4-5 = 1), A=B=bf16 (bits 7-9, 10-12 = 1), K-major A and B,
-      // N>>3 at bits 17-22, M>>4 at bits 24-28
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) |
-                             ((uint32_t)(TC_BM >> 4) << 24);
+      const uint32_t idesc = idesc_bf16(TC_BM, BN, false, false);
       for (int it = 0; it < total_iters; ++it) {
         const int s = it % stages;
         const uint32_t ph = (uint32_t)(it / stages) & 1u;
         mbar_wait(s_u32(&full_bar[s]), ph);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const uint32_t sa = s_u32(smem + (size_t)s * stage_bytes);
-        const uint64_t da = make_sw128_desc(sa);
-        const uint64_t db = make_sw128_desc(sa + a_bytes);
+        const uint64_t da = desc_k_sw128(sa);
+        const uint64_t db = desc_k_sw128(sa + a_bytes);
 #pragma unroll
         for (int k = 0; k < TC_BK / UMMA_K; ++k) {
           // advance 16 bf16 = 32 bytes inside the 128-byte swizzle row: +2 in the (addr >> 4) field
@@ -240,13 +148,13 @@ k_typed_linear_tc(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
     const int lg = warp & 3;
     const int row = lg * 32 + lane;
     mbar_wait(s_u32(tmem_full_bar), 0);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc_fence_after();
     float* orow = out + cblk.out_off + (m0 + row) * cblk.ld + n0;
     const bool row_ok = row < rows_here;
     for (int c = 0; c < BN; c += 16) {
       uint32_t r[16];
       tmem_ld16(tmem_base + ((uint32_t)(lg * 32) << 16) + (uint32_t)c, r);
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+      tmem_ld_wait();
       if (row_ok) {
 #pragma unroll
         for (int j = 0; j < 16; j += 4) {
@@ -260,25 +168,24 @@ k_typed_linear_tc(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)tmem_cols)
-                 : "memory");
+    tmem_dealloc<1>(tmem_base, (uint32_t)tmem_cols);
   }
 }
 
 
 // ---- W-stationary persistent GEMM (default) -------------------------------------------------------
-// A "unit" = one column task (group, column block, n-tile of BN columns) x a chunk of up to MCH m-tiles.
+// A "unit" = one column task (group, column block, n-tile of BN columns) x a chunk of up to TC2_MCH m-tiles.
 // The CTA keeps the column task's W_hi / W_lo tiles (all K) resident in shared memory, streams the A_hi / A_lo
 // k-blocks of successive m-tiles through a ring, and issues per k-block the three products
 // A_hi*W_hi + A_hi*W_lo + A_lo*W_hi into a double-buffered TMEM accumulator, so the epilogue of m-tile i
 // overlaps the MMAs of m-tile i+1.  Units are ordered m-chunk-major so that CTAs running concurrently read the
 // same A rows from L2 with different W.  L2->SM traffic per output tile drops from 384 KB (tile-per-CTA kernel
 // below) to 128 KB (+ W amortised over the chunk).
-static int tc2_mch() { static int v = [] { const char* e = getenv("HGT_TC_MCH"); int x = e ? atoi(e) : 8; return x < 1 ? 1 : x; }(); return v; }
-static int tc2_stage_cap() { static int v = [] { const char* e = getenv("HGT_TC_STAGES"); int x = e ? atoi(e) : 8; return x < 2 ? 2 : x; }(); return v; }
+constexpr int TC2_MCH = 8;                     // m-tiles (tc3: 256-row pair steps) per unit
+constexpr int TC2_STAGE_CAP = 8;               // A ring stages at most
 
 // Epilogue of one accumulator tile, shared by the persistent kernels.  8 epilogue warps: warp e (0..7) reads TMEM
 // lane quarter (warp id % 4) and the 16-column chunks c0 = 16*(e/4), +32, ...  TMEM hands each lane one ROW, so the
@@ -286,41 +193,15 @@ static int tc2_stage_cap() { static int v = [] { const char* e = getenv("HGT_TC_
 // (full 32-byte sectors).  All shared-memory reads are issued before the dependent adds / predicated stores.
 constexpr int TC2_EPI_WARPS = 8;
 constexpr int TC2_THREADS = 64 + 32 * TC2_EPI_WARPS;
-constexpr int TC2_STG_LD = 20;                 // floats per staged row (16 + 4 pad)
+// The staging region is sized for rows of 20 floats, although the swizzled drain below uses 16 of them: its size enters
+// the shared-memory budget and with it the A-ring stage counts of both persistent kernels.
+constexpr int TC2_STG_LD = 20;
 constexpr int TC2_STAGE_BYTES = TC2_EPI_WARPS * 32 * TC2_STG_LD * 4;
 
-__device__ __forceinline__ void tc_epilogue_tile(uint32_t t_row, int n_cols, int chunk0, float* stg, const float* s_bias,
-                                                 float* out_tile, int64_t ld, int64_t rows_left, int lane) {
-  // out_tile: address of (first row of this warp's 32-row slab, column 0 of the tile); rows_left: valid rows in the slab
-  const int sub = lane & 3, rsel = lane >> 2;
-  for (int c0 = 16 * chunk0; c0 < n_cols; c0 += 32) {
-    uint32_t r[16];
-    tmem_ld16(t_row + (uint32_t)c0, r);
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int j = 0; j < 16; j += 4)
-      *reinterpret_cast<uint4*>(stg + lane * TC2_STG_LD + j) = make_uint4(r[j], r[j + 1], r[j + 2], r[j + 3]);
-    __syncwarp();
-    const float4 b = *reinterpret_cast<const float4*>(s_bias + c0 + sub * 4);
-    float4 v[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) v[k] = *reinterpret_cast<const float4*>(stg + (8 * k + rsel) * TC2_STG_LD + sub * 4);
-    __syncwarp();
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int rr = 8 * k + rsel;
-      if (rr < rows_left) {
-        float4 w = v[k];
-        w.x += b.x; w.y += b.y; w.z += b.z; w.w += b.w;
-        *reinterpret_cast<float4*>(out_tile + (int64_t)rr * ld + c0 + sub * 4) = w;
-      }
-    }
-  }
-}
-
-// Same tile, software-pipelined: the TMEM load of chunk i+1 is in flight while chunk i goes through the staging buffer
-// and out to global memory (two named register buffers), and the staging buffer is swizzled so that neither side has
-// bank conflicts.  Measured at C2 together with the .cta-scope pair barriers below: projection 3.90 -> 3.81 ms
+// The drain is software-pipelined: the TMEM load of chunk i+1 is in flight while chunk i goes through the staging
+// buffer and out to global memory (two named register buffers), and the staging buffer is swizzled so that neither side
+// has bank conflicts.  Measured at C2 together with the .cta-scope pair barriers: projection 3.90 -> 3.81 ms against the
+// round-1 drain; a drain straight from registers without the transpose ran at the same speed
 // (profiles/r02_gemm_epilogue_ab.md); see DESIGN.md section 9 for what was ruled out as the limiter.
 __device__ __forceinline__ void tc_epi_chunk(const uint32_t (&r)[16], int c0, float* stg, const float* s_bias,
                                              float* out_tile, int64_t ld, int64_t rows_left, int lane) {
@@ -359,85 +240,27 @@ __device__ __forceinline__ void tc_epilogue_tile_pf(uint32_t t_row, int n_cols, 
   tmem_ld16(t_row + (uint32_t)c0, ra);
   for (; c0 < n_cols; c0 += 64) {
     const bool has_b = c0 + 32 < n_cols;
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");       // ra has landed
+    tmem_ld_wait();                                                    // ra has landed
     if (has_b) tmem_ld16(t_row + (uint32_t)(c0 + 32), rb);
     tc_epi_chunk(ra, c0, stg, s_bias, out_tile, ld, rows_left, lane);
     if (!has_b) break;
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");       // rb has landed
+    tmem_ld_wait();                                                    // rb has landed
     if (c0 + 64 < n_cols) tmem_ld16(t_row + (uint32_t)(c0 + 64), ra);
     tc_epi_chunk(rb, c0 + 32, stg, s_bias, out_tile, ld, rows_left, lane);
-  }
-}
-
-// Direct drain (HGT_TC_EPI bit 2, opt-in): tcgen05.ld.16x256b hands each quad of lanes 32 contiguous bytes of an
-// accumulator row (the m16n8 fragment layout: registers {0,1} = row lane/4, columns 2*(lane%4)+{0,1}; {2,3} = row
-// lane/4 + 8; the next four registers the next 8 columns), so the tile goes from registers to global memory as full
-// 32-byte sectors with no trip through shared memory.  A warp covers its 32 TMEM lanes with two 16-lane loads.
-// Parity-green on the whole GPU suite and the SAME speed as the staged drain at C2 (projection 3.778 vs 3.788 ms,
-// profiles/r02_gemm_epilogue_ab.md) — so the transpose's share of the shared-memory port is not what holds the kernel;
-// kept as an option because it needs no staging buffer.
-__device__ __forceinline__ void tmem_ld_16x256b_x2(uint32_t taddr, uint32_t (&r)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.16x256b.x2.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr));
-}
-
-__device__ __forceinline__ void tc_epi_direct_store(const uint32_t (&v)[8], int row0, int c0, const float* s_bias,
-                                                    float* out_tile, int64_t ld, int64_t rows_left, int lane) {
-  const int q = lane & 3, r0 = row0 + (lane >> 2);
-#pragma unroll
-  for (int i = 0; i < 2; ++i) {
-    const int col = c0 + 8 * i + 2 * q;
-    const float2 b = *reinterpret_cast<const float2*>(s_bias + col);
-    if (r0 < rows_left)
-      *reinterpret_cast<float2*>(out_tile + (int64_t)r0 * ld + col) =
-          make_float2(__uint_as_float(v[4 * i]) + b.x, __uint_as_float(v[4 * i + 1]) + b.y);
-    if (r0 + 8 < rows_left)
-      *reinterpret_cast<float2*>(out_tile + (int64_t)(r0 + 8) * ld + col) =
-          make_float2(__uint_as_float(v[4 * i + 2]) + b.x, __uint_as_float(v[4 * i + 3]) + b.y);
-  }
-}
-
-__device__ __forceinline__ void tc_epilogue_tile_direct(uint32_t t_row, int n_cols, int chunk0, const float* s_bias,
-                                                        float* out_tile, int64_t ld, int64_t rows_left, int lane) {
-  uint32_t a0[8], a1[8], b0[8], b1[8];                       // (rows 0-15, rows 16-31) of two chunks in flight
-  int c0 = 16 * chunk0;
-  if (c0 >= n_cols) return;
-  tmem_ld_16x256b_x2(t_row + (uint32_t)c0, a0);
-  tmem_ld_16x256b_x2(t_row + (16u << 16) + (uint32_t)c0, a1);
-  for (; c0 < n_cols; c0 += 64) {
-    const bool has_b = c0 + 32 < n_cols;
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-    if (has_b) {
-      tmem_ld_16x256b_x2(t_row + (uint32_t)(c0 + 32), b0);
-      tmem_ld_16x256b_x2(t_row + (16u << 16) + (uint32_t)(c0 + 32), b1);
-    }
-    tc_epi_direct_store(a0, 0, c0, s_bias, out_tile, ld, rows_left, lane);
-    tc_epi_direct_store(a1, 16, c0, s_bias, out_tile, ld, rows_left, lane);
-    if (!has_b) break;
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-    if (c0 + 64 < n_cols) {
-      tmem_ld_16x256b_x2(t_row + (uint32_t)(c0 + 64), a0);
-      tmem_ld_16x256b_x2(t_row + (16u << 16) + (uint32_t)(c0 + 64), a1);
-    }
-    tc_epi_direct_store(b0, 0, c0 + 32, s_bias, out_tile, ld, rows_left, lane);
-    tc_epi_direct_store(b1, 16, c0 + 32, s_bias, out_tile, ld, rows_left, lane);
   }
 }
 
 struct Tc2Sched {
   int32_t first_unit[kMaxGroups + 1];
   int32_t n_tiles_n;
-  int32_t epi;                                   // bit 0: pipelined epilogue; bit 1: .cta-scope pair barriers; bit 2: direct drain (default 3)
 };
-static int tc2_epi() { static int v = [] { const char* e = getenv("HGT_TC_EPI"); return e ? atoi(e) : 3; }(); return v; }
 
 __global__ void __launch_bounds__(TC2_THREADS, 1)
 k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                    const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
                    const float* __restrict__ bias, int Kp, int cb_width, int BN, int stages, int tmem_cols,
                    const hgt_lin_group* __restrict__ groups, int n_groups,
-                   const hgt_lin_cblock* __restrict__ cblocks, float* __restrict__ out, Tc2Sched sc, int MCH) {
+                   const hgt_lin_cblock* __restrict__ cblocks, float* __restrict__ out, Tc2Sched sc) {
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = smem_dyn + ((1024u - (s_u32(smem_dyn) & 1023u)) & 1023u);   // keeps the shared address space
   const int k_blocks = (Kp + TC_BK - 1) / TC_BK;
@@ -464,10 +287,10 @@ k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
   const int total_units = sc.first_unit[n_groups];
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a_hi) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a_lo) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w_hi) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w_lo) : "memory");
+    prefetch_map(&map_a_hi);
+    prefetch_map(&map_a_lo);
+    prefetch_map(&map_w_hi);
+    prefetch_map(&map_w_lo);
     for (int s = 0; s < stages; ++s) {
       mbar_init(s_u32(&a_full[s]), 1);
       mbar_init(s_u32(&a_empty[s]), 1);
@@ -478,17 +301,14 @@ k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
       mbar_init(s_u32(&t_full[b]), 1);
       mbar_init(s_u32(&t_empty[b]), TC2_EPI_WARPS);                  // one arrival per epilogue warp
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_ptr_smem)),
-                 "r"((uint32_t)tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(s_u32(tmem_ptr_smem), (uint32_t)tmem_cols);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
 
   // unit decode shared by all roles
@@ -506,8 +326,8 @@ k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
     const int nt = col - cb * sc.n_tiles_n;
     const hgt_lin_cblock cblk = cblocks[grp.cb_first + cb];
     const int64_t mt_total = (grp.m + TC_BM - 1) / TC_BM;
-    un.m_first = (int64_t)chunk * MCH;
-    un.n_mt = (int)min((int64_t)MCH, mt_total - un.m_first);
+    un.m_first = (int64_t)chunk * TC2_MCH;
+    un.n_mt = (int)min((int64_t)TC2_MCH, mt_total - un.m_first);
     un.a_row0 = (int)grp.a_row0;
     un.m_rows = grp.m;
     un.n0 = nt * BN;
@@ -545,8 +365,7 @@ k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
   } else if (warp == 1) {
     if (lane == 0) {
       // ===== MMA issuer =====
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) |
-                             ((uint32_t)(TC_BM >> 4) << 24);
+      const uint32_t idesc = idesc_bf16(TC_BM, BN, false, false);
       uint32_t a_it = 0, unit_it = 0, acc_it = 0;
       for (int u = blockIdx.x; u < total_units; u += gridDim.x, ++unit_it) {
         Unit un;
@@ -555,18 +374,18 @@ k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
         for (int mt = 0; mt < un.n_mt; ++mt, ++acc_it) {
           const uint32_t buf = acc_it & 1u;
           mbar_wait(s_u32(&t_empty[buf]), ((acc_it >> 1) & 1u) ^ 1u);  // epilogue drained this accumulator
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const uint32_t tmem_d = tmem_base + buf * (uint32_t)BN;
           for (int j = 0; j < 2 * k_blocks; ++j, ++a_it) {
             const int s = a_it % stages;
             const int kb = j >> 1;
             mbar_wait(s_u32(&a_full[s]), (a_it / stages) & 1u);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const uint64_t d_a = make_sw128_desc(s_u32(a_smem + (size_t)s * a_stage));
-            const uint64_t d_whi = make_sw128_desc(s_u32(w_smem + (size_t)(2 * kb) * b_bytes_al));
+            tc_fence_after();
+            const uint64_t d_a = desc_k_sw128(s_u32(a_smem + (size_t)s * a_stage));
+            const uint64_t d_whi = desc_k_sw128(s_u32(w_smem + (size_t)(2 * kb) * b_bytes_al));
             if (!(j & 1)) {
               // A_hi(kb): A_hi*W_hi + A_hi*W_lo
-              const uint64_t d_wlo = make_sw128_desc(s_u32(w_smem + (size_t)(2 * kb + 1) * b_bytes_al));
+              const uint64_t d_wlo = desc_k_sw128(s_u32(w_smem + (size_t)(2 * kb + 1) * b_bytes_al));
 #pragma unroll
               for (int k = 0; k < TC_BK / UMMA_K; ++k) {
                 const uint64_t o = (uint64_t)(2 * k);
@@ -604,28 +423,20 @@ k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
       for (int mt = 0; mt < un.n_mt; ++mt, ++acc_it) {
         const uint32_t buf = acc_it & 1u;
         mbar_wait(s_u32(&t_full[buf]), (acc_it >> 1) & 1u);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const int64_t m0 = (un.m_first + mt) * TC_BM + lg * 32;
-        if (sc.epi & 4)
-          tc_epilogue_tile_direct(tmem_base + ((uint32_t)(lg * 32) << 16) + buf * (uint32_t)BN, BN, e >> 2, s_bias,
-                                  out + un.out_off + m0 * un.ld + un.n0, un.ld, un.m_rows - m0, lane);
-        else if (sc.epi & 1)
-          tc_epilogue_tile_pf(tmem_base + ((uint32_t)(lg * 32) << 16) + buf * (uint32_t)BN, BN, e >> 2, stg, s_bias,
-                              out + un.out_off + m0 * un.ld + un.n0, un.ld, un.m_rows - m0, lane);
-        else
-          tc_epilogue_tile(tmem_base + ((uint32_t)(lg * 32) << 16) + buf * (uint32_t)BN, BN, e >> 2, stg, s_bias,
-                           out + un.out_off + m0 * un.ld + un.n0, un.ld, un.m_rows - m0, lane);
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_epilogue_tile_pf(tmem_base + ((uint32_t)(lg * 32) << 16) + buf * (uint32_t)BN, BN, e >> 2, stg, s_bias,
+                            out + un.out_off + m0 * un.ld + un.n0, un.ld, un.m_rows - m0, lane);
+        tc_fence_before();
         __syncwarp();
-        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(s_u32(&t_empty[buf])) : "memory");
+        if (lane == 0) mbar_arrive(s_u32(&t_empty[buf]));
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)tmem_cols)
-                 : "memory");
+    tmem_dealloc<1>(tmem_base, (uint32_t)tmem_cols);
   }
 }
 
@@ -641,98 +452,12 @@ k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
 // peer-bit-masked address, the leader's producer posts expect_tx for both); a_empty / w_empty / t_full are
 // per-CTA and signalled by multicast tcgen05.commit; t_empty lives in the leader and collects the 8 epilogue
 // warps of the pair.
-constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tma_load_2d_2sm(uint32_t smem_dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_dst), "l"(map), "r"(bar & kPeerBitMask), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void umma_bf16_ss_2sm(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                                 uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(bar), "h"((uint16_t)3)
-      : "memory");
-}
-// Barrier traffic between the two CTAs of a pair carries no generic-proxy data: operands arrive through TMA
-// (complete_tx), accumulators are handed over with tcgen05.commit / tcgen05.fence.  The arrive / wait therefore use the
-// default .cta-scope forms.  (The .release.cluster arrive compiles to MEMBAR.ALL.GPU + ERRBAR, which made every
-// epilogue warp wait for its global stores to be acknowledged before it could hand the accumulator back, and the
-// .acquire.cluster wait adds an L1 invalidate per wait: profiles/r02_gemm_tc3_c2_epi1_ncu_raw.csv, stall_membar = 20 %
-// of the warp samples.)
-// `strong` keeps the old forms for A/B runs (HGT_TC_EPI bit 1 clear).
-__device__ __forceinline__ void mbar_arrive_cta(uint32_t bar, uint32_t cta, bool strong) {
-  if (strong)
-    asm volatile(
-        "{\n\t"
-        ".reg .b32 ra;\n\t"
-        "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-        "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t"
-        "}"
-        ::"r"(bar), "r"(cta)
-        : "memory");
-  else
-    asm volatile(
-        "{\n\t"
-        ".reg .b32 ra;\n\t"
-        "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-        "mbarrier.arrive.shared::cluster.b64 _, [ra];\n\t"
-        "}"
-        ::"r"(bar), "r"(cta)
-        : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity, bool strong) {
-  uint32_t ok = 0;
-  if (strong) {
-    while (!ok) {
-      asm volatile(
-          "{\n\t"
-          ".reg .pred p;\n\t"
-          "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-          "selp.u32 %0, 1, 0, p;\n\t"
-          "}"
-          : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    }
-  } else {
-    while (!ok) {
-      asm volatile(
-          "{\n\t"
-          ".reg .pred p;\n\t"
-          "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-          "selp.u32 %0, 1, 0, p;\n\t"
-          "}"
-          : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    }
-  }
-}
-
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC2_THREADS, 1)
 k_typed_linear_tc3(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                    const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
                    const float* __restrict__ bias, int Kp, int cb_width, int stages,
                    const hgt_lin_group* __restrict__ groups, int n_groups,
-                   const hgt_lin_cblock* __restrict__ cblocks, float* __restrict__ out, Tc2Sched sc, int MCH) {
+                   const hgt_lin_cblock* __restrict__ cblocks, float* __restrict__ out, Tc2Sched sc) {
   constexpr int BNH = 128;              // W columns resident per CTA
   constexpr int BNP = 256;              // columns per pair step
   constexpr int BMP = 256;              // rows per pair step
@@ -762,13 +487,12 @@ k_typed_linear_tc3(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
   const int pair_id = blockIdx.x >> 1;
   const int n_pairs = gridDim.x >> 1;
   const int total_units = sc.first_unit[n_groups];
-  const bool strong = !(sc.epi & 2);
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a_hi) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a_lo) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w_hi) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w_lo) : "memory");
+    prefetch_map(&map_a_hi);
+    prefetch_map(&map_a_lo);
+    prefetch_map(&map_w_hi);
+    prefetch_map(&map_w_lo);
     for (int s = 0; s < stages; ++s) {
       mbar_init(s_u32(&a_full[s]), 1);
       mbar_init(s_u32(&a_empty[s]), 1);
@@ -779,19 +503,16 @@ k_typed_linear_tc3(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
       mbar_init(s_u32(&t_full[b]), 1);
       mbar_init(s_u32(&t_empty[b]), 2 * TC2_EPI_WARPS);              // epilogue warps of both CTAs (used in the leader)
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   __syncthreads();
   cluster_sync_all();                                                // both CTAs' barriers exist before any remote arrive
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_ptr_smem)),
-                 "r"(512u)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tmem_alloc<2>(s_u32(tmem_ptr_smem), 512u);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
 
   struct Unit { int64_t pm_first; int n_pm; int a_row0; int w_row; int64_t m_rows; int64_t out_off; int64_t ld; int n0;
@@ -808,8 +529,8 @@ k_typed_linear_tc3(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
     const int nt = col - cb * sc.n_tiles_n;
     const hgt_lin_cblock cblk = cblocks[grp.cb_first + cb];
     const int64_t pm_total = (grp.m + BMP - 1) / BMP;
-    un.pm_first = (int64_t)chunk * MCH;
-    un.n_pm = (int)min((int64_t)MCH, pm_total - un.pm_first);
+    un.pm_first = (int64_t)chunk * TC2_MCH;
+    un.n_pm = (int)min((int64_t)TC2_MCH, pm_total - un.pm_first);
     un.a_row0 = (int)grp.a_row0;
     un.m_rows = grp.m;
     un.n0 = nt * BNP;
@@ -826,7 +547,7 @@ k_typed_linear_tc3(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
       for (int u = pair_id; u < total_units; u += n_pairs, ++unit_it) {
         Unit un;
         decode(u, un);
-        mbar_wait_cluster(s_u32(w_empty), (unit_it & 1u) ^ 1u, strong);
+        mbar_wait(s_u32(w_empty), (unit_it & 1u) ^ 1u);
         if (leader) mbar_expect_tx(s_u32(w_full), 2u * (uint32_t)k_blocks * 2 * b_bytes);
         const int w_row = un.w_row + (int)cta * BNH;
         for (int kb = 0; kb < k_blocks; ++kb) {
@@ -837,7 +558,7 @@ k_typed_linear_tc3(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
           const int a_row = un.a_row0 + (int)((un.pm_first + pm) * BMP) + (int)cta * TC_BM;
           for (int j = 0; j < 2 * k_blocks; ++j, ++a_it) {
             const int s = a_it % stages;
-            mbar_wait_cluster(s_u32(&a_empty[s]), ((a_it / stages) & 1u) ^ 1u, strong);
+            mbar_wait(s_u32(&a_empty[s]), ((a_it / stages) & 1u) ^ 1u);
             const uint32_t bar = s_u32(&a_full[s]);
             if (leader) mbar_expect_tx(bar, 2u * a_bytes);
             tma_load_2d_2sm(s_u32(a_smem + (size_t)s * a_bytes), (j & 1) ? &map_a_lo : &map_a_hi, (j >> 1) * TC_BK,
@@ -849,27 +570,26 @@ k_typed_linear_tc3(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
   } else if (warp == 1) {
     if (lane == 0 && leader) {
       // ===== MMA issuer (leader CTA only) =====
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BNP >> 3) << 17) |
-                             ((uint32_t)(BMP >> 4) << 24);
+      const uint32_t idesc = idesc_bf16(BMP, BNP, false, false);
       uint32_t a_it = 0, unit_it = 0, acc_it = 0;
       for (int u = pair_id; u < total_units; u += n_pairs, ++unit_it) {
         Unit un;
         decode(u, un);
-        mbar_wait_cluster(s_u32(w_full), unit_it & 1u, strong);
+        mbar_wait(s_u32(w_full), unit_it & 1u);
         for (int pm = 0; pm < un.n_pm; ++pm, ++acc_it) {
           const uint32_t buf = acc_it & 1u;
-          mbar_wait_cluster(s_u32(&t_empty[buf]), ((acc_it >> 1) & 1u) ^ 1u, strong);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          mbar_wait(s_u32(&t_empty[buf]), ((acc_it >> 1) & 1u) ^ 1u);
+          tc_fence_after();
           const uint32_t tmem_d = tmem_base + buf * (uint32_t)BNP;
           for (int j = 0; j < 2 * k_blocks; ++j, ++a_it) {
             const int s = a_it % stages;
             const int kb = j >> 1;
-            mbar_wait_cluster(s_u32(&a_full[s]), (a_it / stages) & 1u, strong);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const uint64_t d_a = make_sw128_desc(s_u32(a_smem + (size_t)s * a_bytes));
-            const uint64_t d_whi = make_sw128_desc(s_u32(w_smem + (size_t)(2 * kb) * b_bytes));
+            mbar_wait(s_u32(&a_full[s]), (a_it / stages) & 1u);
+            tc_fence_after();
+            const uint64_t d_a = desc_k_sw128(s_u32(a_smem + (size_t)s * a_bytes));
+            const uint64_t d_whi = desc_k_sw128(s_u32(w_smem + (size_t)(2 * kb) * b_bytes));
             if (!(j & 1)) {
-              const uint64_t d_wlo = make_sw128_desc(s_u32(w_smem + (size_t)(2 * kb + 1) * b_bytes));
+              const uint64_t d_wlo = desc_k_sw128(s_u32(w_smem + (size_t)(2 * kb + 1) * b_bytes));
 #pragma unroll
               for (int k = 0; k < TC_BK / UMMA_K; ++k) {
                 const uint64_t o = (uint64_t)(2 * k);
@@ -905,62 +625,29 @@ k_typed_linear_tc3(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
       asm volatile("bar.sync 1, 256;" ::: "memory");
       for (int pm = 0; pm < un.n_pm; ++pm, ++acc_it) {
         const uint32_t buf = acc_it & 1u;
-        mbar_wait_cluster(s_u32(&t_full[buf]), (acc_it >> 1) & 1u, strong);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        mbar_wait(s_u32(&t_full[buf]), (acc_it >> 1) & 1u);
+        tc_fence_after();
         const int64_t m0 = (un.pm_first + pm) * BMP + (int64_t)cta * TC_BM + lg * 32;
-        if (sc.epi & 4)
-          tc_epilogue_tile_direct(tmem_base + ((uint32_t)(lg * 32) << 16) + buf * (uint32_t)BNP, BNP, e >> 2, s_bias,
-                                  out + un.out_off + m0 * un.ld + un.n0, un.ld, un.m_rows - m0, lane);
-        else if (sc.epi & 1)
-          tc_epilogue_tile_pf(tmem_base + ((uint32_t)(lg * 32) << 16) + buf * (uint32_t)BNP, BNP, e >> 2, stg, s_bias,
-                              out + un.out_off + m0 * un.ld + un.n0, un.ld, un.m_rows - m0, lane);
-        else
-          tc_epilogue_tile(tmem_base + ((uint32_t)(lg * 32) << 16) + buf * (uint32_t)BNP, BNP, e >> 2, stg, s_bias,
-                           out + un.out_off + m0 * un.ld + un.n0, un.ld, un.m_rows - m0, lane);
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_epilogue_tile_pf(tmem_base + ((uint32_t)(lg * 32) << 16) + buf * (uint32_t)BNP, BNP, e >> 2, stg, s_bias,
+                            out + un.out_off + m0 * un.ld + un.n0, un.ld, un.m_rows - m0, lane);
+        tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive_cta(s_u32(&t_empty[buf]), 0, strong);      // the leader's barrier collects both CTAs
+        if (lane == 0) mbar_arrive_cta(s_u32(&t_empty[buf]), 0);      // the leader's barrier collects both CTAs
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   cluster_sync_all();                                                // peer may still be reading our W through the MMA
   if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    tmem_dealloc<2>(tmem_base, 512u);
   }
 }
 
 // ---- host side ------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn) return fn;
-  void* p = nullptr;
-  cudaDriverEntryPointQueryResult q;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-      q != cudaDriverEntryPointSuccess)
-    return nullptr;
-  fn = reinterpret_cast<EncodeTiledFn>(p);
-  return fn;
-}
-
+// operand [rows, Kp] bf16, box {TC_BK columns, box_rows rows}
 int make_map(CUtensorMap* m, const void* base, int64_t rows, int Kp, int box_rows) {
-  EncodeTiledFn fn = get_encode_fn();
-  HGT_REQUIRE(fn != nullptr, "hgt_typed_linear: cuTensorMapEncodeTiled not available from the driver");
-  cuuint64_t dims[2] = {(cuuint64_t)Kp, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)Kp * 2};
-  cuuint32_t box[2] = {(cuuint32_t)TC_BK, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  HGT_REQUIRE(r == CUDA_SUCCESS, "hgt_typed_linear: cuTensorMapEncodeTiled failed (%d) rows=%lld Kp=%d box=%d",
-              (int)r, (long long)rows, Kp, box_rows);
-  return 0;
+  return hgt_make_tma_map_bf16(m, base, rows, Kp, Kp, box_rows);
 }
 
 int pick_bn(int cb_width) {
@@ -980,10 +667,23 @@ void extents(const hgt_lin_group* h_groups, int n_groups, int cb_width, int64_t*
   }
 }
 
-}  // namespace
+// Unit prefix of the persistent kernels: per group, chunks of TC2_MCH steps of `step_rows` rows x column tasks.
+int tc2_schedule(const hgt_lin_group* h_groups, int n_groups, int step_rows, int n_tiles_n, Tc2Sched* sc,
+                 int64_t* units) {
+  sc->n_tiles_n = n_tiles_n;
+  int64_t u = 0;
+  for (int g = 0; g < n_groups; ++g) {
+    sc->first_unit[g] = (int32_t)u;
+    const int64_t steps = (h_groups[g].m + step_rows - 1) / step_rows;
+    u += (steps + TC2_MCH - 1) / TC2_MCH * h_groups[g].n_cblocks * n_tiles_n;
+    HGT_REQUIRE(u < 2147483647ll, "hgt_typed_linear(tc): too many units");
+  }
+  sc->first_unit[n_groups] = (int32_t)u;
+  *units = u;
+  return 0;
+}
 
-static const bool g_tc_no_pair = [] { const char* e = getenv("HGT_TC_NO_PAIR"); return e && e[0] == '1'; }();
-static const bool g_tc_tile_per_cta = [] { const char* e = getenv("HGT_TC_TILE_PER_CTA"); return e && e[0] == '1'; }();
+}  // namespace
 
 bool hgt_typed_linear_tc_supported(int64_t lda, int32_t K, int32_t cb_width) {
   (void)lda;
@@ -1057,47 +757,29 @@ static int tc_run(const float* A, int64_t lda, const __nv_bfloat16* a_hi_in, con
   __nv_bfloat16* a_lo = reinterpret_cast<__nv_bfloat16*>(p); p += hgt_align_up((size_t)a_rows * Kp * 2, 256);
   __nv_bfloat16* w_hi = reinterpret_cast<__nv_bfloat16*>(p); p += hgt_align_up((size_t)w_rows * Kp * 2, 256);
   __nv_bfloat16* w_lo = reinterpret_cast<__nv_bfloat16*>(p);
-  {
-    int64_t n = a_rows * (Kp / 4);
-    if (a_hi_in) {
-      a_hi = const_cast<__nv_bfloat16*>(a_hi_in);            // split by the producer (e.g. the edge kernel)
-      a_lo = const_cast<__nv_bfloat16*>(a_lo_in);
-    } else if (n > 0) {
-      k_split_bf16<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(A, lda, a_rows, K, Kp, a_hi, a_lo);
-      HGT_LAUNCH_CHECK();
-    }
-    n = w_rows * (Kp / 4);
-    if (n > 0) k_split_bf16<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(W, K, w_rows, K, Kp, w_hi, w_lo);
-    HGT_LAUNCH_CHECK();
-  }
-  CUtensorMap m_a_hi, m_a_lo, m_w_hi, m_w_lo;
   int rc;
+  if (a_hi_in) {
+    a_hi = const_cast<__nv_bfloat16*>(a_hi_in);              // split by the producer (e.g. the edge kernel)
+    a_lo = const_cast<__nv_bfloat16*>(a_lo_in);
+  } else if ((rc = hgt_act_split_launch(A, lda, a_rows, K, Kp, 0, nullptr, a_hi, a_lo, st))) {
+    return rc;
+  }
+  if ((rc = hgt_act_split_launch(W, K, w_rows, K, Kp, 0, nullptr, w_hi, w_lo, st))) return rc;
+  CUtensorMap m_a_hi, m_a_lo, m_w_hi, m_w_lo;
   if ((rc = make_map(&m_a_hi, a_hi, a_rows, Kp, TC_BM))) return rc;
   if ((rc = make_map(&m_a_lo, a_lo, a_rows, Kp, TC_BM))) return rc;
-  if ((rc = make_map(&m_w_hi, w_hi, w_rows, Kp, BN))) return rc;
-  if ((rc = make_map(&m_w_lo, w_lo, w_rows, Kp, BN))) return rc;
 
   const int k_blocks = (Kp + TC_BK - 1) / TC_BK;
-  if (!g_tc_tile_per_cta && !g_tc_no_pair && cb_width % 256 == 0) {
+  const size_t a_stage = (size_t)TC_BM * TC_BK * 2;
+  if (cb_width % 256 == 0) {
     // ---- 2-CTA kernel: 128 W columns resident per CTA, pair tile 256 x 256 ----
     const size_t w_region = (size_t)k_blocks * 2 * 128 * TC_BK * 2;
-    const size_t a_stage = (size_t)TC_BM * TC_BK * 2;
     const size_t misc = 1024 + 256 + 256 * 4 + 64 + TC2_STAGE_BYTES + 1024;
     if (w_region + misc + 4 * a_stage <= 227 * 1024) {
-      int stages = (int)((227 * 1024 - w_region - misc) / a_stage);
-      if (stages > tc2_stage_cap()) stages = tc2_stage_cap();
+      const int stages = min((int)((227 * 1024 - w_region - misc) / a_stage), TC2_STAGE_CAP);
       Tc2Sched sc;
-      const int mch = tc2_mch();
-      sc.n_tiles_n = cb_width / 256;
-      sc.epi = tc2_epi();
-      int64_t units = 0;
-      for (int g = 0; g < n_groups; ++g) {
-        sc.first_unit[g] = (int32_t)units;
-        int64_t pm = (h_groups[g].m + 255) / 256;
-        units += (pm + mch - 1) / mch * h_groups[g].n_cblocks * sc.n_tiles_n;
-        HGT_REQUIRE(units < 2147483647ll, "hgt_typed_linear(tc): too many units");
-      }
-      sc.first_unit[n_groups] = (int32_t)units;
+      int64_t units;
+      if ((rc = tc2_schedule(h_groups, n_groups, 256, cb_width / 256, &sc, &units))) return rc;
       if (units == 0) return 0;
       if ((rc = make_map(&m_w_hi, w_hi, w_rows, Kp, 128))) return rc;
       if ((rc = make_map(&m_w_lo, w_lo, w_rows, Kp, 128))) return rc;
@@ -1107,60 +789,38 @@ static int tc_run(const float* A, int64_t lda, const __nv_bfloat16* a_hi_in, con
       if (pairs > units) pairs = (int)units;
       HGT_CHECK_CUDA(cudaFuncSetAttribute(k_typed_linear_tc3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       k_typed_linear_tc3<<<2 * pairs, TC2_THREADS, smem, st>>>(m_a_hi, m_a_lo, m_w_hi, m_w_lo, bias, Kp, cb_width,
-                                                               stages, groups, n_groups, cblocks, out, sc, mch);
+                                                               stages, groups, n_groups, cblocks, out, sc);
       HGT_LAUNCH_CHECK();
       return 0;
     }
   }
-  if (!g_tc_tile_per_cta) {
-    // ---- W-stationary persistent kernel ----
-    // widest n-tile whose resident W (all K, hi + lo) still leaves room for >= 4 A stages of 16 KB
-    const size_t a_stage = (size_t)TC_BM * TC_BK * 2;
-    int bn = 0, stages = 0;
-    size_t w_region = 0;
-    for (int c = 128; c >= 16; c -= 16) {
-      if (cb_width % c) continue;
-      const size_t wr = (size_t)k_blocks * 2 * (((size_t)c * TC_BK * 2 + 1023) & ~(size_t)1023);
-      const size_t misc = 1024 + 256 + (size_t)c * 4 + 64 + TC2_STAGE_BYTES + 1024;
-      if (wr + misc + 4 * a_stage > 227 * 1024) continue;
-      bn = c;
-      w_region = wr;
-      stages = (int)((227 * 1024 - wr - misc) / a_stage);
-      break;
-    }
-    if (bn > 0) {
-      if (stages > tc2_stage_cap()) stages = tc2_stage_cap();
-      if (stages >= 2) {
-        Tc2Sched sc;
-        const int mch = tc2_mch();
-        sc.n_tiles_n = cb_width / bn;
-        sc.epi = tc2_epi();
-        int64_t units = 0;
-        for (int g = 0; g < n_groups; ++g) {
-          sc.first_unit[g] = (int32_t)units;
-          int64_t mt = (h_groups[g].m + TC_BM - 1) / TC_BM;
-          units += (mt + mch - 1) / mch * h_groups[g].n_cblocks * sc.n_tiles_n;
-          HGT_REQUIRE(units < 2147483647ll, "hgt_typed_linear(tc): too many units");
-        }
-        sc.first_unit[n_groups] = (int32_t)units;
-        if (units == 0) return 0;
-        if ((rc = make_map(&m_w_hi, w_hi, w_rows, Kp, bn))) return rc;
-        if ((rc = make_map(&m_w_lo, w_lo, w_rows, Kp, bn))) return rc;
-        int tmem_cols = 32;
-        while (tmem_cols < 2 * bn) tmem_cols <<= 1;
-        size_t smem = 1024 + w_region + (size_t)stages * a_stage + (2 * stages + 6) * 8 + 16 + (size_t)bn * 4 + 64 +
-                      TC2_STAGE_BYTES;
-        HGT_CHECK_CUDA(cudaFuncSetAttribute(k_typed_linear_tc2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int grid = hgt_sm_count();
-        if (grid > units) grid = (int)units;
-        k_typed_linear_tc2<<<grid, TC2_THREADS, smem, st>>>(m_a_hi, m_a_lo, m_w_hi, m_w_lo, bias, Kp, cb_width, bn,
-                                                            stages, tmem_cols, groups, n_groups, cblocks, out, sc, mch);
-        HGT_LAUNCH_CHECK();
-        return 0;
-      }
-    }
+  // ---- W-stationary persistent kernel ----
+  // widest n-tile whose resident W (all K, hi + lo) still leaves room for >= 4 A stages of 16 KB
+  for (int bn = 128; bn >= 16; bn -= 16) {
+    if (cb_width % bn) continue;
+    const size_t w_region = (size_t)k_blocks * 2 * (((size_t)bn * TC_BK * 2 + 1023) & ~(size_t)1023);
+    const size_t misc = 1024 + 256 + (size_t)bn * 4 + 64 + TC2_STAGE_BYTES + 1024;
+    if (w_region + misc + 4 * a_stage > 227 * 1024) continue;
+    const int stages = min((int)((227 * 1024 - w_region - misc) / a_stage), TC2_STAGE_CAP);
+    Tc2Sched sc;
+    int64_t units;
+    if ((rc = tc2_schedule(h_groups, n_groups, TC_BM, cb_width / bn, &sc, &units))) return rc;
+    if (units == 0) return 0;
+    if ((rc = make_map(&m_w_hi, w_hi, w_rows, Kp, bn))) return rc;
+    if ((rc = make_map(&m_w_lo, w_lo, w_rows, Kp, bn))) return rc;
+    int tmem_cols = 32;
+    while (tmem_cols < 2 * bn) tmem_cols <<= 1;
+    size_t smem = 1024 + w_region + (size_t)stages * a_stage + (2 * stages + 6) * 8 + 16 + (size_t)bn * 4 + 64 +
+                  TC2_STAGE_BYTES;
+    HGT_CHECK_CUDA(cudaFuncSetAttribute(k_typed_linear_tc2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int grid = hgt_sm_count();
+    if (grid > units) grid = (int)units;
+    k_typed_linear_tc2<<<grid, TC2_THREADS, smem, st>>>(m_a_hi, m_a_lo, m_w_hi, m_w_lo, bias, Kp, cb_width, bn,
+                                                        stages, tmem_cols, groups, n_groups, cblocks, out, sc);
+    HGT_LAUNCH_CHECK();
+    return 0;
   }
-  // ---- one tile per CTA (fallback for very wide K; HGT_TC_TILE_PER_CTA=1 forces it) ----
+  // ---- one tile per CTA: no resident W fits (Kp > 2240, i.e. more than 35 k-blocks even at n-tile 16) ----
   TcTilePrefix tp;
   tp.n_tiles_n = cb_width / BN;
   int64_t total = 0;
@@ -1171,6 +831,8 @@ static int tc_run(const float* A, int64_t lda, const __nv_bfloat16* a_hi_in, con
   }
   tp.first_tile[n_groups] = (int32_t)total;
   if (total == 0) return 0;
+  if ((rc = make_map(&m_w_hi, w_hi, w_rows, Kp, BN))) return rc;
+  if ((rc = make_map(&m_w_lo, w_lo, w_rows, Kp, BN))) return rc;
 
   const uint32_t a_bytes = TC_BM * TC_BK * 2;
   const uint32_t b_bytes_al = ((uint32_t)BN * TC_BK * 2 + 1023) & ~1023u;

@@ -309,14 +309,7 @@ k_halo_pull_split(const float* const* __restrict__ peers, const int32_t* __restr
         if (c < vec_per_row) {
           if (owner[b] == self_rank) out_f32[r * vec_per_row + c] = v[b][i];
           const float f[4] = {v[b][i].x, v[b][i].y, v[b][i].z, v[b][i].w};
-          __nv_bfloat16 h[4], l[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            h[j] = __float2bfloat16_rn(f[j]);
-            l[j] = __float2bfloat16_rn(f[j] - __bfloat162float(h[j]));
-          }
-          hi[r * vec_per_row + c] = *reinterpret_cast<uint2*>(h);
-          lo[r * vec_per_row + c] = *reinterpret_cast<uint2*>(l);
+          hgt_split_bf16x4(f, &hi[r * vec_per_row + c], &lo[r * vec_per_row + c]);
         }
       }
     }
@@ -354,14 +347,7 @@ k_halo_push_split(const float4* __restrict__ x_own, const int32_t* __restrict__ 
       if (c < vec_per_row) {
         if (peer == self_rank) x_local_f32[drow * vec_per_row + c] = v[k];
         const float f[4] = {v[k].x, v[k].y, v[k].z, v[k].w};
-        __nv_bfloat16 h[4], l[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          h[j] = __float2bfloat16_rn(f[j]);
-          l[j] = __float2bfloat16_rn(f[j] - __bfloat162float(h[j]));
-        }
-        hi[c] = *reinterpret_cast<uint2*>(h);
-        lo[c] = *reinterpret_cast<uint2*>(l);
+        hgt_split_bf16x4(f, hi + c, lo + c);
       }
     }
   }

@@ -78,14 +78,7 @@ k_update_epilogue(const float* __restrict__ o, const float* __restrict__ x, cons
 // The next layer's projection GEMM consumes its input as a bf16 hi/lo split: emit it here instead of re-reading `out`.
 __device__ __forceinline__ void split_store(uint2* hi, uint2* lo, int64_t idx, const float4& v) {
   const float f[4] = {v.x, v.y, v.z, v.w};
-  __nv_bfloat16 h[4], l[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    h[j] = __float2bfloat16_rn(f[j]);
-    l[j] = __float2bfloat16_rn(f[j] - __bfloat162float(h[j]));
-  }
-  hi[idx] = *reinterpret_cast<uint2*>(h);
-  lo[idx] = *reinterpret_cast<uint2*>(l);
+  hgt_split_bf16x4(f, hi + idx, lo + idx);
 }
 
 // Vectorised variant: d % 4 == 0, each lane owns NV float4 chunks (chunk c = lane + 32*i), 128-bit loads/stores.

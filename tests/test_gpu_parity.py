@@ -571,30 +571,39 @@ def test_full_size_c5_16m_sampled_rows_including_hubs():
 
 
 def test_typed_linear_more_groups_than_one_launch_holds():
-    """Schemas with > 64 <type, relation> groups (ADVICE r1): the entry point launches in chunks."""
+    """Schemas with > 64 <type, relation> groups (ADVICE r1): the entry point launches in chunks.  The second shape,
+    K = 2304, leaves no room for a resident W tile, so the tensor-core path takes the one-tile-per-CTA kernel."""
     import ctypes
+    import re
+    from torch.profiler import profile, ProfilerActivity
     from pyhgt_b200 import _lib, plan as P
     dev = _dev()
-    K, width, n_g, m = 64, 32, 70, 37
-    gen = torch.Generator().manual_seed(0)
-    A = torch.randn(n_g * m, K, generator=gen)
-    W = torch.randn(n_g * width, K, generator=gen)
-    b = torch.randn(n_g * width, generator=gen)
-    groups = [(i * m, m, i * width, 1, i, 1) for i in range(n_g)]
-    cblocks = [(i * m * width, width) for i in range(n_g)]
-    for impl in (1, 2):
-        tab = P._pack_groups(groups, cblocks, dev)
-        out = torch.zeros(n_g * m * width, device=dev)
-        wsb = ctypes.c_size_t()
-        _lib.call("hgt_typed_linear_workspace_bytes", tab[1].ctypes.data, n_g, K, width, impl, ctypes.byref(wsb))
-        ws = torch.empty(max(wsb.value, 1), dtype=torch.uint8, device=dev)
-        Ad, Wd, bd = A.to(dev), W.to(dev), b.to(dev)
-        _lib.call("hgt_typed_linear", Ad.data_ptr(), K, Wd.data_ptr(), bd.data_ptr(), K, width, tab[0].data_ptr(),
-                  tab[1].ctypes.data, n_g, tab[3].data_ptr(), out.data_ptr(), impl, ws.data_ptr(), ws.numel(),
-                  torch.cuda.current_stream().cuda_stream)
-        ref = torch.stack([A[i * m:(i + 1) * m].double() @ W[i * width:(i + 1) * width].double().t()
-                           + b[i * width:(i + 1) * width].double() for i in range(n_g)]).float()
-        _close(out.view(n_g, m, width), ref, "typed linear, 70 groups, impl %d" % impl)
+    for K, width, n_g, m in ((64, 32, 70, 37), (2304, 256, 2, 300)):
+        gen = torch.Generator().manual_seed(0)
+        A = torch.randn(n_g * m, K, generator=gen)
+        W = torch.randn(n_g * width, K, generator=gen)
+        b = torch.randn(n_g * width, generator=gen)
+        groups = [(i * m, m, i * width, 1, i, 1) for i in range(n_g)]
+        cblocks = [(i * m * width, width) for i in range(n_g)]
+        for impl in (1, 2):
+            tab = P._pack_groups(groups, cblocks, dev)
+            out = torch.zeros(n_g * m * width, device=dev)
+            wsb = ctypes.c_size_t()
+            _lib.call("hgt_typed_linear_workspace_bytes", tab[1].ctypes.data, n_g, K, width, impl, ctypes.byref(wsb))
+            ws = torch.empty(max(wsb.value, 1), dtype=torch.uint8, device=dev)
+            Ad, Wd, bd = A.to(dev), W.to(dev), b.to(dev)
+            torch.cuda.synchronize()
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                _lib.call("hgt_typed_linear", Ad.data_ptr(), K, Wd.data_ptr(), bd.data_ptr(), K, width,
+                          tab[0].data_ptr(), tab[1].ctypes.data, n_g, tab[3].data_ptr(), out.data_ptr(), impl,
+                          ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream)
+                torch.cuda.synchronize()
+            ref = torch.stack([A[i * m:(i + 1) * m].double() @ W[i * width:(i + 1) * width].double().t()
+                               + b[i * width:(i + 1) * width].double() for i in range(n_g)]).float()
+            _close(out.view(n_g, m, width), ref, "typed linear, K=%d, %d groups, impl %d" % (K, n_g, impl))
+            if impl == 2 and K > 2240:
+                names = [e.key for e in prof.key_averages()]
+                assert any(re.search(r"k_typed_linear_tc(?![23])", n) for n in names), names
 
 
 def test_backward_two_graphs_same_pairs_no_stale_tables():
