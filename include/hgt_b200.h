@@ -231,6 +231,46 @@ int hgt_edge_backward(const float* q, const float* kv, const float* kvr, const f
                       const int32_t* d_tile_counts, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Deterministic backward (the path pyhgt_b200 takes under torch.use_deterministic_algorithms(True)).
+ * Same results as the default backward up to the order of floating-point sums, but every sum runs in an order fixed
+ * by the problem shape: no floating-point atomics, and no partitioning that depends on the card.  Two runs on the same
+ * inputs give the same bits.  Each *_det call takes its non-det sibling's arguments plus a workspace sized by its
+ * *_workspace_bytes query; none allocates or synchronises.
+ * ---------------------------------------------------------------------------------------------- */
+
+/* Stable group-by: ptr [n_keys+1] = exclusive prefix of the key histogram; pos [n] = the positions i of key[i] grouped
+ * by key, increasing inside each group (stable radix sort).  Keys must lie in [0, n_keys). */
+int hgt_plan_group_by_workspace_bytes(int64_t n, int32_t n_keys, size_t* out_bytes);
+int hgt_plan_group_by(const int32_t* key, int64_t n, int32_t n_keys, int32_t* ptr, int32_t* pos, void* workspace,
+                      size_t workspace_bytes, void* stream);
+/* csr_dst [n_edges]: the destination (rank) of every position of the destination-sorted CSR row_ptr [n_nodes+1]. */
+int hgt_plan_csr_dst(const int32_t* row_ptr, int64_t n_nodes, int64_t n_edges, int32_t* csr_dst, void* stream);
+
+/* One edge index for the deterministic edge backward: segments ptr [n_keys+1] over the CSR positions pos (pos NULL:
+ * the positions themselves, i.e. the destination CSR), cut into tiles / hubs by hgt_plan_tiles over ptr.  n_tiles,
+ * n_split, n_hubs: exact counts, or with d_counts (hgt_plan_tiles' sync-free mode) the bounds the arrays were sized with. */
+typedef struct {
+  const int32_t* ptr;
+  const int32_t* pos;
+  const int32_t* tiles;
+  const int32_t* hubs;
+  const int32_t* d_counts;
+  int32_t n_tiles, n_split, n_hubs, reserved;
+} hgt_tile_set;
+
+/* Deterministic hgt_edge_backward.  dst: the destination CSR (row_ptr, tiles / hubs of the forward); src: the CSR
+ * positions grouped by kv_row (n_keys = kv_rows_total, trailing zero row included); rte: grouped by rte_row
+ * (n_keys = P*240+1), or NULL without RTE.  csr_dst from hgt_plan_csr_dst.  Every row of dq [N,d], dkv [kv_rows_total,2d]
+ * and dkvr [P*240+1,2d] is written (rows without edges as zeros): no zero-initialisation is needed. */
+int hgt_edge_backward_det_workspace_bytes(int64_t n_nodes, int32_t d, int32_t n_heads, const hgt_tile_set* dst,
+                                          const hgt_tile_set* src, const hgt_tile_set* rte, size_t* out_bytes);
+int hgt_edge_backward_det(const float* q, const float* kv, const float* kvr, const float* agg, const float* dagg,
+                          const float* stats, const int32_t* kv_row, const int32_t* rte_row, const int32_t* csr_dst,
+                          const hgt_tile_set* dst, const hgt_tile_set* src, const hgt_tile_set* rte, int64_t n_nodes,
+                          int32_t d, int32_t n_heads, float* dq, float* dkv, float* dkvr, void* workspace,
+                          size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Backward of the typed linears (training path).  For the group / column-block tables of the forward call:
  *   dA[a_row0_g + m, k]             = sum_c sum_n dOut_c[m, n] * W[w_row0_g + c*cb_width + n, k]   (* gelu'(gelu_aux) if given)
  *   dW[w_row0_g + c*cb_width + n,k] += sum_m dOut_c[m, n] * A[a_row0_g + m, k]
@@ -254,6 +294,19 @@ int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, const void* dou
                          float* dA, int32_t accumulate_dA, const float* gelu_aux, float* dW, float* db,
                          int32_t impl, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Deterministic hgt_typed_linear_bwd (same arguments and semantics): partial dW / db tiles go to the workspace and are
+ * summed in chunk order; the SIMT dA walks overlapping groups in group order. */
+int hgt_typed_linear_bwd_det_workspace_bytes(const hgt_lin_group* h_groups, int32_t n_groups,
+                                             const hgt_lin_cblock* h_cblocks, int32_t K, int32_t cb_width, int64_t lda,
+                                             int64_t dout_elems, int32_t have_dout_split, int32_t have_a_split,
+                                             int32_t impl, size_t* out_bytes);
+int hgt_typed_linear_bwd_det(const float* dout, const void* dout_hi, const void* dout_lo, int64_t dout_elems,
+                             const float* A, int64_t lda, const void* a_hi, const void* a_lo,
+                             const float* W, int32_t K, int32_t cb_width, const hgt_lin_group* groups,
+                             const hgt_lin_group* h_groups, int32_t n_groups, const hgt_lin_cblock* h_cblocks,
+                             float* dA, int32_t accumulate_dA, const float* gelu_aux, float* dW, float* db,
+                             int32_t impl, void* workspace, size_t workspace_bytes, void* stream);
+
 /* act(in) as fp32 (out_f32 [rows, K], or NULL) and/or as the bf16 hi/lo operand split (hi/lo [rows, K], or NULL; needs
  * K % 8 == 0).  act: 0 = identity, 1 = exact-erf gelu (conv.py:119).  The training forward keeps the split for the
  * backward pass (it is the A operand of the dW product). */
@@ -269,6 +322,13 @@ int hgt_update_backward(const float* dout, const float* o, const float* x, const
                         const float* skip, const float* norm_w, const int32_t* perm, const int32_t* type_active,
                         int64_t n_nodes, int32_t d,
                         float* d_o, float* d_x, float* d_skip, float* d_norm_w, float* d_norm_b, void* stream);
+/* Deterministic hgt_update_backward: per-warp partial sums of d skip / d norm in the workspace, summed in row order. */
+int hgt_update_backward_det_workspace_bytes(int64_t n_nodes, int32_t num_types, int32_t d, size_t* out_bytes);
+int hgt_update_backward_det(const float* dout, const float* o, const float* x, const int32_t* type_row0,
+                            int32_t num_types, const float* skip, const float* norm_w, const int32_t* perm,
+                            const int32_t* type_active, int64_t n_nodes, int32_t d, float* d_o, float* d_x,
+                            float* d_skip, float* d_norm_w, float* d_norm_b, void* workspace, size_t workspace_bytes,
+                            void* stream);
 
 /* Backward of hgt_fold_weights for the K'/V' blocks: from d W_cat / d b_cat to the gradients of k_linears / v_linears
  * (stacked [T, d_out, d_in] / [T, d_out]) and relation_att / relation_msg [R,H,dk,dk], relation_pri [R,H]; all outputs
@@ -279,6 +339,15 @@ int hgt_fold_backward(const float* d_w_cat, const float* d_b_cat, const float* c
                       int32_t n_heads, int32_t d_in, int32_t d_out, int32_t n_pairs, const int32_t* pair_type,
                       const int32_t* pair_rel, const int32_t* cat_row0, float* d_wk, float* d_bk, float* d_wv,
                       float* d_bv, float* d_att, float* d_msg, float* d_pri, void* stream);
+/* Deterministic hgt_fold_backward: each type (relation) sums its pairs in pair order. */
+int hgt_fold_backward_det_workspace_bytes(int32_t num_relations, int32_t n_heads, int32_t d_out, size_t* out_bytes);
+int hgt_fold_backward_det(const float* d_w_cat, const float* d_b_cat, const float* const* wk, const float* const* bk,
+                          const float* const* wv, const float* const* bv, const float* relation_att,
+                          const float* relation_msg, const float* relation_pri, int32_t num_types,
+                          int32_t num_relations, int32_t n_heads, int32_t d_in, int32_t d_out, int32_t n_pairs,
+                          const int32_t* pair_type, const int32_t* pair_rel, const int32_t* cat_row0, float* d_wk,
+                          float* d_bk, float* d_wv, float* d_bv, float* d_att, float* d_msg, float* d_pri,
+                          void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Update epilogue (conv.py:129-133): y = o*sigmoid(skip[t]) + x*(1-sigmoid(skip[t])); LayerNorm_t(y)

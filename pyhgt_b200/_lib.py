@@ -51,7 +51,29 @@ SIGNATURES = {
     "hgt_conv_workspace_bytes": [_p, _c.POINTER(_sz)],
     "hgt_conv_forward": [_p, _p, _sz, _p],
     "hgt_update_epilogue": [_p, _p, _p, _i32, _p, _p, _p, _p, _p, _i64, _i32, _p, _p, _p, _p],
+    # deterministic backward (torch.use_deterministic_algorithms)
+    "hgt_plan_group_by_workspace_bytes": [_i64, _i32, _c.POINTER(_sz)],
+    "hgt_plan_group_by": [_p, _i64, _i32, _p, _p, _p, _sz, _p],
+    "hgt_plan_csr_dst": [_p, _i64, _i64, _p, _p],
+    "hgt_edge_backward_det_workspace_bytes": [_i64, _i32, _i32, _p, _p, _p, _c.POINTER(_sz)],
+    "hgt_edge_backward_det": [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _i32, _i32, _p, _p, _p, _p, _sz, _p],
+    "hgt_typed_linear_bwd_det_workspace_bytes": [_p, _i32, _p, _i32, _i32, _i64, _i64, _i32, _i32, _i32,
+                                                 _c.POINTER(_sz)],
+    "hgt_typed_linear_bwd_det": [_p, _p, _p, _i64, _p, _i64, _p, _p, _p, _i32, _i32, _p, _p, _i32, _p, _p, _i32, _p, _p,
+                                 _p, _i32, _p, _sz, _p],
+    "hgt_update_backward_det_workspace_bytes": [_i64, _i32, _i32, _c.POINTER(_sz)],
+    "hgt_update_backward_det": [_p, _p, _p, _p, _i32, _p, _p, _p, _p, _i64, _i32, _p, _p, _p, _p, _p, _p, _sz, _p],
+    "hgt_fold_backward_det_workspace_bytes": [_i32, _i32, _i32, _c.POINTER(_sz)],
+    "hgt_fold_backward_det": [_p, _p, _p, _p, _p, _p, _p, _p, _p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p,
+                              _p, _p, _p, _p, _p, _p, _sz, _p],
 }
+
+
+class TileSet(ctypes.Structure):
+    """Mirror of `hgt_tile_set` (include/hgt_b200.h): one edge index of the deterministic edge backward."""
+    _fields_ = [("ptr", ctypes.c_void_p), ("pos", ctypes.c_void_p), ("tiles", ctypes.c_void_p),
+                ("hubs", ctypes.c_void_p), ("d_counts", ctypes.c_void_p), ("n_tiles", ctypes.c_int32),
+                ("n_split", ctypes.c_int32), ("n_hubs", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 class ConvArgs(ctypes.Structure):
     """Mirror of `hgt_conv_args` (include/hgt_b200.h); field order and types must match the C struct exactly

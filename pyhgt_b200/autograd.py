@@ -11,6 +11,11 @@ Every stage is a custom autograd.Function whose forward AND backward are hand-wr
     _EdgeAttention   hgt_edge_forward / hgt_edge_backward        score -> softmax by destination -> weighted aggregation
     _UpdateEpilogue  hgt_update_epilogue / hgt_update_backward   sigmoid(skip) gate + LayerNorm (conv.py:129-133)
 
+Under ``torch.use_deterministic_algorithms(True)`` (read when a backward runs, like PyTorch's own ops) every backward
+stage takes its ``*_det`` entry point instead: the same gradients up to summation order, with every sum in an order fixed
+by the problem shape (no floating-point atomics), so the gradient bits repeat from run to run.  The edge backward then
+runs source-major over an index built on first use and cached on the plan (plan.det_index).
+
 No per-edge intermediates are kept: the edge backward recomputes the softmax weights from the saved per-destination
 (max, sum); the typed linears keep the bf16 hi/lo split of their input (the A operand of the dW product).  No cuBLAS,
 no torch matmul on this path.  Gradients reach ``node_inp`` and every parameter of conv.py:28-54 including ``emb.*``.
@@ -27,6 +32,22 @@ from . import plan as _plan
 
 def _stream():
     return torch.cuda.current_stream().cuda_stream
+
+
+def _det():
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def _det_scratch(nbytes, dev):
+    """Workspace of a *_det call.  Those calls write every scratch byte before reading it, so the NaN fill torch gives
+    torch.empty under deterministic mode (fill_uninitialized_memory) would only cost a pass over it."""
+    det_mod = torch.utils.deterministic
+    fill = det_mod.fill_uninitialized_memory
+    det_mod.fill_uninitialized_memory = False
+    try:
+        return torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+    finally:
+        det_mod.fill_uninitialized_memory = fill
 
 
 def _tc_shape_ok(K, width):
@@ -90,12 +111,13 @@ class _TypedLinear(torch.autograd.Function):
         dw = torch.zeros_like(w_cat)                                   # small: [sum of out rows, K]
         db = torch.zeros(w_cat.shape[0], dtype=torch.float32, device=dev) if ctx.has_bias else None
         impl = 2 if ctx.use_tc else 1
+        fn = "hgt_typed_linear_bwd_det" if _det() else "hgt_typed_linear_bwd"
         a_f32 = a_act if a_act is not None else a                      # SIMT dW operand (act already applied)
         # tables whose groups overlap in rows (sharded per-pair compaction) come with disjoint sub-tables: the first call
         # writes dA, the others accumulate into it; dW / db accumulate anyway
         tables = getattr(ctx.table, "bwd_tables", None) or [ctx.table]
         if not ctx.use_tc:
-            tables = [ctx.table]                                       # the SIMT dX uses atomics: overlap is fine
+            tables = [ctx.table]                                       # the SIMT dX adds up overlapping groups itself
         if need_da:
             # hgt_typed_linear_bwd zeroes the gaps between the first table's groups; rows past its last group (other
             # sub-tables' rows, nodes of unknown type) are zeroed here
@@ -107,10 +129,11 @@ class _TypedLinear(torch.autograd.Function):
             g_dev, g_host, n_g, _ = tab
             c_host = tab.c_host
             wsb = ctypes.c_size_t()
-            _lib.call("hgt_typed_linear_bwd_workspace_bytes", g_host.ctypes.data, n_g, c_host.ctypes.data, K, width, K,
+            _lib.call(fn + "_workspace_bytes", g_host.ctypes.data, n_g, c_host.ctypes.data, K, width, K,
                       ctx.out_elems, 0, int(hi is not None), impl, ctypes.byref(wsb))
-            ws = torch.empty(max(wsb.value, 1), dtype=torch.uint8, device=dev)
-            _lib.call("hgt_typed_linear_bwd", dout.data_ptr(), None, None, ctx.out_elems, _lib.ptr(a_f32), K, _lib.ptr(hi),
+            ws = (_det_scratch(wsb.value, dev) if fn.endswith("_det") else
+                  torch.empty(max(wsb.value, 1), dtype=torch.uint8, device=dev))
+            _lib.call(fn, dout.data_ptr(), None, None, ctx.out_elems, _lib.ptr(a_f32), K, _lib.ptr(hi),
                       _lib.ptr(lo), w_cat.data_ptr(), K, width, g_dev.data_ptr(), g_host.ctypes.data, n_g,
                       c_host.ctypes.data, _lib.ptr(da), int(ti > 0), a.data_ptr() if ctx.act else None, dw.data_ptr(),
                       _lib.ptr(db), impl, ws.data_ptr(), ws.numel(), _stream())
@@ -161,8 +184,21 @@ class _EdgeAttention(torch.autograd.Function):
         dq = dproj[lt.q_off:lt.q_off + N * d]
         dkv = dproj[lt.kv_off:]
         dkvr = torch.empty_like(kvr) if kvr is not None else None
-        ws = torch.empty(256, dtype=torch.uint8, device=proj.device)
         dagg = dagg.contiguous()
+        if _det():
+            # every row of dq / dkv / dkvr is written by the call: no zero fill
+            csr_dst, dst, src, rte = _plan.det_index(plan, kvr is not None)
+            wsb = ctypes.c_size_t()
+            _lib.call("hgt_edge_backward_det_workspace_bytes", N, d, H, ctypes.byref(dst.c), ctypes.byref(src.c),
+                      None if rte is None else ctypes.byref(rte.c), ctypes.byref(wsb))
+            ws = _det_scratch(wsb.value, proj.device)
+            _lib.call("hgt_edge_backward_det", q.data_ptr(), kv.data_ptr(), _lib.ptr(kvr), agg.data_ptr(),
+                      dagg.data_ptr(), stats.data_ptr(), plan.kv_row.data_ptr(),
+                      None if kvr is None else plan.rte_row.data_ptr(), csr_dst.data_ptr(), ctypes.byref(dst.c),
+                      ctypes.byref(src.c), None if rte is None else ctypes.byref(rte.c), N, d, H, dq.data_ptr(),
+                      dkv.data_ptr(), _lib.ptr(dkvr), ws.data_ptr(), ws.numel(), _stream())
+            return dproj, dkvr, None, None, None, None, None, None
+        ws = torch.empty(256, dtype=torch.uint8, device=proj.device)
         _lib.call("hgt_edge_backward", q.data_ptr(), kv.data_ptr(), _lib.ptr(kvr), agg.data_ptr(), dagg.data_ptr(),
                   stats.data_ptr(), plan.row_ptr.data_ptr(), plan.kv_row.data_ptr(),
                   None if kvr is None else plan.rte_row.data_ptr(), plan.tiles.data_ptr(), plan.n_tiles, N, d, H,
@@ -204,11 +240,18 @@ class _FoldWeights(torch.autograd.Function):
         d_bk, d_bv = torch.empty((T, d), **f32), torch.empty((T, d), **f32)
         d_att, d_msg = torch.empty((R, H, dk, dk), **f32), torch.empty((R, H, dk, dk), **f32)
         d_pri = torch.empty((R, H), **f32)
-        _lib.call("hgt_fold_backward", dw_cat.data_ptr(), db_cat.data_ptr(), tabs[2].data_ptr(), tabs[3].data_ptr(),
-                  tabs[4].data_ptr(), tabs[5].data_ptr(), m.relation_att.data_ptr(), m.relation_msg.data_ptr(),
-                  m.relation_pri.data_ptr(), T, R, H, d_in, d, plan.n_pairs, plan.pair_type_dev.data_ptr(),
-                  plan.pair_rel_dev.data_ptr(), lt.cat_row0_dev.data_ptr(), d_wk.data_ptr(), d_bk.data_ptr(),
-                  d_wv.data_ptr(), d_bv.data_ptr(), d_att.data_ptr(), d_msg.data_ptr(), d_pri.data_ptr(), _stream())
+        args = (dw_cat.data_ptr(), db_cat.data_ptr(), tabs[2].data_ptr(), tabs[3].data_ptr(),
+                tabs[4].data_ptr(), tabs[5].data_ptr(), m.relation_att.data_ptr(), m.relation_msg.data_ptr(),
+                m.relation_pri.data_ptr(), T, R, H, d_in, d, plan.n_pairs, plan.pair_type_dev.data_ptr(),
+                plan.pair_rel_dev.data_ptr(), lt.cat_row0_dev.data_ptr(), d_wk.data_ptr(), d_bk.data_ptr(),
+                d_wv.data_ptr(), d_bv.data_ptr(), d_att.data_ptr(), d_msg.data_ptr(), d_pri.data_ptr())
+        if _det():
+            wsb = ctypes.c_size_t()
+            _lib.call("hgt_fold_backward_det_workspace_bytes", R, H, d, ctypes.byref(wsb))
+            ws = _det_scratch(wsb.value, dev)
+            _lib.call("hgt_fold_backward_det", *args, ws.data_ptr(), ws.numel(), _stream())
+        else:
+            _lib.call("hgt_fold_backward", *args, _stream())
         # W_q / b_q rows of W_cat are plain copies: their gradient is the matching slice
         d_wq = [dw_cat[lt.q_row0[t]:lt.q_row0[t] + d] for t in range(T)]
         d_bq = [db_cat[lt.q_row0[t]:lt.q_row0[t] + d] for t in range(T)]
@@ -246,9 +289,16 @@ class _UpdateEpilogue(torch.autograd.Function):
         d_skip = torch.empty(T, dtype=torch.float32, device=dev) if ctx.has_skip else None
         d_nw = torch.empty((T, d), dtype=torch.float32, device=dev) if ctx.has_norm else None
         d_nb = torch.empty((T, d), dtype=torch.float32, device=dev) if ctx.has_norm else None
-        _lib.call("hgt_update_backward", dout.data_ptr(), o.data_ptr(), x.data_ptr(), type_row0.data_ptr(), T,
-                  _lib.ptr(skip), _lib.ptr(norm_w), _lib.ptr(perm), _lib.ptr(type_active), N, d, d_o.data_ptr(),
-                  d_x.data_ptr(), _lib.ptr(d_skip), _lib.ptr(d_nw), _lib.ptr(d_nb), _stream())
+        args = (dout.data_ptr(), o.data_ptr(), x.data_ptr(), type_row0.data_ptr(), T,
+                _lib.ptr(skip), _lib.ptr(norm_w), _lib.ptr(perm), _lib.ptr(type_active), N, d, d_o.data_ptr(),
+                d_x.data_ptr(), _lib.ptr(d_skip), _lib.ptr(d_nw), _lib.ptr(d_nb))
+        if _det():
+            wsb = ctypes.c_size_t()
+            _lib.call("hgt_update_backward_det_workspace_bytes", N, T, d, ctypes.byref(wsb))
+            ws = _det_scratch(wsb.value, dev)
+            _lib.call("hgt_update_backward_det", *args, ws.data_ptr(), ws.numel(), _stream())
+        else:
+            _lib.call("hgt_update_backward", *args, _stream())
         return d_o, d_x, d_skip, d_nw, d_nb, None, None, None, None
 
 

@@ -61,3 +61,20 @@ unsigned long long g_hgt_launches = 0;
 extern "C" uint64_t hgt_kernel_launches(void) { return g_hgt_launches; }
 extern "C" const char* hgt_last_error(void) { return g_err; }
 extern "C" int hgt_abi_version(void) { return 2; }
+
+__global__ void k_ordered_sum(const float* __restrict__ part, const hgt_sum_seg* __restrict__ segs, int64_t n,
+                              float* __restrict__ dst) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const hgt_sum_seg s = segs[blockIdx.y];
+  dst[s.dst + i] += hgt_chunk_sum(part + s.part + i, s.chunks, n);
+}
+
+int hgt_ordered_sum_launch(const float* part, const hgt_sum_seg* segs, int n_segs, int64_t n, float* dst,
+                           cudaStream_t st) {
+  if (n_segs == 0 || n == 0) return 0;
+  HGT_REQUIRE(n_segs <= 65535, "hgt_ordered_sum_launch: %d segments exceed the grid limit", n_segs);
+  k_ordered_sum<<<dim3((unsigned)((n + 255) / 256), (unsigned)n_segs), 256, 0, st>>>(part, segs, n, dst);
+  HGT_LAUNCH_CHECK();
+  return 0;
+}

@@ -58,3 +58,20 @@ __device__ __forceinline__ void hgt_split_bf16x4(const float (&v)[4], uint2* hi,
   *hi = *reinterpret_cast<uint2*>(h);
   *lo = *reinterpret_cast<uint2*>(l);
 }
+
+// ---- ordered reductions (deterministic backward, torch.use_deterministic_algorithms) ------------------------------------
+// Partial results of a reduction are written to [chunks, stride] scratch and summed in chunk order, so the bits of the
+// result depend only on the problem shape, never on which CTA finished first.
+__device__ __forceinline__ float hgt_chunk_sum(const float* part, int chunks, int64_t stride) {
+  float s = 0.f;
+  for (int c = 0; c < chunks; ++c) s += part[(int64_t)c * stride];
+  return s;
+}
+// One segment of hgt_ordered_sum_launch: dst[dst + i] += sum_{c < chunks} part[part + c * n + i]  (i < n).
+struct hgt_sum_seg {
+  int64_t part, dst;
+  int32_t chunks, pad;
+};
+// segs: device array of n_segs segments (all of width n).
+int hgt_ordered_sum_launch(const float* part, const hgt_sum_seg* segs, int n_segs, int64_t n, float* dst,
+                           cudaStream_t st);

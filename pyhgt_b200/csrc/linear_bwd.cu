@@ -107,10 +107,12 @@ struct GcTask {            // one (group, column block)
 
 // One CTA = one task x SPLIT_ROWS rows.  Thread (cx, ry): float4 column cx*4, rows ry, ry+RY, ...; column sums are reduced
 // across ry in shared memory and added to db with one atomic per column and CTA.
+// DET: the CTA's column sums go to db_part[unit][width] instead (summed in unit order by hgt_ordered_sum_launch).
 constexpr int SPLIT_ROWS = 256;
-__global__ void __launch_bounds__(256)
-k_split_colsum(const float* __restrict__ dout, const GcTask* __restrict__ tasks, int n_tasks, int width,
-               __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo, float* __restrict__ db) {
+template <bool DET>
+__device__ __forceinline__ void split_colsum_body(const float* __restrict__ dout, const GcTask* __restrict__ tasks,
+                                                  int n_tasks, int width, __nv_bfloat16* __restrict__ hi,
+                                                  __nv_bfloat16* __restrict__ lo, float* __restrict__ db) {
   __shared__ float red[256 * 4];
   int unit = blockIdx.x, t = 0;
   while (t + 1 < n_tasks && unit >= tasks[t + 1].first_unit) ++t;
@@ -143,12 +145,23 @@ k_split_colsum(const float* __restrict__ dout, const GcTask* __restrict__ tasks,
         for (int j = 0; j < 4; ++j) {
           float a = 0.f;
           for (int y = 0; y < ryn; ++y) a += red[(y * cxn + cx) * 4 + j];
-          atomicAdd(db + tk.w_row + c0 * 4 + j, a);
+          if (DET) db[(int64_t)unit * width + c0 * 4 + j] = a;
+          else atomicAdd(db + tk.w_row + c0 * 4 + j, a);
         }
       }
       __syncthreads();
     }
   }
+}
+__global__ void __launch_bounds__(256)
+k_split_colsum(const float* __restrict__ dout, const GcTask* __restrict__ tasks, int n_tasks, int width,
+               __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo, float* __restrict__ db) {
+  split_colsum_body<false>(dout, tasks, n_tasks, width, hi, lo, db);
+}
+__global__ void __launch_bounds__(256)
+k_det_split_colsum(const float* __restrict__ dout, const GcTask* __restrict__ tasks, int n_tasks, int width,
+                   __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo, float* __restrict__ db_part) {
+  split_colsum_body<true>(dout, tasks, n_tasks, width, hi, lo, db_part);
 }
 
 // ---- dX: dA tile = sum over (column block, k-block) of dOut tile x W^T tile --------------------------------------------
@@ -292,9 +305,12 @@ k_lin_dx_tc(const CUtensorMap* __restrict__ maps, int map_wt, const GcTask* __re
 }
 
 // ---- dW: [128 rows of the column block] x [BN columns of K_in] += dOut_c^T A over a chunk of rows ---------------------
-__global__ void __launch_bounds__(BW_THREADS, 1)
-k_lin_dw_tc(const CUtensorMap* __restrict__ maps, const GcTask* __restrict__ tasks, int n_tasks, int K_in, int width,
-            int m_tiles, int n_tiles, int chunk_rows, float* __restrict__ dW) {
+// DET: the tile is stored to dW_part[global chunk][width][K_in] (global chunk = first_unit / (m_tiles * n_tiles) + chunk)
+// and the chunks are summed in order afterwards.
+template <bool DET>
+__device__ __forceinline__ void lin_dw_tc_body(const CUtensorMap* __restrict__ maps, const GcTask* __restrict__ tasks,
+                                               int n_tasks, int K_in, int width, int m_tiles, int n_tiles,
+                                               int chunk_rows, float* __restrict__ dW) {
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = smem_dyn + ((1024u - (s_u32(smem_dyn) & 1023u)) & 1023u);
   constexpr int STAGES = 2;
@@ -395,7 +411,9 @@ k_lin_dw_tc(const CUtensorMap* __restrict__ maps, const GcTask* __restrict__ tas
     mbar_wait(s_u32(tmem_full_bar), 0);
     tc_fence_after();
     const bool row_ok = total_iters > 0 && mt * 128 + row < width;
-    float* wrow = dW + ((int64_t)tk.w_row + mt * 128 + row) * K_in + n0;
+    const int64_t out_row = DET ? ((int64_t)tk.first_unit / (m_tiles * n_tiles) + chunk) * width + mt * 128 + row
+                                : (int64_t)tk.w_row + mt * 128 + row;
+    float* wrow = dW + out_row * K_in + n0;
     for (int c = 0; c < bn; c += 16) {
       uint32_t r[16];
       tmem_ld16(tmem_base + ((uint32_t)(lg * 32) << 16) + (uint32_t)c, r);
@@ -403,9 +421,14 @@ k_lin_dw_tc(const CUtensorMap* __restrict__ maps, const GcTask* __restrict__ tas
       if (row_ok) {
 #pragma unroll
         for (int j = 0; j < 16; j += 4) {
-          asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(wrow + c + j), "f"(__uint_as_float(r[j])),
-                       "f"(__uint_as_float(r[j + 1])), "f"(__uint_as_float(r[j + 2])), "f"(__uint_as_float(r[j + 3]))
-                       : "memory");
+          if (DET) {
+            *reinterpret_cast<float4*>(wrow + c + j) = make_float4(__uint_as_float(r[j]), __uint_as_float(r[j + 1]),
+                                                                   __uint_as_float(r[j + 2]), __uint_as_float(r[j + 3]));
+          } else {
+            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(wrow + c + j), "f"(__uint_as_float(r[j])),
+                         "f"(__uint_as_float(r[j + 1])), "f"(__uint_as_float(r[j + 2])), "f"(__uint_as_float(r[j + 3]))
+                         : "memory");
+          }
         }
       }
     }
@@ -416,10 +439,32 @@ k_lin_dw_tc(const CUtensorMap* __restrict__ maps, const GcTask* __restrict__ tas
     tmem_dealloc<1>(tmem_base, 256u);
   }
 }
+__global__ void __launch_bounds__(BW_THREADS, 1)
+k_lin_dw_tc(const CUtensorMap* __restrict__ maps, const GcTask* __restrict__ tasks, int n_tasks, int K_in, int width,
+            int m_tiles, int n_tiles, int chunk_rows, float* __restrict__ dW) {
+  lin_dw_tc_body<false>(maps, tasks, n_tasks, K_in, width, m_tiles, n_tiles, chunk_rows, dW);
+}
+__global__ void __launch_bounds__(BW_THREADS, 1)
+k_det_lin_dw_tc(const CUtensorMap* __restrict__ maps, const GcTask* __restrict__ tasks, int n_tasks, int K_in,
+                int width, int m_tiles, int n_tiles, int chunk_rows, float* __restrict__ dW_part) {
+  lin_dw_tc_body<true>(maps, tasks, n_tasks, K_in, width, m_tiles, n_tiles, chunk_rows, dW_part);
+}
 
 // ---- SIMT fp32 fallbacks ------------------------------------------------------------------------------------------------
 // dA[a_row0 + m, k] (+)= sum_c sum_n dOut_c[m, n] * W[w_row + n, k].  One thread per (m, k); atomicAdd because groups may
 // share A rows (the RTE tables: every <type, relation> pair projects the same 240-row table).
+__device__ __forceinline__ float lin_dx_term(const float* __restrict__ dout, const float* __restrict__ W,
+                                             const GcTask* __restrict__ tasks, int task0, int n_cblocks, int64_t m,
+                                             int k, int K_in, int width) {
+  float acc = 0.f;
+  for (int c = 0; c < n_cblocks; ++c) {
+    const GcTask tk = tasks[task0 + c];
+    const float* drow = dout + tk.out_off + m * tk.ld;
+    const float* wcol = W + (int64_t)tk.w_row * K_in + k;
+    for (int n = 0; n < width; ++n) acc = fmaf(drow[n], wcol[(int64_t)n * K_in], acc);
+  }
+  return acc;
+}
 __global__ void k_lin_dx_simt(const float* __restrict__ dout, const float* __restrict__ W, const GcTask* __restrict__ tasks,
                               const int32_t* __restrict__ group_task0, const hgt_lin_group* __restrict__ groups,
                               int n_groups, const int64_t* __restrict__ group_first, int K_in, int width,
@@ -432,24 +477,42 @@ __global__ void k_lin_dx_simt(const float* __restrict__ dout, const float* __res
   const int64_t li = i - group_first[g];
   const int64_t m = li / K_in;
   const int k = (int)(li - m * K_in);
-  float acc = 0.f;
-  for (int c = 0; c < grp.n_cblocks; ++c) {
-    const GcTask tk = tasks[group_task0[g] + c];
-    const float* drow = dout + tk.out_off + m * tk.ld;
-    const float* wcol = W + (int64_t)tk.w_row * K_in + k;
-    for (int n = 0; n < width; ++n) acc = fmaf(drow[n], wcol[(int64_t)n * K_in], acc);
-  }
+  float acc = lin_dx_term(dout, W, tasks, group_task0[g], grp.n_cblocks, m, k, K_in, width);
   const int64_t o = (grp.a_row0 + m) * K_in + k;
   if (gelu_aux) acc *= gelu_grad(gelu_aux[o]);
   atomicAdd(dA + o, acc);
 }
+// Deterministic variant: one thread per dA element (row, k) of the first a_rows rows; it walks the groups covering its
+// row in group order and stores once.
+__global__ void k_det_lin_dx_simt(const float* __restrict__ dout, const float* __restrict__ W,
+                                  const GcTask* __restrict__ tasks, const int32_t* __restrict__ group_task0,
+                                  const hgt_lin_group* __restrict__ groups, int n_groups, int64_t a_rows, int K_in,
+                                  int width, const float* __restrict__ gelu_aux, float* __restrict__ dA) {
+  const int64_t o = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (o >= a_rows * K_in) return;
+  const int64_t row = o / K_in;
+  const int k = (int)(o - row * K_in);
+  float acc = dA[o];
+  for (int g = 0; g < n_groups; ++g) {
+    const hgt_lin_group grp = groups[g];
+    if (row < grp.a_row0 || row >= grp.a_row0 + grp.m) continue;
+    float t = lin_dx_term(dout, W, tasks, group_task0[g], grp.n_cblocks, row - grp.a_row0, k, K_in, width);
+    if (gelu_aux) t *= gelu_grad(gelu_aux[o]);
+    acc += t;
+  }
+  dA[o] = acc;
+}
 
 // dW[w_row + n, k] += sum_m dOut_c[m, n] * A[a_row0 + m, k];  db[w_row + n] += sum_m dOut_c[m, n].
 // One CTA = one task x (32 n) x (32 k) x a chunk of rows; 256 threads, 4 outputs each.
+// DET: the tile goes to dW_part[global chunk][width][K_in] and the bias sums to db_part[global chunk][width]
+// (global chunk = first_unit / (n_tiles * k_tiles) + chunk), summed in chunk order afterwards.
 constexpr int DW_SIMT_ROWS = 2048;
-__global__ void __launch_bounds__(256)
-k_lin_dw_simt(const float* __restrict__ dout, const float* __restrict__ A, int64_t lda, const GcTask* __restrict__ tasks,
-              int n_tasks, int K_in, int width, int n_tiles, int k_tiles, float* __restrict__ dW, float* __restrict__ db) {
+template <bool DET>
+__device__ __forceinline__ void lin_dw_simt_body(const float* __restrict__ dout, const float* __restrict__ A, int64_t lda,
+                                                 const GcTask* __restrict__ tasks, int n_tasks, int K_in, int width,
+                                                 int n_tiles, int k_tiles, float* __restrict__ dW,
+                                                 float* __restrict__ db) {
   __shared__ float sd[32][33], sa[32][33];
   int unit = blockIdx.x, t = 0;
   while (t + 1 < n_tasks && unit >= tasks[t + 1].first_unit) ++t;
@@ -488,22 +551,60 @@ k_lin_dw_simt(const float* __restrict__ dout, const float* __restrict__ A, int64
     }
     __syncthreads();
   }
+  const int64_t crow = ((int64_t)tk.first_unit / (n_tiles * k_tiles) + chunk) * width;   // DET: partial row base
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     const int n = n0 + ty + 8 * j;
-    if (n < width && k0 + tx < K_in) atomicAdd(dW + ((int64_t)tk.w_row + n) * K_in + k0 + tx, acc[j]);
+    if (n < width && k0 + tx < K_in) {
+      if (DET) dW[(crow + n) * K_in + k0 + tx] = acc[j];
+      else atomicAdd(dW + ((int64_t)tk.w_row + n) * K_in + k0 + tx, acc[j]);
+    }
   }
-  if (db && tk.has_bias && ktile == 0 && ty == 0 && n0 + tx < width) atomicAdd(db + tk.w_row + n0 + tx, bsum);
+  if (db && tk.has_bias && ktile == 0 && ty == 0 && n0 + tx < width) {
+    if (DET) db[crow + n0 + tx] = bsum;
+    else atomicAdd(db + tk.w_row + n0 + tx, bsum);
+  }
+}
+__global__ void __launch_bounds__(256)
+k_lin_dw_simt(const float* __restrict__ dout, const float* __restrict__ A, int64_t lda, const GcTask* __restrict__ tasks,
+              int n_tasks, int K_in, int width, int n_tiles, int k_tiles, float* __restrict__ dW, float* __restrict__ db) {
+  lin_dw_simt_body<false>(dout, A, lda, tasks, n_tasks, K_in, width, n_tiles, k_tiles, dW, db);
+}
+__global__ void __launch_bounds__(256)
+k_det_lin_dw_simt(const float* __restrict__ dout, const float* __restrict__ A, int64_t lda,
+                  const GcTask* __restrict__ tasks, int n_tasks, int K_in, int width, int n_tiles, int k_tiles,
+                  float* __restrict__ dW_part, float* __restrict__ db_part) {
+  lin_dw_simt_body<true>(dout, A, lda, tasks, n_tasks, K_in, width, n_tiles, k_tiles, dW_part, db_part);
 }
 
 // ---- host helpers ---------------------------------------------------------------------------------------------------------
+// The deterministic path sizes the tensor-core dW chunks as if the card had this many SMs: the chunking decides which
+// partial sums are formed, so it must depend on the problem shape only, not on the card or partition it runs on.
+constexpr int kDetChunkSms = 148;
+
 struct BwdLayout {
-  bool tc;
+  bool tc, det;
   int Kp, wpad;
   int64_t a_rows, w_rows, wt_cols;
   int n_tasks;
-  size_t off_maps, off_tasks, off_gt0, off_gfirst, off_dhi, off_dlo, off_ahi, off_alo, off_wthi, off_wtlo, total;
+  int64_t dw_chunk;          // tensor-core dW reduction chunk (rows)
+  size_t off_maps, off_tasks, off_gt0, off_gfirst, off_dhi, off_dlo, off_ahi, off_alo, off_wthi, off_wtlo;
+  size_t off_wpart, off_bpart, off_segs, total;   // deterministic path: partial sums and their segment tables
 };
+
+int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
+
+// Rows per k_lin_dw_tc work unit: a few waves of CTAs over the whole product.
+int64_t dw_tc_chunk(const hgt_lin_group* h_groups, int n_groups, int K, int width, int sms) {
+  const int m_tiles = (width + 127) / 128, n_tiles = (K + 255) / 256;
+  int64_t work = 0;
+  for (int g = 0; g < n_groups; ++g) work += h_groups[g].m * h_groups[g].n_cblocks * m_tiles * n_tiles;
+  int64_t chunk = work / (4 * (int64_t)sms);
+  chunk = (chunk + BK - 1) / BK * BK;
+  if (chunk < 1024) chunk = 1024;
+  if (chunk > 32768) chunk = 32768;
+  return chunk;
+}
 
 bool groups_overlap(const hgt_lin_group* h, int n) {
   for (int i = 0; i < n; ++i)
@@ -529,8 +630,9 @@ bool bwd_tc_ok(const hgt_lin_group* h_groups, int n_groups, const hgt_lin_cblock
 }
 
 BwdLayout bwd_layout(const hgt_lin_group* h_groups, int n_groups, const hgt_lin_cblock* h_cb, int K, int width,
-                     int64_t lda, int64_t dout_elems, bool have_dsplit, bool have_asplit, int impl) {
+                     int64_t lda, int64_t dout_elems, bool have_dsplit, bool have_asplit, int impl, bool det) {
   BwdLayout L{};
+  L.det = det;
   L.tc = impl == 2 || (impl == 0 && bwd_tc_ok(h_groups, n_groups, h_cb, K, width, lda));
   L.Kp = K;
   L.wpad = (width + BK - 1) / BK * BK;
@@ -557,6 +659,20 @@ BwdLayout bwd_layout(const hgt_lin_group* h_groups, int n_groups, const hgt_lin_
     L.off_wthi = take((size_t)K * L.wt_cols * 2);
     L.off_wtlo = take((size_t)K * L.wt_cols * 2);
   }
+  if (det) {
+    // dW chunks and db units of every task (tensor cores: dW chunks of dw_chunk rows, db units of SPLIT_ROWS rows;
+    // SIMT: both in chunks of DW_SIMT_ROWS rows)
+    L.dw_chunk = L.tc ? dw_tc_chunk(h_groups, n_groups, K, width, kDetChunkSms) : DW_SIMT_ROWS;
+    const int64_t b_rows = L.tc ? SPLIT_ROWS : DW_SIMT_ROWS;
+    int64_t wc = 0, bc = 0;
+    for (int g = 0; g < n_groups; ++g) {
+      wc += h_groups[g].n_cblocks * ceil_div(h_groups[g].m, L.dw_chunk);
+      bc += h_groups[g].n_cblocks * ceil_div(h_groups[g].m, b_rows);
+    }
+    L.off_wpart = take((size_t)wc * width * K * sizeof(float));
+    L.off_bpart = take((size_t)bc * width * sizeof(float));
+    L.off_segs = take((size_t)(2 * L.n_tasks + 1) * sizeof(hgt_sum_seg));
+  }
   L.total = p + 256;
   return L;
 }
@@ -582,31 +698,46 @@ extern "C" int hgt_act_split(const float* in, int64_t ld, int64_t rows, int32_t 
                               reinterpret_cast<__nv_bfloat16*>(lo), (cudaStream_t)stream_);
 }
 
+static int bwd_workspace_bytes(const hgt_lin_group* h_groups, int32_t n_groups, const hgt_lin_cblock* h_cblocks,
+                               int32_t K, int32_t cb_width, int64_t lda, int64_t dout_elems, int32_t have_dout_split,
+                               int32_t have_a_split, int32_t impl, size_t* out_bytes, bool det) {
+  HGT_REQUIRE(out_bytes && (n_groups == 0 || (h_groups && h_cblocks)), "hgt_typed_linear_bwd_workspace_bytes: NULL argument");
+  HGT_REQUIRE(n_groups >= 0 && n_groups <= kMaxGroups, "hgt_typed_linear_bwd: n_groups=%d exceeds %d", n_groups, kMaxGroups);
+  *out_bytes = bwd_layout(h_groups, n_groups, h_cblocks, K, cb_width, lda, dout_elems, have_dout_split != 0,
+                          have_a_split != 0, impl, det).total;
+  return 0;
+}
+
 extern "C" int hgt_typed_linear_bwd_workspace_bytes(const hgt_lin_group* h_groups, int32_t n_groups,
                                                     const hgt_lin_cblock* h_cblocks, int32_t K, int32_t cb_width,
                                                     int64_t lda, int64_t dout_elems, int32_t have_dout_split,
                                                     int32_t have_a_split, int32_t impl, size_t* out_bytes) {
-  HGT_REQUIRE(out_bytes && (n_groups == 0 || (h_groups && h_cblocks)), "hgt_typed_linear_bwd_workspace_bytes: NULL argument");
-  HGT_REQUIRE(n_groups >= 0 && n_groups <= kMaxGroups, "hgt_typed_linear_bwd: n_groups=%d exceeds %d", n_groups, kMaxGroups);
-  *out_bytes = bwd_layout(h_groups, n_groups, h_cblocks, K, cb_width, lda, dout_elems, have_dout_split != 0,
-                          have_a_split != 0, impl).total;
-  return 0;
+  return bwd_workspace_bytes(h_groups, n_groups, h_cblocks, K, cb_width, lda, dout_elems, have_dout_split, have_a_split,
+                             impl, out_bytes, false);
 }
 
-extern "C" int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, const void* dout_lo, int64_t dout_elems,
-                                    const float* A, int64_t lda, const void* a_hi_in, const void* a_lo_in,
-                                    const float* W, int32_t K, int32_t cb_width, const hgt_lin_group* groups,
-                                    const hgt_lin_group* h_groups, int32_t n_groups, const hgt_lin_cblock* h_cblocks,
-                                    float* dA, int32_t accumulate_dA, const float* gelu_aux, float* dW, float* db,
-                                    int32_t impl, void* workspace, size_t workspace_bytes, void* stream_) {
-  cudaStream_t st = (cudaStream_t)stream_;
+extern "C" int hgt_typed_linear_bwd_det_workspace_bytes(const hgt_lin_group* h_groups, int32_t n_groups,
+                                                        const hgt_lin_cblock* h_cblocks, int32_t K, int32_t cb_width,
+                                                        int64_t lda, int64_t dout_elems, int32_t have_dout_split,
+                                                        int32_t have_a_split, int32_t impl, size_t* out_bytes) {
+  return bwd_workspace_bytes(h_groups, n_groups, h_cblocks, K, cb_width, lda, dout_elems, have_dout_split, have_a_split,
+                             impl, out_bytes, true);
+}
+
+static int typed_linear_bwd(const float* dout, const void* dout_hi, const void* dout_lo, int64_t dout_elems,
+                            const float* A, int64_t lda, const void* a_hi_in, const void* a_lo_in, const float* W,
+                            int32_t K, int32_t cb_width, const hgt_lin_group* groups, const hgt_lin_group* h_groups,
+                            int32_t n_groups, const hgt_lin_cblock* h_cblocks, float* dA, int32_t accumulate_dA,
+                            const float* gelu_aux, float* dW, float* db, int32_t impl, void* workspace,
+                            size_t workspace_bytes, cudaStream_t st, bool det) {
   HGT_REQUIRE(n_groups >= 0 && n_groups <= kMaxGroups, "hgt_typed_linear_bwd: n_groups=%d exceeds %d", n_groups, kMaxGroups);
   HGT_REQUIRE(K > 0 && cb_width > 0 && W, "hgt_typed_linear_bwd: K=%d cb_width=%d", K, cb_width);
   if (n_groups == 0) return 0;
   HGT_REQUIRE(groups && h_groups && h_cblocks, "hgt_typed_linear_bwd: NULL group tables");
   const bool have_dsplit = dout_hi && dout_lo, have_asplit = a_hi_in && a_lo_in;
   HGT_REQUIRE(dout || have_dsplit, "hgt_typed_linear_bwd: neither dout nor its bf16 split given");
-  const BwdLayout L = bwd_layout(h_groups, n_groups, h_cblocks, K, cb_width, lda, dout_elems, have_dsplit, have_asplit, impl);
+  const BwdLayout L = bwd_layout(h_groups, n_groups, h_cblocks, K, cb_width, lda, dout_elems, have_dsplit, have_asplit,
+                                impl, det);
   HGT_REQUIRE(workspace && workspace_bytes >= L.total, "hgt_typed_linear_bwd: workspace too small (%zu < %zu)",
               workspace_bytes, L.total);
   if (L.tc)
@@ -661,13 +792,38 @@ extern "C" int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, cons
   HGT_CHECK_CUDA(cudaMemcpyAsync(d_gt0, gt0.data(), gt0.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   HGT_CHECK_CUDA(cudaMemcpyAsync(d_gfirst, gfirst.data(), gfirst.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
   int rc;
+  // deterministic path: partial sums of task t start at chunk first_unit / units_per_chunk; one segment per task
+  float* w_part = det ? reinterpret_cast<float*>(base + L.off_wpart) : nullptr;
+  float* b_part = det ? reinterpret_cast<float*>(base + L.off_bpart) : nullptr;
+  hgt_sum_seg* d_segs = det ? reinterpret_cast<hgt_sum_seg*>(base + L.off_segs) : nullptr;
+  // segs [0, nt): db (tasks with a bias), [nt, 2 nt): dW.  Summed in chunk order into db / dW.
+  auto ordered_sums = [&](bool do_w, bool do_b, int64_t units_per_chunk) -> int {
+    std::vector<hgt_sum_seg> segs(2 * nt + 1);
+    int nb = 0, nw = 0;
+    for (int t = 0; t < nt; ++t) {
+      const int64_t c0 = tasks[t].first_unit / units_per_chunk;
+      if (do_b && tasks[t].has_bias)
+        segs[nb++] = hgt_sum_seg{c0 * cb_width, tasks[t].w_row, tasks[t].n_chunks, 0};
+      if (do_w) segs[nt + nw++] = hgt_sum_seg{c0 * cb_width * K, (int64_t)tasks[t].w_row * K, tasks[t].n_chunks, 0};
+    }
+    HGT_CHECK_CUDA(cudaMemcpyAsync(d_segs, segs.data(), segs.size() * sizeof(hgt_sum_seg), cudaMemcpyHostToDevice, st));
+    int r;
+    if (nb && (r = hgt_ordered_sum_launch(b_part, d_segs, nb, cb_width, db, st))) return r;
+    if (nw && (r = hgt_ordered_sum_launch(w_part, d_segs + nt, nw, (int64_t)cb_width * K, dW, st))) return r;
+    return 0;
+  };
 
   if (!L.tc) {
     // ---------------- SIMT fp32 path ----------------
     if (dA) {
       if (!accumulate_dA) HGT_CHECK_CUDA(cudaMemsetAsync(dA, 0, (size_t)L.a_rows * K * sizeof(float), st));
       if ((rc = upload_tasks())) return rc;
-      if (elems > 0) {
+      if (det && L.a_rows > 0) {
+        k_det_lin_dx_simt<<<(unsigned)((L.a_rows * K + 255) / 256), 256, 0, st>>>(dout, W, d_tasks, d_gt0, groups,
+                                                                                  n_groups, L.a_rows, K, cb_width,
+                                                                                  gelu_aux, dA);
+        HGT_LAUNCH_CHECK();
+      } else if (!det && elems > 0) {
         k_lin_dx_simt<<<(unsigned)((elems + 255) / 256), 256, 0, st>>>(dout, W, d_tasks, d_gt0, groups, n_groups, d_gfirst, K,
                                                                        cb_width, gelu_aux, dA);
         HGT_LAUNCH_CHECK();
@@ -683,7 +839,12 @@ extern "C" int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, cons
         HGT_REQUIRE(units < 2147483647ll, "hgt_typed_linear_bwd: too many units");
       }
       if ((rc = upload_tasks())) return rc;
-      if (units > 0) {
+      if (units > 0 && det) {
+        k_det_lin_dw_simt<<<(unsigned)units, 256, 0, st>>>(dout, A, lda, d_tasks, nt, K, cb_width, n_tiles, k_tiles,
+                                                            w_part, db ? b_part : nullptr);
+        HGT_LAUNCH_CHECK();
+        if ((rc = ordered_sums(true, db != nullptr, (int64_t)n_tiles * k_tiles))) return rc;
+      } else if (units > 0) {
         k_lin_dw_simt<<<(unsigned)units, 256, 0, st>>>(dout, A, lda, d_tasks, nt, K, cb_width, n_tiles, k_tiles, dW, db);
         HGT_LAUNCH_CHECK();
       }
@@ -708,11 +869,16 @@ extern "C" int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, cons
     int64_t units = 0;
     for (int t = 0; t < nt; ++t) {
       tasks[t].first_unit = (int32_t)units;
-      units += (tasks[t].rows + SPLIT_ROWS - 1) / SPLIT_ROWS;
+      tasks[t].n_chunks = (int32_t)((tasks[t].rows + SPLIT_ROWS - 1) / SPLIT_ROWS);
+      units += tasks[t].n_chunks;
       HGT_REQUIRE(units < 2147483647ll, "hgt_typed_linear_bwd: too many units");
     }
     if ((rc = upload_tasks())) return rc;
-    if (units > 0) {
+    if (units > 0 && det) {
+      k_det_split_colsum<<<(unsigned)units, 256, 0, st>>>(dout, d_tasks, nt, cb_width, d_hi, d_lo, db ? b_part : nullptr);
+      HGT_LAUNCH_CHECK();
+      if (db && (rc = ordered_sums(false, true, 1))) return rc;
+    } else if (units > 0) {
       k_split_colsum<<<(unsigned)units, 256, 0, st>>>(dout, d_tasks, nt, cb_width, d_hi, d_lo, db);
       HGT_LAUNCH_CHECK();
     }
@@ -784,13 +950,7 @@ extern "C" int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, cons
   // 6. dW
   if (dW) {
     const int m_tiles = (cb_width + 127) / 128, n_tiles = (K + 255) / 256;
-    // chunk the reduction so that the grid has a few waves of CTAs
-    int64_t work = 0;
-    for (int t = 0; t < nt; ++t) work += tasks[t].rows * m_tiles * n_tiles;
-    int64_t chunk = work / (4 * (int64_t)hgt_sm_count());
-    chunk = (chunk + BK - 1) / BK * BK;
-    if (chunk < 1024) chunk = 1024;
-    if (chunk > 32768) chunk = 32768;
+    const int64_t chunk = det ? L.dw_chunk : dw_tc_chunk(h_groups, n_groups, K, cb_width, hgt_sm_count());
     int64_t units = 0;
     for (int t = 0; t < nt; ++t) {
       tasks[t].first_unit = (int32_t)units;
@@ -804,11 +964,42 @@ extern "C" int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, cons
     if (units > 0) {
       const int n_atoms = std::min(4, (K + 63) / 64);
       const size_t smem = 1024 + 2 * (size_t)(2 * 2 * ATOM_BYTES + 2 * n_atoms * ATOM_BYTES) + 8 * 8 + 16;
-      HGT_CHECK_CUDA(cudaFuncSetAttribute(k_lin_dw_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k_lin_dw_tc<<<(unsigned)units, BW_THREADS, smem, st>>>(d_maps, d_tasks2, nt, K, cb_width, m_tiles, n_tiles, (int)chunk,
-                                                             dW);
-      HGT_LAUNCH_CHECK();
+      if (det) {
+        HGT_CHECK_CUDA(cudaFuncSetAttribute(k_det_lin_dw_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_det_lin_dw_tc<<<(unsigned)units, BW_THREADS, smem, st>>>(d_maps, d_tasks2, nt, K, cb_width, m_tiles, n_tiles,
+                                                                   (int)chunk, w_part);
+        HGT_LAUNCH_CHECK();
+        if ((rc = ordered_sums(true, false, (int64_t)m_tiles * n_tiles))) return rc;
+      } else {
+        HGT_CHECK_CUDA(cudaFuncSetAttribute(k_lin_dw_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_lin_dw_tc<<<(unsigned)units, BW_THREADS, smem, st>>>(d_maps, d_tasks2, nt, K, cb_width, m_tiles, n_tiles,
+                                                               (int)chunk, dW);
+        HGT_LAUNCH_CHECK();
+      }
     }
   }
   return 0;
+}
+
+extern "C" int hgt_typed_linear_bwd(const float* dout, const void* dout_hi, const void* dout_lo, int64_t dout_elems,
+                                    const float* A, int64_t lda, const void* a_hi_in, const void* a_lo_in,
+                                    const float* W, int32_t K, int32_t cb_width, const hgt_lin_group* groups,
+                                    const hgt_lin_group* h_groups, int32_t n_groups, const hgt_lin_cblock* h_cblocks,
+                                    float* dA, int32_t accumulate_dA, const float* gelu_aux, float* dW, float* db,
+                                    int32_t impl, void* workspace, size_t workspace_bytes, void* stream_) {
+  return typed_linear_bwd(dout, dout_hi, dout_lo, dout_elems, A, lda, a_hi_in, a_lo_in, W, K, cb_width, groups, h_groups,
+                          n_groups, h_cblocks, dA, accumulate_dA, gelu_aux, dW, db, impl, workspace, workspace_bytes,
+                          (cudaStream_t)stream_, false);
+}
+
+extern "C" int hgt_typed_linear_bwd_det(const float* dout, const void* dout_hi, const void* dout_lo, int64_t dout_elems,
+                                        const float* A, int64_t lda, const void* a_hi_in, const void* a_lo_in,
+                                        const float* W, int32_t K, int32_t cb_width, const hgt_lin_group* groups,
+                                        const hgt_lin_group* h_groups, int32_t n_groups,
+                                        const hgt_lin_cblock* h_cblocks, float* dA, int32_t accumulate_dA,
+                                        const float* gelu_aux, float* dW, float* db, int32_t impl, void* workspace,
+                                        size_t workspace_bytes, void* stream_) {
+  return typed_linear_bwd(dout, dout_hi, dout_lo, dout_elems, A, lda, a_hi_in, a_lo_in, W, K, cb_width, groups, h_groups,
+                          n_groups, h_cblocks, dA, accumulate_dA, gelu_aux, dW, db, impl, workspace, workspace_bytes,
+                          (cudaStream_t)stream_, true);
 }

@@ -353,9 +353,98 @@ k_halo_push_split(const float4* __restrict__ x_own, const int32_t* __restrict__ 
   }
 }
 
+// ---- group-by (deterministic backward: the source-major index) ---------------------------------------------------------
+__global__ void k_key_hist(const int32_t* __restrict__ key, int64_t n, int32_t* __restrict__ counts,
+                           int32_t* __restrict__ iota) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  atomicAdd(&counts[key[i]], 1);
+  iota[i] = (int32_t)i;
+}
+
+// csr_dst[c] = the destination (rank) whose segment [row_ptr[k], row_ptr[k+1]) holds CSR position c.
+__global__ void k_csr_dst(const int32_t* __restrict__ row_ptr, int64_t n_nodes, int64_t n_edges,
+                          int32_t* __restrict__ csr_dst) {
+  const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (c >= n_edges) return;
+  int64_t lo = 0, hi = n_nodes;                   // last k with row_ptr[k] <= c
+  while (hi - lo > 1) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (row_ptr[mid] <= c) lo = mid;
+    else hi = mid;
+  }
+  csr_dst[c] = (int32_t)lo;
+}
+
+struct GroupScratch {
+  int32_t *keys_out, *iota, *counts;
+  void* cub_tmp;
+  size_t cub_bytes;
+};
+size_t carve_group(GroupScratch& s, void* base, int64_t n, int32_t n_keys) {
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    size_t o = off;
+    off += hgt_align_up(bytes, 256);
+    return base ? (char*)base + o : (char*)nullptr;
+  };
+  s.keys_out = (int32_t*)take(sizeof(int32_t) * (n + 1));
+  s.iota = (int32_t*)take(sizeof(int32_t) * (n + 1));
+  s.counts = (int32_t*)take(sizeof(int32_t) * ((size_t)n_keys + 1));
+  size_t a = cub_sort_bytes(n + 1), b = cub_scan_bytes((int64_t)n_keys + 1);
+  s.cub_bytes = a > b ? a : b;
+  s.cub_tmp = take(s.cub_bytes);
+  return off;
+}
+
 inline unsigned blocks_for(int64_t n) { return (unsigned)((n + kThreads - 1) / kThreads); }
 
 }  // namespace
+
+extern "C" int hgt_plan_group_by_workspace_bytes(int64_t n, int32_t n_keys, size_t* out_bytes) {
+  HGT_REQUIRE(out_bytes && n >= 0 && n < 2147483000ll && n_keys >= 1 && n_keys < 2147483000,
+              "hgt_plan_group_by_workspace_bytes: n=%lld / n_keys=%d outside the int32 index range", (long long)n, n_keys);
+  GroupScratch s;
+  *out_bytes = carve_group(s, nullptr, n, n_keys) + 256;
+  return 0;
+}
+
+extern "C" int hgt_plan_group_by(const int32_t* key, int64_t n, int32_t n_keys, int32_t* ptr, int32_t* pos,
+                                 void* workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t st = (cudaStream_t)stream_;
+  HGT_REQUIRE(ptr && (n == 0 || (key && pos)), "hgt_plan_group_by: NULL argument");
+  size_t need = 0;
+  int rc = hgt_plan_group_by_workspace_bytes(n, n_keys, &need);
+  if (rc) return rc;
+  HGT_REQUIRE(workspace && workspace_bytes >= need, "hgt_plan_group_by: workspace too small (%zu < %zu)",
+              workspace_bytes, need);
+  GroupScratch s;
+  carve_group(s, reinterpret_cast<void*>(hgt_align_up(reinterpret_cast<size_t>(workspace), 256)), n, n_keys);
+  HGT_CHECK_CUDA(cudaMemsetAsync(s.counts, 0, sizeof(int32_t) * ((size_t)n_keys + 1), st));
+  if (n > 0) {
+    k_key_hist<<<blocks_for(n), kThreads, 0, st>>>(key, n, s.counts, s.iota);
+    HGT_LAUNCH_CHECK();
+  }
+  size_t tmp = s.cub_bytes;
+  HGT_CHECK_CUDA(cub::DeviceScan::ExclusiveSum(s.cub_tmp, tmp, (const int32_t*)s.counts, ptr, n_keys + 1, st));
+  if (n > 0) {
+    // LSD radix sort: stable, so each key's positions stay in increasing (CSR) order
+    tmp = s.cub_bytes;
+    HGT_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(s.cub_tmp, tmp, key, s.keys_out, (const int32_t*)s.iota, pos, (int)n,
+                                                   0, bits_for(n_keys > 1 ? n_keys : 2), st));
+  }
+  return 0;
+}
+
+extern "C" int hgt_plan_csr_dst(const int32_t* row_ptr, int64_t n_nodes, int64_t n_edges, int32_t* csr_dst,
+                                void* stream_) {
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (n_edges == 0) return 0;
+  HGT_REQUIRE(row_ptr && csr_dst && n_nodes > 0, "hgt_plan_csr_dst: NULL argument or no nodes");
+  k_csr_dst<<<blocks_for(n_edges), kThreads, 0, st>>>(row_ptr, n_nodes, n_edges, csr_dst);
+  HGT_LAUNCH_CHECK();
+  return 0;
+}
 
 extern "C" int hgt_plan_workspace_bytes(int64_t n_nodes, int64_t n_edges, size_t* out_bytes) {
   HGT_REQUIRE(out_bytes, "hgt_plan_workspace_bytes: out_bytes is NULL");

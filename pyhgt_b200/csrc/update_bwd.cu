@@ -14,14 +14,17 @@ namespace {
 constexpr int UB_WARPS = 8;
 constexpr int UB_ROWS_PER_WARP = 16;
 
-template <int NPL>
-__global__ void __launch_bounds__(UB_WARPS * 32)
-k_update_bwd(const float* __restrict__ dout, const float* __restrict__ o, const float* __restrict__ x,
-             const int32_t* __restrict__ type_row0, int T, const float* __restrict__ skip,
-             const float* __restrict__ norm_w, const int32_t* __restrict__ perm,
-             const int32_t* __restrict__ type_active, int64_t n_nodes, int d,
-             float* __restrict__ d_o, float* __restrict__ d_x, float* __restrict__ d_skip, float* __restrict__ d_nw,
-             float* __restrict__ d_nb) {
+// DET: no atomics; warp w writes its per-type sums [d nw | d nb | d a] to part[(w + t) * (2d + 1)] (a warp's rows span
+// consecutive types, so w + t is unique per (warp, type) and the slots of one type are contiguous in warp order), and
+// k_det_update_reduce sums them in warp order.
+template <int NPL, bool DET>
+__device__ __forceinline__ void update_bwd_body(const float* __restrict__ dout, const float* __restrict__ o,
+                                                const float* __restrict__ x, const int32_t* __restrict__ type_row0,
+                                                int T, const float* __restrict__ skip, const float* __restrict__ norm_w,
+                                                const int32_t* __restrict__ perm, const int32_t* __restrict__ type_active,
+                                                int64_t n_nodes, int d, float* __restrict__ d_o, float* __restrict__ d_x,
+                                                float* __restrict__ d_skip, float* __restrict__ d_nw,
+                                                float* __restrict__ d_nb, float* __restrict__ part) {
   extern __shared__ float s_red[];                  // [2*d + 1] block-level partial sums (uniform-type blocks)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t block_row0 = (int64_t)blockIdx.x * UB_WARPS * UB_ROWS_PER_WARP;
@@ -32,9 +35,11 @@ k_update_bwd(const float* __restrict__ dout, const float* __restrict__ o, const 
     return t;
   };
   const int t_first = type_of(block_row0), t_last = type_of(block_row1 - 1);
-  const bool uniform = t_first == t_last;
-  for (int i = threadIdx.x; i < 2 * d + 1; i += blockDim.x) s_red[i] = 0.f;
-  __syncthreads();
+  const bool uniform = !DET && t_first == t_last;
+  if (!DET) {
+    for (int i = threadIdx.x; i < 2 * d + 1; i += blockDim.x) s_red[i] = 0.f;
+    __syncthreads();
+  }
 
   float acc_w[NPL], acc_b[NPL];
   float acc_a = 0.f;
@@ -50,7 +55,15 @@ k_update_bwd(const float* __restrict__ dout, const float* __restrict__ o, const 
       for (int s = 16; s > 0; s >>= 1) da += __shfl_xor_sync(0xffffffffu, da, s);
       da *= a * (1.0f - a);
     }
-    if (uniform) {
+    if (DET) {
+      float* w = part + ((int64_t)blockIdx.x * UB_WARPS + warp + t) * (2 * d + 1);
+#pragma unroll
+      for (int i = 0; i < NPL; ++i) {
+        const int c = lane + 32 * i;
+        if (c < d) { w[c] = acc_w[i]; w[d + c] = acc_b[i]; }
+      }
+      if (lane == 0) w[2 * d] = da;
+    } else if (uniform) {
       if (lane == 0 && skip) atomicAdd(&s_red[2 * d], da);
       if (norm_w) {
 #pragma unroll
@@ -159,7 +172,7 @@ k_update_bwd(const float* __restrict__ dout, const float* __restrict__ o, const 
     }
   }
   flush(cur_t);
-  if (uniform) {
+  if (!DET && uniform) {
     __syncthreads();
     if (t_first < T) {
       if (norm_w) {
@@ -173,10 +186,67 @@ k_update_bwd(const float* __restrict__ dout, const float* __restrict__ o, const 
   }
 }
 
+template <int NPL>
+__global__ void __launch_bounds__(UB_WARPS * 32)
+k_update_bwd(const float* __restrict__ dout, const float* __restrict__ o, const float* __restrict__ x,
+             const int32_t* __restrict__ type_row0, int T, const float* __restrict__ skip,
+             const float* __restrict__ norm_w, const int32_t* __restrict__ perm,
+             const int32_t* __restrict__ type_active, int64_t n_nodes, int d,
+             float* __restrict__ d_o, float* __restrict__ d_x, float* __restrict__ d_skip, float* __restrict__ d_nw,
+             float* __restrict__ d_nb) {
+  update_bwd_body<NPL, false>(dout, o, x, type_row0, T, skip, norm_w, perm, type_active, n_nodes, d, d_o, d_x, d_skip,
+                              d_nw, d_nb, nullptr);
+}
+template <int NPL>
+__global__ void __launch_bounds__(UB_WARPS * 32)
+k_det_update_bwd(const float* __restrict__ dout, const float* __restrict__ o, const float* __restrict__ x,
+                 const int32_t* __restrict__ type_row0, int T, const float* __restrict__ skip,
+                 const float* __restrict__ norm_w, const int32_t* __restrict__ perm,
+                 const int32_t* __restrict__ type_active, int64_t n_nodes, int d, float* __restrict__ d_o,
+                 float* __restrict__ d_x, float* __restrict__ part) {
+  update_bwd_body<NPL, true>(dout, o, x, type_row0, T, skip, norm_w, perm, type_active, n_nodes, d, d_o, d_x, nullptr,
+                             nullptr, nullptr, part);
+}
+
+// One thread per (type t, column j of [d nw | d nb | d a]): sums the slots of the warps holding rows of t, in warp order.
+__global__ void k_det_update_reduce(const float* __restrict__ part, const int32_t* __restrict__ type_row0, int T, int d,
+                                    const float* __restrict__ skip, float* __restrict__ d_skip,
+                                    float* __restrict__ d_nw, float* __restrict__ d_nb) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  const int W = 2 * d + 1;
+  if (i >= (int64_t)T * W) return;
+  const int t = (int)(i / W), j = (int)(i - (int64_t)t * W);
+  const int64_t r0 = type_row0[t], r1 = type_row0[t + 1];
+  float s = 0.f;
+  if (r1 > r0) {
+    const int64_t w0 = r0 / UB_ROWS_PER_WARP, w1 = (r1 - 1) / UB_ROWS_PER_WARP;
+    s = hgt_chunk_sum(part + (w0 + t) * W + j, (int)(w1 - w0 + 1), W);
+  }
+  if (j < d) { if (d_nw) d_nw[(int64_t)t * d + j] = s; }
+  else if (j < 2 * d) { if (d_nb) d_nb[(int64_t)t * d + j - d] = s; }
+  else if (skip) d_skip[t] = s;
+}
+
 // ---- fold backward -----------------------------------------------------------------------------------------------------
 // Forward (linear.cu k_fold_pairs):  W'[p,which][h*dk+c, col] = s * sum_a rel[r,h,a,c] * W[t][h*dk+a, col]  (col = d_in: bias)
 // with rel = relation_att, s = pri[r,h]/sqrt(dk) for K' (which 0) and rel = relation_msg, s = 1 for V' (which 1).
 // (a) d W[t][h*dk+a, col] += s * sum_c rel[a,c] * G[h*dk+c, col]           one thread per (p, which, row h*dk+a, col)
+__device__ __forceinline__ float fold_w_term(const float* __restrict__ g_w, const float* __restrict__ g_b,
+                                             const float* __restrict__ rel_att, const float* __restrict__ rel_msg,
+                                             const float* __restrict__ rel_pri, int H, int dk, int d_in, int d_out,
+                                             int r, int cat_row0, int which, int row, int col) {
+  const int h = row / dk, a = row - h * dk;
+  const float* rel = (which ? rel_msg : rel_att) + ((int64_t)(r * H + h) * dk) * dk;   // [a][c]
+  const int64_t g_row0 = (int64_t)cat_row0 + which * d_out + h * dk;
+  float acc = 0.f;
+  if (col < d_in) {
+    for (int c = 0; c < dk; ++c) acc = fmaf(rel[a * dk + c], g_w[(g_row0 + c) * d_in + col], acc);
+  } else {
+    for (int c = 0; c < dk; ++c) acc = fmaf(rel[a * dk + c], g_b[g_row0 + c], acc);
+  }
+  if (!which) acc *= rel_pri[r * H + h] * rsqrtf((float)dk);
+  return acc;
+}
 __global__ void k_fold_bwd_w(const float* __restrict__ g_w, const float* __restrict__ g_b,
                              const float* __restrict__ rel_att, const float* __restrict__ rel_msg,
                              const float* __restrict__ rel_pri, int H, int d_in, int d_out, int n_pairs,
@@ -193,24 +263,54 @@ __global__ void k_fold_bwd_w(const float* __restrict__ g_w, const float* __restr
   rem -= which * per_block;
   const int row = (int)(rem / (d_in + 1));
   const int col = (int)(rem - (int64_t)row * (d_in + 1));
-  const int h = row / dk, a = row - h * dk;
-  const int t = pair_type[p], r = pair_rel[p];
-  const float* rel = (which ? rel_msg : rel_att) + ((int64_t)(r * H + h) * dk) * dk;   // [a][c]
-  const int64_t g_row0 = (int64_t)cat_row0[p] + which * d_out + h * dk;
-  float acc = 0.f;
-  if (col < d_in) {
-    for (int c = 0; c < dk; ++c) acc = fmaf(rel[a * dk + c], g_w[(g_row0 + c) * d_in + col], acc);
-  } else {
-    for (int c = 0; c < dk; ++c) acc = fmaf(rel[a * dk + c], g_b[g_row0 + c], acc);
-  }
-  if (!which) acc *= rel_pri[r * H + h] * rsqrtf((float)dk);
+  const int t = pair_type[p];
+  const float acc = fold_w_term(g_w, g_b, rel_att, rel_msg, rel_pri, H, dk, d_in, d_out, pair_rel[p], cat_row0[p], which,
+                                row, col);
   if (col < d_in) atomicAdd((which ? d_wv : d_wk) + ((int64_t)t * d_out + row) * d_in + col, acc);
   else atomicAdd((which ? d_bv : d_bk) + (int64_t)t * d_out + row, acc);
+}
+// Deterministic variant: one thread per (type, which, row, col) walks the pairs of its type in pair order and stores once.
+__global__ void k_det_fold_w(const float* __restrict__ g_w, const float* __restrict__ g_b,
+                             const float* __restrict__ rel_att, const float* __restrict__ rel_msg,
+                             const float* __restrict__ rel_pri, int T, int H, int d_in, int d_out, int n_pairs,
+                             const int32_t* __restrict__ pair_type, const int32_t* __restrict__ pair_rel,
+                             const int32_t* __restrict__ cat_row0, float* __restrict__ d_wk, float* __restrict__ d_bk,
+                             float* __restrict__ d_wv, float* __restrict__ d_bv) {
+  const int dk = d_out / H;
+  const int64_t per_block = (int64_t)d_out * (d_in + 1);
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= per_block * 2 * T) return;
+  const int t = (int)(i / (2 * per_block));
+  int64_t rem = i - (int64_t)t * 2 * per_block;
+  const int which = (int)(rem / per_block);
+  rem -= which * per_block;
+  const int row = (int)(rem / (d_in + 1));
+  const int col = (int)(rem - (int64_t)row * (d_in + 1));
+  float acc = 0.f;
+  for (int p = 0; p < n_pairs; ++p)
+    if (pair_type[p] == t)
+      acc += fold_w_term(g_w, g_b, rel_att, rel_msg, rel_pri, H, dk, d_in, d_out, pair_rel[p], cat_row0[p], which, row, col);
+  if (col < d_in) (which ? d_wv : d_wk)[((int64_t)t * d_out + row) * d_in + col] = acc;
+  else (which ? d_bv : d_bk)[(int64_t)t * d_out + row] = acc;
 }
 
 // (b) val[a,c] = sum_col W[t][h*dk+a, col] * G[h*dk+c, col]  (bias column included);
 //     d rel[r,h,a,c] += s * val;   d pri[r,h] += sum_{a,c} att[a,c] * val / sqrt(dk)   (K' only)
 // One warp per (p, which, h, a, c); lanes split the columns.
+__device__ __forceinline__ float fold_rel_term(const float* __restrict__ g_w, const float* __restrict__ g_b,
+                                               const float* const* __restrict__ wk, const float* const* __restrict__ bk,
+                                               const float* const* __restrict__ wv, const float* const* __restrict__ bv,
+                                               int d_in, int d_out, int dk, int t, int cat_row0, int which, int h, int a,
+                                               int c, int lane) {
+  const float* w = (which ? wv[t] : wk[t]) + (int64_t)(h * dk + a) * d_in;
+  const int64_t g_row = (int64_t)cat_row0 + which * d_out + h * dk + c;
+  const float* g = g_w + g_row * d_in;
+  float val = 0.f;
+  for (int col = lane; col < d_in; col += 32) val = fmaf(w[col], g[col], val);
+  if (lane == 0) val = fmaf((which ? bv[t] : bk[t])[h * dk + a], g_b[g_row], val);
+  for (int s = 16; s > 0; s >>= 1) val += __shfl_xor_sync(0xffffffffu, val, s);
+  return val;
+}
 __global__ void k_fold_bwd_rel(const float* __restrict__ g_w, const float* __restrict__ g_b,
                                const float* const* __restrict__ wk, const float* const* __restrict__ bk,
                                const float* const* __restrict__ wv, const float* const* __restrict__ bv,
@@ -230,14 +330,9 @@ __global__ void k_fold_bwd_rel(const float* __restrict__ g_w, const float* __res
   const int h = (int)(rem / (dk * dk));
   rem -= (int64_t)h * dk * dk;
   const int a = (int)(rem / dk), c = (int)(rem - (int64_t)a * dk);
-  const int t = pair_type[p], r = pair_rel[p];
-  const float* w = (which ? wv[t] : wk[t]) + (int64_t)(h * dk + a) * d_in;
-  const int64_t g_row = (int64_t)cat_row0[p] + which * d_out + h * dk + c;
-  const float* g = g_w + g_row * d_in;
-  float val = 0.f;
-  for (int col = lane; col < d_in; col += 32) val = fmaf(w[col], g[col], val);
-  if (lane == 0) val = fmaf((which ? bv[t] : bk[t])[h * dk + a], g_b[g_row], val);
-  for (int s = 16; s > 0; s >>= 1) val += __shfl_xor_sync(0xffffffffu, val, s);
+  const int r = pair_rel[p];
+  const float val = fold_rel_term(g_w, g_b, wk, bk, wv, bv, d_in, d_out, dk, pair_type[p], cat_row0[p], which, h, a, c,
+                                  lane);
   if (lane == 0) {
     const int64_t ridx = ((int64_t)(r * H + h) * dk + a) * dk + c;
     if (which) {
@@ -246,6 +341,44 @@ __global__ void k_fold_bwd_rel(const float* __restrict__ g_w, const float* __res
       const float inv = rsqrtf((float)dk);
       atomicAdd(d_att + ridx, val * rel_pri[r * H + h] * inv);
       atomicAdd(d_pri + r * H + h, val * rel_att[ridx] * inv);
+    }
+  }
+}
+
+// Deterministic variant: one warp per (relation, which, h, a, c) walks the pairs of its relation in pair order.  d pri
+// needs a further sum over (a, c): each warp stores its term to pri_part[a * dk + c][r * H + h], and the caller sums
+// those dk * dk chunks in order.
+__global__ void k_det_fold_rel(const float* __restrict__ g_w, const float* __restrict__ g_b,
+                               const float* const* __restrict__ wk, const float* const* __restrict__ bk,
+                               const float* const* __restrict__ wv, const float* const* __restrict__ bv,
+                               const float* __restrict__ rel_att, const float* __restrict__ rel_pri, int R, int H,
+                               int d_in, int d_out, int n_pairs, const int32_t* __restrict__ pair_type,
+                               const int32_t* __restrict__ pair_rel, const int32_t* __restrict__ cat_row0,
+                               float* __restrict__ d_att, float* __restrict__ d_msg, float* __restrict__ pri_part) {
+  const int dk = d_out / H;
+  const int lane = threadIdx.x & 31;
+  const int64_t wid = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+  const int64_t per_rel = (int64_t)2 * H * dk * dk;
+  if (wid >= per_rel * R) return;
+  const int r = (int)(wid / per_rel);
+  int64_t rem = wid - (int64_t)r * per_rel;
+  const int which = (int)(rem / ((int64_t)H * dk * dk));
+  rem -= (int64_t)which * H * dk * dk;
+  const int h = (int)(rem / (dk * dk));
+  rem -= (int64_t)h * dk * dk;
+  const int a = (int)(rem / dk), c = (int)(rem - (int64_t)a * dk);
+  float sum = 0.f;
+  for (int p = 0; p < n_pairs; ++p)
+    if (pair_rel[p] == r)
+      sum += fold_rel_term(g_w, g_b, wk, bk, wv, bv, d_in, d_out, dk, pair_type[p], cat_row0[p], which, h, a, c, lane);
+  if (lane == 0) {
+    const int64_t ridx = ((int64_t)(r * H + h) * dk + a) * dk + c;
+    if (which) {
+      d_msg[ridx] = sum;
+    } else {
+      const float inv = rsqrtf((float)dk);
+      d_att[ridx] = sum * rel_pri[r * H + h] * inv;
+      pri_part[((int64_t)a * dk + c) * R * H + r * H + h] = sum * rel_att[ridx] * inv;
     }
   }
 }
@@ -260,6 +393,15 @@ void launch_update_bwd(const float* dout, const float* o, const float* x, const 
   k_update_bwd<NPL><<<grid, UB_WARPS * 32, (2 * d + 1) * sizeof(float), st>>>(dout, o, x, type_row0, T, skip, norm_w, perm,
                                                                              type_active, n, d, d_o, d_x, d_skip, d_nw,
                                                                              d_nb);
+}
+template <int NPL>
+void launch_det_update_bwd(const float* dout, const float* o, const float* x, const int32_t* type_row0, int T,
+                           const float* skip, const float* norm_w, const int32_t* perm, const int32_t* type_active,
+                           int64_t n, int d, float* d_o, float* d_x, float* part, cudaStream_t st) {
+  const int rows_per_block = UB_WARPS * UB_ROWS_PER_WARP;
+  const unsigned grid = (unsigned)((n + rows_per_block - 1) / rows_per_block);
+  k_det_update_bwd<NPL><<<grid, UB_WARPS * 32, 0, st>>>(dout, o, x, type_row0, T, skip, norm_w, perm, type_active, n, d,
+                                                        d_o, d_x, part);
 }
 
 }  // namespace
@@ -328,4 +470,107 @@ extern "C" int hgt_fold_backward(const float* d_w_cat, const float* d_b_cat, con
     HGT_LAUNCH_CHECK();
   }
   return 0;
+}
+
+// Partial sums of the deterministic update backward: one [2d + 1] slot per (warp, type it touches).
+static size_t update_det_part_floats(int64_t n_nodes, int32_t num_types, int32_t d) {
+  const int64_t warps = (n_nodes + UB_WARPS * UB_ROWS_PER_WARP - 1) / (UB_WARPS * UB_ROWS_PER_WARP) * UB_WARPS;
+  return (size_t)(warps + num_types) * (2 * (size_t)d + 1);
+}
+
+extern "C" int hgt_update_backward_det_workspace_bytes(int64_t n_nodes, int32_t num_types, int32_t d,
+                                                       size_t* out_bytes) {
+  HGT_REQUIRE(out_bytes && n_nodes >= 0 && num_types >= 1 && d >= 1, "hgt_update_backward_det_workspace_bytes: bad argument");
+  *out_bytes = update_det_part_floats(n_nodes, num_types, d) * sizeof(float) + 256;
+  return 0;
+}
+
+extern "C" int hgt_update_backward_det(const float* dout, const float* o, const float* x, const int32_t* type_row0,
+                                       int32_t num_types, const float* skip, const float* norm_w, const int32_t* perm,
+                                       const int32_t* type_active, int64_t n_nodes, int32_t d, float* d_o, float* d_x,
+                                       float* d_skip, float* d_norm_w, float* d_norm_b, void* workspace,
+                                       size_t workspace_bytes, void* stream_) {
+  cudaStream_t st = (cudaStream_t)stream_;
+  HGT_REQUIRE(dout && o && x && type_row0 && d_o && d_x && (d_skip || !skip), "hgt_update_backward_det: NULL argument");
+  HGT_REQUIRE(d >= 1 && d <= 1024, "hgt_update_backward_det: d=%d unsupported (max 1024)", d);
+  HGT_REQUIRE(num_types >= 1, "hgt_update_backward_det: num_types=%d", num_types);
+  HGT_REQUIRE(!norm_w || (d_norm_w && d_norm_b), "hgt_update_backward_det: LayerNorm gradients need output buffers");
+  size_t need = 0;
+  hgt_update_backward_det_workspace_bytes(n_nodes, num_types, d, &need);
+  HGT_REQUIRE(workspace && workspace_bytes >= need, "hgt_update_backward_det: workspace too small (%zu < %zu)",
+              workspace_bytes, need);
+  float* part = reinterpret_cast<float*>(hgt_align_up(reinterpret_cast<size_t>(workspace), 256));
+  if (n_nodes > 0) {
+    const int npl = (d + 31) / 32;
+#define HGT_UB(N) launch_det_update_bwd<N>(dout, o, x, type_row0, num_types, skip, norm_w, perm, type_active, n_nodes, d, \
+                                           d_o, d_x, part, st)
+    if (npl <= 2) HGT_UB(2);
+    else if (npl <= 4) HGT_UB(4);
+    else if (npl <= 8) HGT_UB(8);
+    else if (npl <= 16) HGT_UB(16);
+    else HGT_UB(32);
+#undef HGT_UB
+    HGT_LAUNCH_CHECK();
+  }
+  // every (type, column) is written, also for types without rows
+  const int64_t total = (int64_t)num_types * (2 * d + 1);
+  k_det_update_reduce<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(part, type_row0, num_types, d, skip, d_skip,
+                                                                      norm_w ? d_norm_w : nullptr,
+                                                                      norm_w ? d_norm_b : nullptr);
+  HGT_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int hgt_fold_backward_det_workspace_bytes(int32_t num_relations, int32_t n_heads, int32_t d_out,
+                                                     size_t* out_bytes) {
+  HGT_REQUIRE(out_bytes && n_heads > 0 && d_out % n_heads == 0 && num_relations >= 0,
+              "hgt_fold_backward_det_workspace_bytes: bad argument");
+  const size_t dk = d_out / n_heads;
+  *out_bytes = 256 + hgt_align_up((size_t)num_relations * n_heads * dk * dk * sizeof(float), 256) + sizeof(hgt_sum_seg);
+  return 0;
+}
+
+extern "C" int hgt_fold_backward_det(const float* d_w_cat, const float* d_b_cat, const float* const* wk,
+                                     const float* const* bk, const float* const* wv, const float* const* bv,
+                                     const float* relation_att, const float* relation_msg, const float* relation_pri,
+                                     int32_t num_types, int32_t num_relations, int32_t n_heads, int32_t d_in,
+                                     int32_t d_out, int32_t n_pairs, const int32_t* pair_type, const int32_t* pair_rel,
+                                     const int32_t* cat_row0, float* d_wk, float* d_bk, float* d_wv, float* d_bv,
+                                     float* d_att, float* d_msg, float* d_pri, void* workspace, size_t workspace_bytes,
+                                     void* stream_) {
+  cudaStream_t st = (cudaStream_t)stream_;
+  HGT_REQUIRE(n_heads > 0 && d_out % n_heads == 0, "hgt_fold_backward_det: d_out=%d not divisible by n_heads=%d", d_out,
+              n_heads);
+  HGT_REQUIRE(d_wk && d_bk && d_wv && d_bv && d_att && d_msg && d_pri, "hgt_fold_backward_det: NULL output");
+  HGT_REQUIRE(n_pairs == 0 || (d_w_cat && d_b_cat && wk && bk && wv && bv), "hgt_fold_backward_det: NULL input");
+  size_t need = 0;
+  hgt_fold_backward_det_workspace_bytes(num_relations, n_heads, d_out, &need);
+  HGT_REQUIRE(workspace && workspace_bytes >= need, "hgt_fold_backward_det: workspace too small (%zu < %zu)",
+              workspace_bytes, need);
+  const int dk = d_out / n_heads;
+  char* base = reinterpret_cast<char*>(hgt_align_up(reinterpret_cast<size_t>(workspace), 256));
+  float* pri_part = reinterpret_cast<float*>(base);
+  hgt_sum_seg* d_seg = reinterpret_cast<hgt_sum_seg*>(
+      base + hgt_align_up((size_t)num_relations * n_heads * dk * dk * sizeof(float), 256));
+  HGT_CHECK_CUDA(cudaMemsetAsync(d_pri, 0, (size_t)num_relations * n_heads * sizeof(float), st));
+  {
+    const int64_t total = (int64_t)num_types * 2 * d_out * (d_in + 1);
+    if (total > 0) {
+      k_det_fold_w<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(d_w_cat, d_b_cat, relation_att, relation_msg,
+                                                                    relation_pri, num_types, n_heads, d_in, d_out,
+                                                                    n_pairs, pair_type, pair_rel, cat_row0, d_wk, d_bk,
+                                                                    d_wv, d_bv);
+      HGT_LAUNCH_CHECK();
+    }
+  }
+  const int64_t warps = (int64_t)num_relations * 2 * n_heads * dk * dk;
+  if (warps == 0) return 0;
+  k_det_fold_rel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, st>>>(d_w_cat, d_b_cat, wk, bk, wv, bv, relation_att,
+                                                                      relation_pri, num_relations, n_heads, d_in, d_out,
+                                                                      n_pairs, pair_type, pair_rel, cat_row0, d_att,
+                                                                      d_msg, pri_part);
+  HGT_LAUNCH_CHECK();
+  const hgt_sum_seg seg{0, 0, dk * dk, 0};
+  HGT_CHECK_CUDA(cudaMemcpyAsync(d_seg, &seg, sizeof(seg), cudaMemcpyHostToDevice, st));
+  return hgt_ordered_sum_launch(pri_part, d_seg, 1, (int64_t)num_relations * n_heads, d_pri, st);
 }

@@ -61,6 +61,7 @@ class GraphPlan:
     tile_counts_dev: torch.Tensor = None   # sync-free plans: device {n_tiles, n_split, n_hubs}; the host fields are bounds
     flags_dev: torch.Tensor = None         # sync-free plans: range-check flags left on the device (see check())
     _layer_tables: dict = field(default_factory=dict)
+    _det: dict = field(default_factory=dict)  # deterministic backward: source-major indices (det_index)
 
     def check(self):
         """Sync-free plans defer the index range checks: this reads the flags back (one host sync) and raises like
@@ -293,6 +294,60 @@ def build_plan(node_type, edge_index, edge_type, edge_time, num_types, num_relat
                      n_tiles=n_tiles, n_split=n_split, hubs=hubs[:max(n_hubs, 1)], n_hubs=n_hubs,
                      pair_type_dev=pair_type_d, pair_rel_dev=pair_rel_d,
                      tile_counts_dev=n_tiles_d if sync_free else None, flags_dev=flags_d if sync_free else None)
+
+
+# ---- deterministic backward: source-major edge indices -------------------------------------------------------------
+
+class TileIndex:
+    """CSR positions grouped by a key (a [K'|V'] row or an RTE row), with work tiles over the groups.  Keeps the device
+    arrays alive behind the `hgt_tile_set` handed to hgt_edge_backward_det."""
+
+    def __init__(self, ptr, pos, tiles, hubs, counts, n_tiles, n_split, n_hubs):
+        self.tensors = (ptr, pos, tiles, hubs, counts)
+        self.c = _lib.TileSet(_lib.ptr(ptr), _lib.ptr(pos), tiles.data_ptr(), hubs.data_ptr(), _lib.ptr(counts),
+                              n_tiles, n_split, n_hubs, 0)
+
+
+def _group_index(key, E, n_keys, dev):
+    """Group the E CSR positions by key[c] in [0, n_keys) (stable) and tile the groups like the destination CSR.  The
+    tiler runs in its sync-free mode: counts stay on the device and the host fields are the bounds."""
+    st = _stream()
+    i32 = dict(dtype=torch.int32, device=dev)
+    gb, pb = ctypes.c_size_t(), ctypes.c_size_t()
+    _lib.call("hgt_plan_group_by_workspace_bytes", E, n_keys, ctypes.byref(gb))
+    _lib.call("hgt_plan_workspace_bytes", n_keys, E, ctypes.byref(pb))
+    ws = torch.empty(max(gb.value, pb.value), dtype=torch.uint8, device=dev)
+    ptr = torch.empty(n_keys + 1, **i32)
+    pos = torch.empty(max(E, 1), **i32)
+    _lib.call("hgt_plan_group_by", key.data_ptr(), E, n_keys, ptr.data_ptr(), pos.data_ptr(), ws.data_ptr(), ws.numel(),
+              st)
+    max_tiles = (2 * E + n_keys) // (2 * TILE_TARGET_EDGES) + 3 * (E // TILE_SPLIT_EDGES) + 16
+    max_hubs = E // TILE_SPLIT_EDGES + 1
+    tiles = torch.empty((max_tiles, 4), **i32)
+    hubs = torch.empty((max_hubs, 4), **i32)
+    counts = torch.zeros(4, **i32)
+    _lib.call("hgt_plan_tiles", ptr.data_ptr(), n_keys, E, TILE_TARGET_EDGES, TILE_SPLIT_EDGES, tiles.data_ptr(),
+              max_tiles, hubs.data_ptr(), max_hubs, counts.data_ptr(), None, ws.data_ptr(), ws.numel(), st)
+    has_hub = E > TILE_SPLIT_EDGES
+    return TileIndex(ptr, pos, tiles, hubs, counts, max_tiles, 2 * (E // TILE_SPLIT_EDGES) + 1 if has_hub else 0,
+                     max_hubs if has_hub else 0)
+
+
+def det_index(plan, with_rte):
+    """(csr_dst, destination index, [K'|V'] row index, RTE row index or None) for hgt_edge_backward_det, built on the
+    first deterministic backward through this plan and cached on it.  Sync-free: nothing is read back to the host."""
+    d = plan._det
+    dev = plan.row_ptr.device
+    E, N = plan.n_edges, plan.n_nodes
+    if "src" not in d:
+        d["csr_dst"] = torch.empty(max(E, 1), dtype=torch.int32, device=dev)
+        _lib.call("hgt_plan_csr_dst", plan.row_ptr.data_ptr(), N, E, d["csr_dst"].data_ptr(), _stream())
+        d["dst"] = TileIndex(plan.row_ptr, None, plan.tiles, plan.hubs, plan.tile_counts_dev, plan.n_tiles, plan.n_split,
+                             plan.n_hubs)
+        d["src"] = _group_index(plan.kv_row, E, plan.kv_rows + 1, dev)
+    if with_rte and "rte" not in d:
+        d["rte"] = _group_index(plan.rte_row, E, plan.n_pairs * RTE_MAX_LEN + 1, dev)
+    return d["csr_dst"], d["dst"], d["src"], d.get("rte") if with_rte else None
 
 
 # ---- typed-linear descriptor tables (depend on the plan and on the layer's d_in / d_out) -------------
