@@ -187,6 +187,26 @@ int hgt_typed_linear_presplit(const void* a_hi, const void* a_lo, const float* W
                               int32_t n_groups, const hgt_lin_cblock* cblocks, float* out,
                               void* workspace, size_t workspace_bytes, void* stream);
 
+/* bf16-output variants (inference with bf16 [K'|V'] tables): the same product through the same kernels and the same
+ * accumulation order, with the fp32 result (bias included) rounded to nearest even as it is stored.  `out` is bf16 and
+ * cblock offsets / strides count bf16 elements.  The result is bit-identical to the fp32 entry point with the same impl
+ * followed by torch's `.bfloat16()`.  Workspace as for the fp32 entry points.
+ * Alignment: the tensor-core kernels store 8 bf16 (16 bytes) at a time, so on that path (impl 2, or impl 0 choosing it)
+ * `out`, every cblock out_off and ld must be multiples of 8 elements (cb_width % 16 == 0 already holds there); the SIMT
+ * path (impl 1) stores single elements and has no such rule. */
+int hgt_typed_linear_bf16_workspace_bytes(const hgt_lin_group* h_groups, int32_t n_groups, int32_t K,
+                                          int32_t cb_width, int32_t impl, size_t* out_bytes);
+int hgt_typed_linear_bf16(const float* A, int64_t lda, const float* W, const float* bias, int32_t K,
+                          int32_t cb_width, const hgt_lin_group* groups, const hgt_lin_group* h_groups,
+                          int32_t n_groups, const hgt_lin_cblock* cblocks, void* out, int32_t impl,
+                          void* workspace, size_t workspace_bytes, void* stream);
+int hgt_typed_linear_presplit_bf16_workspace_bytes(const hgt_lin_group* h_groups, int32_t n_groups, int32_t K,
+                                                   int32_t cb_width, size_t* out_bytes);
+int hgt_typed_linear_presplit_bf16(const void* a_hi, const void* a_lo, const float* W, const float* bias, int32_t K,
+                                   int32_t cb_width, const hgt_lin_group* groups, const hgt_lin_group* h_groups,
+                                   int32_t n_groups, const hgt_lin_cblock* cblocks, void* out,
+                                   void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Fused edge kernel: gather -> relation-specific score -> softmax by destination -> weighted sum
  * (conv.py:99,108-111 + PyG scatter-add), one pass over the destination-sorted CSR.
@@ -216,6 +236,18 @@ int hgt_edge_forward(const float* q, const float* kv, const float* kvr,
                      float* agg_out, float* att_out, float* stats_out, void* g_hi, void* g_lo,
                      void* workspace, size_t workspace_bytes, int32_t variant, const int32_t* d_tile_counts,
                      const int32_t* type_row0, int32_t num_types, const int32_t* type_active, void* stream);
+/* hgt_edge_forward with bf16 tables: kv [rows+1, 2d] and kvr [P*240+1, 2d] (or NULL) are bf16, everything else as above.
+ * Rows are widened to fp32 as they are loaded; scores, softmax, sums, hub partials and outputs stay fp32.
+ * The bulk-copy ring (variant 2) needs 16-byte rows, i.e. d % 4 == 0 for bf16 rows (d % 2 == 0 for fp32 rows); other d run
+ * the register-gather kernel (variant 1) whatever `variant` asks for, as the fp32 entry point does for its rows. */
+int hgt_edge_forward_bf16kv(const float* q, const void* kv, const void* kvr,
+                            const int32_t* row_ptr, const int32_t* kv_row, const int32_t* rte_row,
+                            const int32_t* csr_eid, const int32_t* tiles, int32_t n_tiles, int32_t n_split_tiles,
+                            const int32_t* hubs, int32_t n_hubs,
+                            int64_t n_nodes, int64_t n_edges, int32_t d, int32_t n_heads, int32_t apply_gelu,
+                            float* agg_out, float* att_out, float* stats_out, void* g_hi, void* g_lo,
+                            void* workspace, size_t workspace_bytes, int32_t variant, const int32_t* d_tile_counts,
+                            const int32_t* type_row0, int32_t num_types, const int32_t* type_active, void* stream);
 
 /* Backward of hgt_edge_forward (training; the reference differentiates the same ops with autograd,
  * OAG/train_paper_field.py:249).  Inputs: the forward's q / kv / kvr tables, its un-activated output
@@ -374,6 +406,14 @@ int hgt_update_epilogue(const float* o, const float* x, const int32_t* type_row0
  * per nn.Linear / nn.LayerNorm of the module (conv.py:34-40).  The plan arrays come from hgt_plan_*; the typed-linear
  * tables are the ones hgt_typed_linear takes (projection: Q + [K'|V'] blocks; rte: K'R/V'R tables; rt: the single
  * 240 x d group of RelTemporalEncoding.lin; upd: a_linears).  Nothing is allocated or synchronised.
+ * kv_bf16 != 0 (inference mode with bf16 tables): the [K'|V'] table and the K'R/V'R tables are stored as bf16, each row
+ * rounded to nearest even after its fp32 GEMM (bias included); Q, the edge kernel's arithmetic and every output stay
+ * fp32.  The projection table then lists the n_q_groups Q groups first (their cblocks address the fp32 Q buffer of
+ * proj_elems floats, from q_off) and the [K'|V'] groups after them (their cblocks address the bf16 table of
+ * (kv_rows + 1) * 2 * d_out elements from 0; kv_off is unused).  kv_bf16 == 0 is the fp32 layer; n_q_groups is ignored.
+ * An fp32-layout projection table passed with kv_bf16 != 0 would address the bf16 table at fp32 offsets: the call
+ * checks the layout on h_proj_groups (n_q_groups groups of one column block, then groups of an even number) and
+ * returns an error otherwise.
  * ---------------------------------------------------------------------------------------------- */
 typedef struct {
   /* sizes and switches */
@@ -417,6 +457,8 @@ typedef struct {
   float* out;                 /* [N or out rows, d_out] */
   float* att;                 /* [E, H] or NULL */
   void* out_hi; void* out_lo; /* optional: out again as the bf16 hi/lo split for the next layer */
+  int32_t kv_bf16;            /* 0: fp32 tables; else bf16 [K'|V'] and K'R/V'R tables (see above) */
+  int32_t n_q_groups;         /* kv_bf16 only: leading Q groups of proj_groups */
 } hgt_conv_args;
 
 uint64_t hgt_conv_args_size(void);   /* sizeof(hgt_conv_args): lets a foreign-language binding check its struct layout */

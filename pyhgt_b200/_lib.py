@@ -51,6 +51,13 @@ SIGNATURES = {
     "hgt_conv_workspace_bytes": [_p, _c.POINTER(_sz)],
     "hgt_conv_forward": [_p, _p, _sz, _p],
     "hgt_update_epilogue": [_p, _p, _p, _i32, _p, _p, _p, _p, _p, _i64, _i32, _p, _p, _p, _p],
+    # bf16 [K'|V'] tables (inference)
+    "hgt_typed_linear_bf16_workspace_bytes": [_p, _i32, _i32, _i32, _i32, _c.POINTER(_sz)],
+    "hgt_typed_linear_bf16": [_p, _i64, _p, _p, _i32, _i32, _p, _p, _i32, _p, _p, _i32, _p, _sz, _p],
+    "hgt_typed_linear_presplit_bf16_workspace_bytes": [_p, _i32, _i32, _i32, _c.POINTER(_sz)],
+    "hgt_typed_linear_presplit_bf16": [_p, _p, _p, _p, _i32, _i32, _p, _p, _i32, _p, _p, _p, _sz, _p],
+    "hgt_edge_forward_bf16kv": [_p, _p, _p, _p, _p, _p, _p, _p, _i32, _i32, _p, _i32, _i64, _i64, _i32, _i32, _i32, _p,
+                                _p, _p, _p, _p, _p, _sz, _i32, _p, _p, _i32, _p, _p],
     # deterministic backward (torch.use_deterministic_algorithms)
     "hgt_plan_group_by_workspace_bytes": [_i64, _i32, _c.POINTER(_sz)],
     "hgt_plan_group_by": [_p, _i64, _i32, _p, _p, _p, _sz, _p],
@@ -88,8 +95,9 @@ class ConvArgs(ctypes.Structure):
             "wq", "bq", "wk", "bk", "wv", "bv", "wa", "ba", "norm_w", "norm_b",
             "relation_att", "relation_msg", "relation_pri", "skip", "emb_weight", "emb_lin_w", "emb_lin_b",
             "x", "x_hi", "x_lo", "out", "att", "out_hi", "out_lo"]
+    _TAIL_I32 = ["kv_bf16", "n_q_groups"]
     _fields_ = ([(n, ctypes.c_int64) for n in _I64] + [(n, ctypes.c_int32) for n in _I32] +
-                [(n, ctypes.c_void_p) for n in _PTR])
+                [(n, ctypes.c_void_p) for n in _PTR] + [(n, ctypes.c_int32) for n in _TAIL_I32])
 
 
 LIN_GROUP_DTYPE = np.dtype([("a_row0", "<i8"), ("m", "<i8"), ("w_row0", "<i4"), ("n_cblocks", "<i4"),

@@ -12,6 +12,10 @@ behind the C ABI in include/hgt_b200.h:
     typed output linear              hgt_typed_linear    a_linears
     gated skip + LayerNorm           hgt_update_epilogue
 
+``HGTConv.kv_dtype = torch.bfloat16`` (or ``set_kv_dtype``) is an opt-in inference mode: the folded [K'|V'] table and
+the RTE tables K'R/V'R are stored as bf16 (each row rounded to nearest even after its fp32 GEMM), which halves the
+bytes the edge kernel gathers; Q, every sum, the softmax, ``att`` and the output stay fp32.
+
 There is no CPU path: CPU tensors raise.  ``GeneralConv`` mirrors conv.py:303-323 so that pyHGT's
 model.py (``from .conv import *``) runs unchanged on top of this module.
 """
@@ -82,6 +86,7 @@ class HGTConv(nn.Module):
     _has_skip = True           # DenseHGTConv (conv.py:143-280) has no skip gate
     emit_split = False         # also write the output as a bf16 hi/lo split for the next layer (model.GNN sets it)
     fused_call = True          # inference goes through ONE C-ABI call (hgt_conv_forward) instead of ~12
+    kv_dtype = torch.float32   # torch.bfloat16: inference with bf16 [K'|V'] / K'R/V'R tables (see set_kv_dtype)
 
     def __init__(self, in_dim, out_dim, num_types, num_relations, n_heads, dropout=0.2, use_norm=True,
                  use_RTE=True, **kwargs):
@@ -157,14 +162,45 @@ class HGTConv(nn.Module):
                     HGTConv.event_sink.append((name, self_.a, self_.b))
         return _T()
 
-    def _typed_linear(self, a, lda, w, bias, k, width, table, out, impl, st):
-        """hgt_typed_linear with its (impl-dependent) workspace; table = (groups_dev, groups_host, n, cblocks_dev)."""
+    def _typed_linear(self, a, lda, w, bias, k, width, table, out, impl, st, groups=None):
+        """hgt_typed_linear with its (impl-dependent) workspace; table = (groups_dev, groups_host, n, cblocks_dev).
+        `groups` = (first, count) restricts the call to a range of the table's groups.  A bf16 `out` selects
+        hgt_typed_linear_bf16 (the same product, rounded to bf16 as it is stored)."""
         g_dev, g_host, n_g, c_dev = table
+        first, n_g = (0, n_g) if groups is None else groups
+        g_ptr, h_ptr = g_dev.data_ptr() + first * g_host.itemsize, g_host.ctypes.data + first * g_host.itemsize
+        sfx = "_bf16" if out.dtype == torch.bfloat16 else ""
         ws_bytes = ctypes.c_size_t()
-        _lib.call("hgt_typed_linear_workspace_bytes", g_host.ctypes.data, n_g, k, width, impl, ctypes.byref(ws_bytes))
+        _lib.call("hgt_typed_linear%s_workspace_bytes" % sfx, h_ptr, n_g, k, width, impl, ctypes.byref(ws_bytes))
         ws = torch.empty(max(ws_bytes.value, 1), dtype=torch.uint8, device=out.device)
-        _lib.call("hgt_typed_linear", a.data_ptr(), lda, w.data_ptr(), _lib.ptr(bias), k, width, g_dev.data_ptr(),
-                  g_host.ctypes.data, n_g, c_dev.data_ptr(), out.data_ptr(), impl, ws.data_ptr(), ws.numel(), st)
+        _lib.call("hgt_typed_linear" + sfx, a.data_ptr(), lda, w.data_ptr(), _lib.ptr(bias), k, width, g_ptr, h_ptr,
+                  n_g, c_dev.data_ptr(), out.data_ptr(), impl, ws.data_ptr(), ws.numel(), st)
+
+    @staticmethod
+    def _presplit_linear(a_hi, a_lo, w, bias, k, width, table, out, st, groups=None):
+        """hgt_typed_linear_presplit (bf16 `out`: hgt_typed_linear_presplit_bf16) over the table's groups, or the range
+        `groups` = (first, count) of them."""
+        g_dev, g_host, n_g, c_dev = table
+        first, n_g = (0, n_g) if groups is None else groups
+        g_ptr, h_ptr = g_dev.data_ptr() + first * g_host.itemsize, g_host.ctypes.data + first * g_host.itemsize
+        sfx = "_bf16" if out.dtype == torch.bfloat16 else ""
+        wsb = ctypes.c_size_t()
+        _lib.call("hgt_typed_linear_presplit%s_workspace_bytes" % sfx, h_ptr, n_g, k, width, ctypes.byref(wsb))
+        ws = torch.empty(max(wsb.value, 1), dtype=torch.uint8, device=out.device)
+        _lib.call("hgt_typed_linear_presplit" + sfx, a_hi.data_ptr(), a_lo.data_ptr(), w.data_ptr(), _lib.ptr(bias), k,
+                  width, g_ptr, h_ptr, n_g, c_dev.data_ptr(), out.data_ptr(), ws.data_ptr(), ws.numel(), st)
+
+    def _kv_bf16(self):
+        """Whether this layer stores its K'/V' tables as bf16 (kv_dtype).  Raises ValueError for a dtype it does not
+        offer, before anything is launched."""
+        dt = self.kv_dtype
+        if dt == torch.float32:
+            return False
+        if dt != torch.bfloat16:
+            raise ValueError("%s.kv_dtype must be torch.float32 or torch.bfloat16, got %r" % (type(self).__name__, dt))
+        if not type(self)._has_skip:
+            raise ValueError("DenseHGTConv has no bf16 K'/V' mode: set kv_dtype = torch.float32")
+        return True
 
     def _check_inputs(self, node_inp, edge_time):
         if node_inp.device.type != "cuda":
@@ -184,7 +220,11 @@ class HGTConv(nn.Module):
 
     def forward(self, node_inp, node_type, edge_index, edge_type, edge_time=None):
         self._check_inputs(node_inp, edge_time)
+        kv_bf16 = self._kv_bf16()
         if torch.is_grad_enabled() and (node_inp.requires_grad or any(p.requires_grad for p in self.parameters())):
+            if kv_bf16:
+                raise ValueError("kv_dtype=torch.bfloat16 is an inference mode and has no backward: run the layer "
+                                 "under torch.no_grad() / torch.inference_mode(), or set kv_dtype = torch.float32")
             from .autograd import hgt_conv_autograd
             return hgt_conv_autograd(self, node_inp, node_type, edge_index, edge_type, edge_time)
         out, att, _ = self._forward_impl(node_inp, node_type, edge_index, edge_type, edge_time,
@@ -203,7 +243,8 @@ class HGTConv(nn.Module):
         N, E = plan.n_nodes, plan.n_edges
         if node_inp.shape[0] != N:
             raise ValueError("node_inp has %d rows but node_type has %d" % (node_inp.shape[0], N))
-        lt = _plan.layer_tables(plan, d_in, d, active_per_type, kv_runs)
+        kv_bf16 = self._kv_bf16()
+        lt = _plan.layer_tables(plan, d_in, d, active_per_type, kv_runs, kv_bf16)
         tabs = [self._ptrs("wq", [l.weight for l in self.q_linears], dev),
                 self._ptrs("bq", [l.bias for l in self.q_linears], dev),
                 self._ptrs("wk", [l.weight for l in self.k_linears], dev),
@@ -217,7 +258,7 @@ class HGTConv(nn.Module):
         scalars = [self.relation_att, self.relation_msg, self.relation_pri, self.skip]
         if self.use_RTE:
             scalars += [self.emb.emb.weight, self.emb.lin.weight, self.emb.lin.bias]
-        key = (id(lt),) + tuple(t.data_ptr() for t in tabs) + tuple(t.data_ptr() for t in scalars)
+        key = (id(lt), kv_bf16) + tuple(t.data_ptr() for t in tabs) + tuple(t.data_ptr() for t in scalars)
         cache = self.__dict__.setdefault("_args_cache", {})
         ent = cache.get(key)
         if ent is None:
@@ -226,6 +267,7 @@ class HGTConv(nn.Module):
             a.q_off, a.kv_off, a.proj_elems = lt.q_off, lt.kv_off, lt.proj_elems
             a.num_types, a.num_relations, a.n_heads, a.d_in, a.d_out, a.n_pairs = T, R, H, d_in, d, plan.n_pairs
             a.use_rte, a.use_norm = int(self.use_RTE), int(self.use_norm)
+            a.kv_bf16, a.n_q_groups = int(kv_bf16), lt.n_q_groups
             a.n_tiles, a.n_split, a.n_hubs = plan.n_tiles, plan.n_split, plan.n_hubs
             a.perm = None if plan.sorted_types else plan.perm.data_ptr()
             a.type_row0 = plan.type_row0_dev.data_ptr()
@@ -288,6 +330,8 @@ class HGTConv(nn.Module):
                       active_per_type=None, out_map=None, out_rows=None, x_split=None, kv_runs=None):
         """out_map / out_rows (sharded runs): int32 [N] map from rank-order row to output row and the number of output
         rows; rows that are not active (halo sources) are never written, so the output holds exactly the owned rows."""
+        if save and self._kv_bf16():
+            raise ValueError("kv_dtype=torch.bfloat16 is an inference mode: nothing is saved for a backward pass")
         if (self.fused_call and not save and HGTConv.event_sink is None and type(self)._has_skip
                 and not (self.training and self.drop.p > 0)):
             return self._forward_fused(node_inp, node_type, edge_index, edge_type, edge_time, want_att,
@@ -332,7 +376,8 @@ class HGTConv(nn.Module):
         N, E, P = plan.n_nodes, plan.n_edges, plan.n_pairs
         if node_inp.shape[0] != N:
             raise ValueError("node_inp has %d rows but node_type has %d" % (node_inp.shape[0], N))
-        lt = _plan.layer_tables(plan, d_in, d, active_per_type, kv_runs)
+        kv_bf16 = self._kv_bf16()
+        lt = _plan.layer_tables(plan, d_in, d, active_per_type, kv_runs, kv_bf16)
         f32 = dict(dtype=torch.float32, device=dev)
         x = node_inp.contiguous()
         if x_split is None and plan.sorted_types and self.linear_impl in (0, 2):
@@ -362,30 +407,38 @@ class HGTConv(nn.Module):
                   plan.pair_rel_dev.data_ptr(), lt.cat_row0_dev.data_ptr(), lt.q_row0_dev.data_ptr(),
                   w_cat.data_ptr(), b_cat.data_ptr(), st)
 
-        # 2. typed projections: Q [N,d] and the folded [K'|V'] table (+ trailing all-zero row)
+        # 2. typed projections: Q [N,d] and the folded [K'|V'] table (+ trailing all-zero row); with bf16 tables the Q
+        #    groups and the K'/V' groups are two calls into two buffers
+        kv_f = dict(dtype=torch.bfloat16, device=dev) if kv_bf16 else f32
         proj = torch.empty(lt.proj_elems, **f32)
         q_tab = proj[lt.q_off:lt.q_off + N * d]
-        kv_tab = proj[lt.kv_off:]
+        kv_tab = torch.empty(lt.kv_elems, **kv_f) if kv_bf16 else proj[lt.kv_off:]
         kv_tab[plan.kv_rows * 2 * d:].zero_()
+        n_g = lt.proj_groups[2]
+        parts = [((0, lt.n_q_groups), proj), ((lt.n_q_groups, n_g - lt.n_q_groups), kv_tab)] if kv_bf16 else [(None, proj)]
+        pre = x_split if plan.sorted_types else None
         with self._stage("proj_linear"):
-            if x_split is not None and plan.sorted_types:
-                # A operand already split by its producer (the fused halo pull): tensor-core GEMM without the split pass
-                g_dev, g_host, n_g, c_dev = lt.proj_groups
-                wsb = ctypes.c_size_t()
-                _lib.call("hgt_typed_linear_presplit_workspace_bytes", g_host.ctypes.data, n_g, d_in, d, ctypes.byref(wsb))
-                ws1 = torch.empty(max(wsb.value, 1), dtype=torch.uint8, device=dev)
-                _lib.call("hgt_typed_linear_presplit", x_split[0].data_ptr(), x_split[1].data_ptr(), w_cat.data_ptr(),
-                          b_cat.data_ptr(), d_in, d, g_dev.data_ptr(), g_host.ctypes.data, n_g, c_dev.data_ptr(),
-                          proj.data_ptr(), ws1.data_ptr(), ws1.numel(), st)
-            else:
-                self._typed_linear(x_sorted, d_in, w_cat, b_cat, d_in, d, lt.proj_groups, proj, self.linear_impl, st)
+            if kv_bf16 and pre is None and self.linear_impl in (0, 2) and d_in % 16 == 0 and d_in >= 64:
+                # two tensor-core GEMMs over the same x: split it once (the GEMM's own split, so the same bits)
+                pre = (torch.empty((N, d_in), dtype=torch.bfloat16, device=dev),
+                       torch.empty((N, d_in), dtype=torch.bfloat16, device=dev))
+                _lib.call("hgt_act_split", x_sorted.data_ptr(), d_in, N, d_in, 0, None, pre[0].data_ptr(),
+                          pre[1].data_ptr(), st)
+            for groups, dst in parts:
+                if pre is not None:
+                    # A operand already split by its producer (the fused halo pull): tensor-core GEMM without the split
+                    # pass
+                    self._presplit_linear(pre[0], pre[1], w_cat, b_cat, d_in, d, lt.proj_groups, dst, st, groups)
+                else:
+                    self._typed_linear(x_sorted, d_in, w_cat, b_cat, d_in, d, lt.proj_groups, dst, self.linear_impl, st,
+                                       groups)
         kvr = None
         if self.use_RTE:
             # RT = lin(emb.weight) [240,d] (conv.py:299), then projected with every pair's K'/V' weights (no bias)
             rt = torch.empty((_plan.RTE_MAX_LEN, d_in), **f32)
             self._typed_linear(self.emb.emb.weight, d_in, self.emb.lin.weight, self.emb.lin.bias, d_in, d_in,
                                lt.rt_group, rt, 1, st)
-            kvr = torch.empty((P * _plan.RTE_MAX_LEN + 1) * 2 * d, **f32)
+            kvr = torch.empty((P * _plan.RTE_MAX_LEN + 1) * 2 * d, **kv_f)
             kvr[P * _plan.RTE_MAX_LEN * 2 * d:].zero_()
             self._typed_linear(rt, d_in, w_cat, None, d_in, d, lt.rte_groups, kvr, 1, st)
 
@@ -403,7 +456,7 @@ class HGTConv(nn.Module):
         att = torch.empty((E, H), **f32) if want_att else None
         stats = torch.empty((N, 2 * H), **f32) if save else None
         with self._stage("edge"):
-            _lib.call("hgt_edge_forward", q_tab.data_ptr(), kv_tab.data_ptr(), _lib.ptr(kvr), plan.row_ptr.data_ptr(),
+            _lib.call("hgt_edge_forward_bf16kv" if kv_bf16 else "hgt_edge_forward", q_tab.data_ptr(), kv_tab.data_ptr(), _lib.ptr(kvr), plan.row_ptr.data_ptr(),
                       plan.kv_row.data_ptr(), _lib.ptr(plan.rte_row) if self.use_RTE else None,
                       plan.csr_eid.data_ptr(), plan.tiles.data_ptr(), plan.n_tiles, plan.n_split,
                       plan.hubs.data_ptr(), plan.n_hubs, N, E, d, H, 1 if (gelu_before_a and not save) else 0,
@@ -424,13 +477,7 @@ class HGTConv(nn.Module):
         o = torch.empty((N, d), **f32)
         with self._stage("upd_linear"):
             if fuse_split:
-                g_dev, g_host, n_g, c_dev = lt.upd_groups
-                wsb = ctypes.c_size_t()
-                _lib.call("hgt_typed_linear_presplit_workspace_bytes", g_host.ctypes.data, n_g, d, d, ctypes.byref(wsb))
-                ws2 = torch.empty(max(wsb.value, 1), dtype=torch.uint8, device=dev)
-                _lib.call("hgt_typed_linear_presplit", g_hi.data_ptr(), g_lo.data_ptr(), wa_cat.data_ptr(),
-                          ba_cat.data_ptr(), d, d, g_dev.data_ptr(), g_host.ctypes.data, n_g, c_dev.data_ptr(),
-                          o.data_ptr(), ws2.data_ptr(), ws2.numel(), st)
+                self._presplit_linear(g_hi, g_lo, wa_cat, ba_cat, d, d, lt.upd_groups, o, st)
             else:
                 self._typed_linear(g_act, d, wa_cat, ba_cat, d, d, lt.upd_groups, o, self.linear_impl, st)
         if self.training and self.drop.p > 0:
@@ -458,6 +505,7 @@ class DenseHGTConv(HGTConv):
 
     def forward(self, node_inp, node_type, edge_index, edge_type, edge_time=None):
         self._check_inputs(node_inp, edge_time)
+        self._kv_bf16()                                            # raises for bf16: this layer has no such mode
         from .autograd import dense_hgt_forward
         return dense_hgt_forward(self, node_inp, node_type, edge_index, edge_type, edge_time)
 
@@ -480,3 +528,17 @@ class GeneralConv(nn.Module):
 
     def forward(self, meta_xs, node_type, edge_index, edge_type, edge_time):
         return self.base_conv(meta_xs, node_type, edge_index, edge_type, edge_time)
+
+
+def set_kv_dtype(module, dtype):
+    """Set `kv_dtype` on every HGTConv in `module`'s tree (e.g. a GNN) and return `module`.
+
+    torch.bfloat16 stores the folded K'/V' tables in bf16 for inference (about half the edge kernel's memory traffic and
+    half the table memory); torch.float32 is the default, exact fp32 path.  The attribute is a plain instance attribute:
+    state_dict and pickling are unchanged."""
+    if dtype not in (torch.float32, torch.bfloat16):
+        raise ValueError("kv_dtype must be torch.float32 or torch.bfloat16, got %r" % (dtype,))
+    for m in module.modules():
+        if isinstance(m, HGTConv):
+            m.kv_dtype = dtype
+    return module

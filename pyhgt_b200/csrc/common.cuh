@@ -59,6 +59,11 @@ __device__ __forceinline__ void hgt_split_bf16x4(const float (&v)[4], uint2* hi,
   *lo = *reinterpret_cast<uint2*>(l);
 }
 
+// Output element of the typed GEMMs: fp32, or bf16 rounded to nearest even (the bf16 [K'|V'] tables of inference).
+// Rounding the finished fp32 value gives the bits of torch's `.bfloat16()` of the fp32 result.
+__device__ __forceinline__ void hgt_store_out(float* p, float v) { *p = v; }
+__device__ __forceinline__ void hgt_store_out(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+
 // ---- ordered reductions (deterministic backward, torch.use_deterministic_algorithms) ------------------------------------
 // Partial results of a reduction are written to [chunks, stride] scratch and summed in chunk order, so the bits of the
 // result depend only on the problem shape, never on which CTA finished first.

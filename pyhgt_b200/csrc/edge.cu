@@ -16,6 +16,10 @@
 //                      ring with mbarrier transaction counting; the warp issues STAGES rows ahead.
 // Roofline: HBM-bound; algorithmic bytes per edge = 2*d*4 (row) + 4 (kv_row) [+4 rte_row, +2*d*4 from L2]
 // and per destination d*4 (Q) + d*4 (agg) + 4 (row_ptr).
+//
+// The tables may also be bf16 (hgt_edge_forward_bf16kv, inference): both variants take the row element type as a
+// template parameter, lanes widen the row to fp32 as they load it, and everything after the load is the fp32 code.
+// A bf16 row halves the per-edge bytes: 2*d*2 + 4.
 #include <cuda_bf16.h>
 
 #include "common.cuh"
@@ -30,8 +34,8 @@ constexpr int kCtaThreads = kWarpsPerCta * 32;
 
 struct EdgeParams {
   const float* q;
-  const float* kv;
-  const float* kvr;          // nullptr when !use_RTE
+  const void* kv;            // [rows+1, 2d] of the kernel's row type (float or __nv_bfloat16)
+  const void* kvr;           // same type; nullptr when !use_RTE
   const int32_t* row_ptr;
   const int32_t* kv_row;
   const int32_t* rte_row;
@@ -86,6 +90,52 @@ __device__ __forceinline__ void load_vec_nc(float (&dst)[VEC], const float* p) {
     asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(dst[0]) : "l"(p));
   }
 }
+// bf16 -> fp32 is exact: the bf16 bits are the upper half of the fp32 word
+__device__ __forceinline__ float bf16_lo(uint32_t u) { return __uint_as_float(u << 16); }
+__device__ __forceinline__ float bf16_hi(uint32_t u) { return __uint_as_float(u & 0xffff0000u); }
+
+// VEC consecutive row elements, widened to fp32: load_row (cached; also shared memory) and load_row_nc (streaming gather)
+template <int VEC>
+__device__ __forceinline__ void load_row(float (&dst)[VEC], const float* p) { load_vec<VEC>(dst, p); }
+template <int VEC>
+__device__ __forceinline__ void load_row_nc(float (&dst)[VEC], const float* p) { load_vec_nc<VEC>(dst, p); }
+template <int VEC>
+__device__ __forceinline__ void widen_bf16(float (&dst)[VEC], const uint32_t* w) {
+  if constexpr (VEC == 1) {
+    dst[0] = bf16_lo(w[0]);
+  } else {
+#pragma unroll
+    for (int i = 0; i < VEC / 2; ++i) { dst[2 * i] = bf16_lo(w[i]); dst[2 * i + 1] = bf16_hi(w[i]); }
+  }
+}
+template <int VEC>
+__device__ __forceinline__ void load_row(float (&dst)[VEC], const __nv_bfloat16* p) {
+  uint32_t w[(VEC + 1) / 2];
+  if constexpr (VEC == 4) {
+    const uint2 u = *reinterpret_cast<const uint2*>(p);
+    w[0] = u.x; w[1] = u.y;
+  } else if constexpr (VEC == 2) {
+    w[0] = *reinterpret_cast<const uint32_t*>(p);
+  } else {
+    w[0] = *reinterpret_cast<const unsigned short*>(p);
+  }
+  widen_bf16<VEC>(dst, w);
+}
+template <int VEC>
+__device__ __forceinline__ void load_row_nc(float (&dst)[VEC], const __nv_bfloat16* p) {
+  uint32_t w[(VEC + 1) / 2];
+  if constexpr (VEC == 4) {
+    asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(w[0]), "=r"(w[1]) : "l"(p));
+  } else if constexpr (VEC == 2) {
+    asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(w[0]) : "l"(p));
+  } else {
+    unsigned short h;
+    asm volatile("ld.global.nc.L1::no_allocate.u16 %0, [%1];" : "=h"(h) : "l"(p));
+    w[0] = h;
+  }
+  widen_bf16<VEC>(dst, w);
+}
+
 template <int VEC>
 __device__ __forceinline__ void store_vec(float* p, const float (&src)[VEC]) {
   using V = typename VecT<VEC>::type;
@@ -200,7 +250,7 @@ __device__ __forceinline__ void finalize_destination(const EdgeParams& p, const 
 // ------------------------------------------------------------------------------------------------
 // variant 1: direct register gather
 // ------------------------------------------------------------------------------------------------
-template <int VEC, int NCH>
+template <typename KvT, int VEC, int NCH>
 __global__ void __launch_bounds__(kCtaThreads, 1)
 k_edge_fwd_ldg(EdgeParams p) {
   // rows in flight per warp: bounded by the register budget (2 * U * NCH * VEC floats of staging)
@@ -208,6 +258,8 @@ k_edge_fwd_ldg(EdgeParams p) {
   const int lane = threadIdx.x & 31;
   const LaneMap lm(p, lane);
   const bool rte = p.kvr != nullptr;
+  const KvT* kv = static_cast<const KvT*>(p.kv);
+  const KvT* kvr = static_cast<const KvT*>(p.kvr);
   const int64_t row_stride = 2 * (int64_t)p.d;
   int offs[NCH];
 #pragma unroll
@@ -245,12 +297,12 @@ k_edge_fwd_ldg(EdgeParams p) {
 #pragma unroll
           for (int u = 0; u < EDGE_UNROLL; ++u) {
             if (u < nb) {
-              const float* row = p.kv + (int64_t)p.kv_row[c0 + u] * row_stride;
+              const KvT* row = kv + (int64_t)p.kv_row[c0 + u] * row_stride;
 #pragma unroll
               for (int t = 0; t < NCH; ++t) {
                 if (offs[t] >= 0) {
-                  load_vec_nc<VEC>(kk[u][t], row + offs[t]);
-                  load_vec_nc<VEC>(vv[u][t], row + p.d + offs[t]);
+                  load_row_nc<VEC>(kk[u][t], row + offs[t]);
+                  load_row_nc<VEC>(vv[u][t], row + p.d + offs[t]);
                 } else {
 #pragma unroll
                   for (int v = 0; v < VEC; ++v) { kk[u][t][v] = 0.f; vv[u][t][v] = 0.f; }
@@ -262,13 +314,13 @@ k_edge_fwd_ldg(EdgeParams p) {
 #pragma unroll
             for (int u = 0; u < EDGE_UNROLL; ++u) {
               if (u < nb) {
-                const float* row = p.kvr + (int64_t)p.rte_row[c0 + u] * row_stride;
+                const KvT* row = kvr + (int64_t)p.rte_row[c0 + u] * row_stride;
 #pragma unroll
                 for (int t = 0; t < NCH; ++t) {
                   if (offs[t] >= 0) {
                     float a[VEC], b[VEC];
-                    load_vec<VEC>(a, row + offs[t]);
-                    load_vec<VEC>(b, row + p.d + offs[t]);
+                    load_row<VEC>(a, row + offs[t]);
+                    load_row<VEC>(b, row + p.d + offs[t]);
 #pragma unroll
                     for (int v = 0; v < VEC; ++v) { kk[u][t][v] += a[v]; vv[u][t][v] += b[v]; }
                   }
@@ -327,7 +379,7 @@ k_edge_fwd_ldg(EdgeParams p) {
 // ------------------------------------------------------------------------------------------------
 // variant 2: bulk async copy (TMA engine) -> per-warp shared-memory ring
 // ------------------------------------------------------------------------------------------------
-template <int VEC, int NCH>
+template <typename KvT, int VEC, int NCH>
 __global__ void __launch_bounds__(kCtaThreads, (VEC * NCH <= 4) ? 2 : 1)   // narrow rows (d_k <= 16): two CTAs per SM
 k_edge_fwd_tma(EdgeParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -336,7 +388,9 @@ k_edge_fwd_tma(EdgeParams p) {
   const LaneMap lm(p, lane);
   const bool rte = p.kvr != nullptr;
   const int S = p.stages;
-  const uint32_t row_bytes = 2u * (uint32_t)p.d * 4u;
+  const KvT* kv = static_cast<const KvT*>(p.kv);
+  const KvT* kvr = static_cast<const KvT*>(p.kvr);
+  const uint32_t row_bytes = 2u * (uint32_t)p.d * (uint32_t)sizeof(KvT);
   const uint32_t slot_bytes = rte ? 2u * row_bytes : row_bytes;
   const int64_t row_stride = 2 * (int64_t)p.d;
   // layout: [warps][S][slot_bytes] rows, then [warps][S] mbarriers
@@ -392,8 +446,8 @@ k_edge_fwd_tma(EdgeParams p) {
         const uint32_t bar = s_u32(&bars[slot]);
         const uint32_t dst = s_u32(ring + (size_t)slot * slot_bytes);
         mbar_expect_tx(bar, slot_bytes);
-        bulk_g2s(dst, p.kv + (int64_t)row * row_stride, row_bytes, bar);
-        if (rte) bulk_g2s(dst + row_bytes, p.kvr + (int64_t)rrow * row_stride, row_bytes, bar);
+        bulk_g2s(dst, kv + (int64_t)row * row_stride, row_bytes, bar);
+        if (rte) bulk_g2s(dst + row_bytes, kvr + (int64_t)rrow * row_stride, row_bytes, bar);
       }
       ++issue_it;
     };
@@ -420,18 +474,18 @@ k_edge_fwd_tma(EdgeParams p) {
         for (int c = seg_begin; c < seg_end; ++c) {
           const uint32_t slot = it % S;
           mbar_wait(s_u32(&bars[slot]), (it / S) & 1u);
-          const float* srow = reinterpret_cast<const float*>(ring + (size_t)slot * slot_bytes);
+          const KvT* srow = reinterpret_cast<const KvT*>(ring + (size_t)slot * slot_bytes);
           float kk[NCH][VEC], vv[NCH][VEC];
           float part = 0.f;
 #pragma unroll
           for (int t = 0; t < NCH; ++t) {
             if (offs[t] >= 0) {
-              load_vec<VEC>(kk[t], srow + offs[t]);
-              load_vec<VEC>(vv[t], srow + p.d + offs[t]);
+              load_row<VEC>(kk[t], srow + offs[t]);
+              load_row<VEC>(vv[t], srow + p.d + offs[t]);
               if (rte) {
                 float a[VEC], b[VEC];
-                load_vec<VEC>(a, srow + row_stride + offs[t]);
-                load_vec<VEC>(b, srow + row_stride + p.d + offs[t]);
+                load_row<VEC>(a, srow + row_stride + offs[t]);
+                load_row<VEC>(b, srow + row_stride + p.d + offs[t]);
 #pragma unroll
                 for (int v = 0; v < VEC; ++v) { kk[t][v] += a[v]; vv[t][v] += b[v]; }
               }
@@ -537,30 +591,30 @@ k_merge_partials(EdgeParams p, const int32_t* __restrict__ hubs, int n_hubs_host
   }
 }
 
-template <int VEC, int NCH>
+template <typename KvT, int VEC, int NCH>
 int launch_variant(const EdgeParams& p, int variant, int grid, size_t smem, cudaStream_t st) {
   if (variant == 1) {
-    k_edge_fwd_ldg<VEC, NCH><<<grid, kCtaThreads, 0, st>>>(p);
+    k_edge_fwd_ldg<KvT, VEC, NCH><<<grid, kCtaThreads, 0, st>>>(p);
   } else {
     static size_t configured = 0;            // per instantiation: raise the dynamic shared-memory limit once, not per launch
     if (smem > configured) {
-      HGT_CHECK_CUDA(cudaFuncSetAttribute(k_edge_fwd_tma<VEC, NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+      HGT_CHECK_CUDA(cudaFuncSetAttribute(k_edge_fwd_tma<KvT, VEC, NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           (int)smem));
       configured = smem;
     }
-    k_edge_fwd_tma<VEC, NCH><<<grid, kCtaThreads, smem, st>>>(p);
+    k_edge_fwd_tma<KvT, VEC, NCH><<<grid, kCtaThreads, smem, st>>>(p);
   }
   HGT_LAUNCH_CHECK();
   return 0;
 }
 
-template <int VEC>
+template <typename KvT, int VEC>
 int dispatch_nch(const EdgeParams& p, int nch, int variant, int grid, size_t smem, cudaStream_t st) {
   switch (nch) {
-    case 1: return launch_variant<VEC, 1>(p, variant, grid, smem, st);
-    case 2: return launch_variant<VEC, 2>(p, variant, grid, smem, st);
-    case 4: return launch_variant<VEC, 4>(p, variant, grid, smem, st);
-    case 8: return launch_variant<VEC, 8>(p, variant, grid, smem, st);
+    case 1: return launch_variant<KvT, VEC, 1>(p, variant, grid, smem, st);
+    case 2: return launch_variant<KvT, VEC, 2>(p, variant, grid, smem, st);
+    case 4: return launch_variant<KvT, VEC, 4>(p, variant, grid, smem, st);
+    case 8: return launch_variant<KvT, VEC, 8>(p, variant, grid, smem, st);
   }
   hgt_set_error("hgt_edge_forward: internal: unsupported chunk count %d", nch);
   return 1;
@@ -574,26 +628,25 @@ extern "C" int hgt_edge_workspace_bytes(int32_t n_split_tiles, int32_t d, int32_
   return 0;
 }
 
-extern "C" int hgt_edge_forward(const float* q, const float* kv, const float* kvr, const int32_t* row_ptr,
-                                const int32_t* kv_row, const int32_t* rte_row, const int32_t* csr_eid,
-                                const int32_t* tiles, int32_t n_tiles, int32_t n_split_tiles, const int32_t* hubs,
-                                int32_t n_hubs, int64_t n_nodes,
-                                int64_t n_edges, int32_t d, int32_t n_heads, int32_t apply_gelu, float* agg_out,
-                                float* att_out, float* stats_out, void* g_hi, void* g_lo, void* workspace,
-                                size_t workspace_bytes, int32_t variant, const int32_t* d_tile_counts,
-                                const int32_t* type_row0, int32_t num_types, const int32_t* type_active,
-                                void* stream_) {
-  cudaStream_t st = (cudaStream_t)stream_;
-  (void)n_edges;
-  HGT_REQUIRE(n_heads >= 1 && n_heads <= 32, "hgt_edge_forward: n_heads=%d unsupported (1..32)", n_heads);
-  HGT_REQUIRE(d % n_heads == 0, "hgt_edge_forward: d=%d not divisible by n_heads=%d", d, n_heads);
-  HGT_REQUIRE((kvr != nullptr) == (rte_row != nullptr), "hgt_edge_forward: kvr and rte_row must go together");
+
+// Shared host side of hgt_edge_forward (fp32 tables) and hgt_edge_forward_bf16kv (bf16 tables).
+template <typename KvT>
+static int edge_forward(const char* fn, const float* q, const void* kv, const void* kvr, const int32_t* row_ptr,
+                        const int32_t* kv_row, const int32_t* rte_row, const int32_t* csr_eid, const int32_t* tiles,
+                        int32_t n_tiles, int32_t n_split_tiles, const int32_t* hubs, int32_t n_hubs, int64_t n_nodes,
+                        int32_t d, int32_t n_heads, int32_t apply_gelu, float* agg_out, float* att_out,
+                        float* stats_out, void* g_hi, void* g_lo, void* workspace, size_t workspace_bytes,
+                        int32_t variant, const int32_t* d_tile_counts, const int32_t* type_row0, int32_t num_types,
+                        const int32_t* type_active, cudaStream_t st) {
+  HGT_REQUIRE(n_heads >= 1 && n_heads <= 32, "%s: n_heads=%d unsupported (1..32)", fn, n_heads);
+  HGT_REQUIRE(d % n_heads == 0, "%s: d=%d not divisible by n_heads=%d", fn, d, n_heads);
+  HGT_REQUIRE((kvr != nullptr) == (rte_row != nullptr), "%s: kvr and rte_row must go together", fn);
   HGT_REQUIRE((g_hi != nullptr) == (g_lo != nullptr) && (agg_out != nullptr || g_hi != nullptr),
-              "hgt_edge_forward: need agg_out and/or the (g_hi, g_lo) pair");
-  HGT_REQUIRE(g_hi == nullptr || d % 8 == 0, "hgt_edge_forward: split output needs d %% 8 == 0 (d=%d)", d);
+              "%s: need agg_out and/or the (g_hi, g_lo) pair", fn);
+  HGT_REQUIRE(g_hi == nullptr || d % 8 == 0, "%s: split output needs d %% 8 == 0 (d=%d)", fn, d);
   size_t need = 0;
   hgt_edge_workspace_bytes(n_split_tiles, d, n_heads, &need);
-  HGT_REQUIRE(workspace_bytes >= need, "hgt_edge_forward: workspace too small (%zu < %zu)", workspace_bytes, need);
+  HGT_REQUIRE(workspace_bytes >= need, "%s: workspace too small (%zu < %zu)", fn, workspace_bytes, need);
   if (n_nodes == 0 || n_tiles == 0) return 0;
 
   EdgeParams p;
@@ -619,13 +672,13 @@ extern "C" int hgt_edge_forward(const float* q, const float* kv, const float* kv
   int chunks = (p.DK + vec * p.LPH - 1) / (vec * p.LPH);
   int nch = 1;
   while (nch < chunks) nch <<= 1;
-  HGT_REQUIRE(nch <= 8, "hgt_edge_forward: head width d_k=%d with %d heads needs %d chunks per lane (max 8)",
-              p.DK, n_heads, chunks);
+  HGT_REQUIRE(nch <= 8, "%s: head width d_k=%d with %d heads needs %d chunks per lane (max 8)", fn, p.DK, n_heads,
+              chunks);
 
   const int sms = hgt_sm_count();
   int grid = sms;
   size_t smem = 0;
-  const size_t row_bytes = 2 * (size_t)d * 4;
+  const size_t row_bytes = 2 * (size_t)d * sizeof(KvT);
   const size_t slot_bytes = kvr ? 2 * row_bytes : row_bytes;
   if (variant == 0) variant = 2;
   // narrow rows (one float4 per lane): the kernel is bound by per-destination latency, not by bytes in flight, so two
@@ -634,28 +687,60 @@ extern "C" int hgt_edge_forward(const float* q, const float* kv, const float* kv
   if (variant == 2) {
     const size_t budget = two_ctas ? 100 * 1024 : 200 * 1024;
     int stages = (int)(budget / (kWarpsPerCta * slot_bytes));
-    if (stages > 8) stages = 8;
+    if (stages > 8) stages = 8;   // also for bf16 rows: a cap of 16 measured no faster (DESIGN.md 4.1)
     if (stages < 2 || row_bytes % 16 != 0) variant = 1;     // rows too wide / misaligned for the ring
     else {
       p.stages = stages;
       smem = (size_t)kWarpsPerCta * stages * (slot_bytes + 8);
     }
   }
-  HGT_REQUIRE(variant == 1 || variant == 2, "hgt_edge_forward: unknown variant %d", variant);
+  HGT_REQUIRE(variant == 1 || variant == 2, "%s: unknown variant %d", fn, variant);
   // persistent grid: one CTA per SM, never more CTAs than tiles/warps
   if (two_ctas && variant == 2) grid = 2 * sms;
   int max_ctas = (n_tiles + kWarpsPerCta - 1) / kWarpsPerCta;
   if (grid > max_ctas) grid = max_ctas;
   HGT_CHECK_CUDA(cudaMemsetAsync(p.tile_counter, 0, sizeof(int32_t), st));
   int rc;
-  if (vec == 4) rc = dispatch_nch<4>(p, nch, variant, grid, smem, st);
-  else if (vec == 2) rc = dispatch_nch<2>(p, nch, variant, grid, smem, st);
-  else rc = dispatch_nch<1>(p, nch, variant, grid, smem, st);
+  if (vec == 4) rc = dispatch_nch<KvT, 4>(p, nch, variant, grid, smem, st);
+  else if (vec == 2) rc = dispatch_nch<KvT, 2>(p, nch, variant, grid, smem, st);
+  else rc = dispatch_nch<KvT, 1>(p, nch, variant, grid, smem, st);
   if (rc) return rc;
   if (n_split_tiles > 0) {
-    HGT_REQUIRE(hubs != nullptr && n_hubs > 0, "hgt_edge_forward: split tiles present but no hub list given");
+    HGT_REQUIRE(hubs != nullptr && n_hubs > 0, "%s: split tiles present but no hub list given", fn);
     k_merge_partials<<<n_hubs < 4 * sms ? n_hubs : 4 * sms, kMergeThreads, 0, st>>>(p, hubs, n_hubs);
     HGT_LAUNCH_CHECK();
   }
   return 0;
+}
+
+extern "C" int hgt_edge_forward(const float* q, const float* kv, const float* kvr, const int32_t* row_ptr,
+                                const int32_t* kv_row, const int32_t* rte_row, const int32_t* csr_eid,
+                                const int32_t* tiles, int32_t n_tiles, int32_t n_split_tiles, const int32_t* hubs,
+                                int32_t n_hubs, int64_t n_nodes,
+                                int64_t n_edges, int32_t d, int32_t n_heads, int32_t apply_gelu, float* agg_out,
+                                float* att_out, float* stats_out, void* g_hi, void* g_lo, void* workspace,
+                                size_t workspace_bytes, int32_t variant, const int32_t* d_tile_counts,
+                                const int32_t* type_row0, int32_t num_types, const int32_t* type_active,
+                                void* stream_) {
+  (void)n_edges;
+  return edge_forward<float>("hgt_edge_forward", q, kv, kvr, row_ptr, kv_row, rte_row, csr_eid, tiles, n_tiles,
+                             n_split_tiles, hubs, n_hubs, n_nodes, d, n_heads, apply_gelu, agg_out, att_out, stats_out,
+                             g_hi, g_lo, workspace, workspace_bytes, variant, d_tile_counts, type_row0, num_types,
+                             type_active, (cudaStream_t)stream_);
+}
+
+extern "C" int hgt_edge_forward_bf16kv(const float* q, const void* kv, const void* kvr, const int32_t* row_ptr,
+                                       const int32_t* kv_row, const int32_t* rte_row, const int32_t* csr_eid,
+                                       const int32_t* tiles, int32_t n_tiles, int32_t n_split_tiles,
+                                       const int32_t* hubs, int32_t n_hubs, int64_t n_nodes, int64_t n_edges, int32_t d,
+                                       int32_t n_heads, int32_t apply_gelu, float* agg_out, float* att_out,
+                                       float* stats_out, void* g_hi, void* g_lo, void* workspace,
+                                       size_t workspace_bytes, int32_t variant, const int32_t* d_tile_counts,
+                                       const int32_t* type_row0, int32_t num_types, const int32_t* type_active,
+                                       void* stream_) {
+  (void)n_edges;
+  return edge_forward<__nv_bfloat16>("hgt_edge_forward_bf16kv", q, kv, kvr, row_ptr, kv_row, rte_row, csr_eid, tiles,
+                                     n_tiles, n_split_tiles, hubs, n_hubs, n_nodes, d, n_heads, apply_gelu, agg_out,
+                                     att_out, stats_out, g_hi, g_lo, workspace, workspace_bytes, variant,
+                                     d_tile_counts, type_row0, num_types, type_active, (cudaStream_t)stream_);
 }

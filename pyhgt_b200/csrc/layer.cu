@@ -4,6 +4,7 @@
 // the given stream without any host synchronisation.  This is what a non-Python host binds for the layer
 // (reference boundary: HGTConv.forward, pyHGT/conv.py:56-134); the Python class uses it too, so that a layer costs
 // one ctypes call instead of a dozen (the reference's sampled-subgraph batches are launch/host-bound).
+// With kv_bf16 the [K'|V'] and K'R/V'R tables are written and gathered as bf16 (inference mode, see the header).
 #include "common.cuh"
 
 int hgt_update_epilogue_impl(const float* o, const float* x, const int32_t* type_row0, int32_t num_types,
@@ -29,6 +30,7 @@ struct Carver {
 
 struct Layout {
   float *x_sorted, *w_cat, *b_cat, *proj, *rt, *kvr, *g_act, *wa_cat, *ba_cat, *o;
+  void *kv16, *kvr16;                                      // kv_bf16: the bf16 tables (else NULL)
   void *g_hi, *g_lo, *ws_proj, *ws_edge, *ws_upd;
   size_t ws_proj_bytes, ws_edge_bytes, ws_upd_bytes, total;
   bool fuse_split, presplit_x;
@@ -46,6 +48,7 @@ int plan_layout(const hgt_conv_args* a, void* base, Layout* L) {
   L->w_cat = c.take<float>((size_t)(a->cat_rows > 0 ? a->cat_rows : 1) * din);
   L->b_cat = c.take<float>((size_t)(a->cat_rows > 0 ? a->cat_rows : 1));
   L->proj = c.take<float>((size_t)a->proj_elems);
+  L->kv16 = a->kv_bf16 ? c.take<__nv_bfloat16>(((size_t)a->kv_rows + 1) * 2 * d) : nullptr;
   int rc;
   if (L->presplit_x)
     rc = hgt_typed_linear_presplit_workspace_bytes(a->h_proj_groups, a->n_proj_groups, din, d, &L->ws_proj_bytes);
@@ -54,9 +57,14 @@ int plan_layout(const hgt_conv_args* a, void* base, Layout* L) {
   if (rc) return rc;
   L->ws_proj = c.take_bytes(L->ws_proj_bytes + 256);
   L->rt = L->kvr = nullptr;
+  L->kvr16 = nullptr;
   if (a->use_rte) {
     L->rt = c.take<float>((size_t)HGT_RTE_MAX_LEN * din);
-    L->kvr = c.take<float>(((size_t)a->n_pairs * HGT_RTE_MAX_LEN + 1) * 2 * d);
+    const size_t kvr_elems = ((size_t)a->n_pairs * HGT_RTE_MAX_LEN + 1) * 2 * d;
+    if (a->kv_bf16)
+      L->kvr16 = c.take<__nv_bfloat16>(kvr_elems);
+    else
+      L->kvr = c.take<float>(kvr_elems);
   }
   if ((rc = hgt_edge_workspace_bytes(a->n_split, d, a->n_heads, &L->ws_edge_bytes))) return rc;
   L->ws_edge = c.take_bytes(L->ws_edge_bytes);
@@ -106,6 +114,19 @@ extern "C" int hgt_conv_forward(const hgt_conv_args* a, void* workspace, size_t 
   HGT_REQUIRE(workspace_bytes >= L.total, "hgt_conv_forward: workspace too small (%zu < %zu)", workspace_bytes, L.total);
   const int64_t N = a->n_nodes;
   const int d = a->d_out, din = a->d_in, T = a->num_types, P = a->n_pairs;
+  const bool bf16 = a->kv_bf16 != 0;
+  HGT_REQUIRE(!bf16 || (a->n_q_groups >= 0 && a->n_q_groups <= a->n_proj_groups),
+              "hgt_conv_forward: n_q_groups=%d outside [0, n_proj_groups=%d]", a->n_q_groups, a->n_proj_groups);
+  if (bf16) {
+    // the bf16 layout: Q groups (one column block each) first, then [K'|V'] groups (an even number of blocks each).
+    // An fp32-layout table (Q and K'/V' blocks in one group, an odd count) would write bf16 rows at fp32 offsets.
+    for (int g = 0; g < a->n_proj_groups; ++g) {
+      const int nc = a->h_proj_groups[g].n_cblocks;
+      HGT_REQUIRE(g < a->n_q_groups ? nc == 1 : nc % 2 == 0,
+                  "hgt_conv_forward: kv_bf16 needs the Q groups (1 column block) first and then the [K'|V'] groups "
+                  "(an even number of blocks); group %d has %d blocks with n_q_groups=%d", g, nc, a->n_q_groups);
+    }
+  }
   if (N == 0) return 0;
 
   const float* x_sorted = a->x;
@@ -118,29 +139,72 @@ extern "C" int hgt_conv_forward(const hgt_conv_args* a, void* workspace, size_t 
                              a->cat_row0, a->q_row0, L.w_cat, L.b_cat, stream)))
     return rc;
   // trailing all-zero [K'|V'] row (edges that match no <s,t,r> triple)
-  HGT_CHECK_CUDA(cudaMemsetAsync(L.proj + a->kv_off + a->kv_rows * 2 * (int64_t)d, 0, sizeof(float) * 2 * d, st));
-  if (L.presplit_x)
-    rc = hgt_typed_linear_presplit(a->x_hi, a->x_lo, L.w_cat, L.b_cat, din, d, a->proj_groups, a->h_proj_groups,
-                                   a->n_proj_groups, a->proj_cblocks, L.proj, L.ws_proj, L.ws_proj_bytes + 256, stream);
+  if (bf16)
+    HGT_CHECK_CUDA(cudaMemsetAsync(reinterpret_cast<__nv_bfloat16*>(L.kv16) + a->kv_rows * 2 * (int64_t)d, 0,
+                                   sizeof(__nv_bfloat16) * 2 * d, st));
   else
-    rc = hgt_typed_linear(x_sorted, din, L.w_cat, L.b_cat, din, d, a->proj_groups, a->h_proj_groups, a->n_proj_groups,
+    HGT_CHECK_CUDA(cudaMemsetAsync(L.proj + a->kv_off + a->kv_rows * 2 * (int64_t)d, 0, sizeof(float) * 2 * d, st));
+  // fp32 groups (all of them, or the leading Q groups with bf16 tables), then the bf16 [K'|V'] groups
+  const int n_f32 = bf16 ? a->n_q_groups : a->n_proj_groups;
+  const int n_kv16 = a->n_proj_groups - n_f32;
+  const hgt_lin_group* kv_groups = a->proj_groups + n_f32;
+  const hgt_lin_group* h_kv_groups = a->h_proj_groups + n_f32;
+  bool presplit = L.presplit_x;
+  const void *x_hi = a->x_hi, *x_lo = a->x_lo;
+  if (bf16 && !presplit && L.fuse_split) {
+    // two tensor-core GEMMs over the same x: split it once, into the g_hi / g_lo buffers (the edge kernel fills them
+    // only after the projection); the presplit GEMM rounds exactly like the GEMM's own split
+    if ((rc = hgt_act_split(x_sorted, din, N, din, 0, nullptr, L.g_hi, L.g_lo, stream))) return rc;
+    presplit = true;
+    x_hi = L.g_hi;
+    x_lo = L.g_lo;
+  }
+  if (presplit)
+    rc = hgt_typed_linear_presplit(x_hi, x_lo, L.w_cat, L.b_cat, din, d, a->proj_groups, a->h_proj_groups,
+                                   n_f32, a->proj_cblocks, L.proj, L.ws_proj, L.ws_proj_bytes + 256, stream);
+  else
+    rc = hgt_typed_linear(x_sorted, din, L.w_cat, L.b_cat, din, d, a->proj_groups, a->h_proj_groups, n_f32,
                           a->proj_cblocks, L.proj, a->linear_impl, L.ws_proj, L.ws_proj_bytes + 256, stream);
   if (rc) return rc;
+  if (bf16 && n_kv16 > 0) {
+    if (presplit)
+      rc = hgt_typed_linear_presplit_bf16(x_hi, x_lo, L.w_cat, L.b_cat, din, d, kv_groups, h_kv_groups, n_kv16,
+                                          a->proj_cblocks, L.kv16, L.ws_proj, L.ws_proj_bytes + 256, stream);
+    else
+      rc = hgt_typed_linear_bf16(x_sorted, din, L.w_cat, L.b_cat, din, d, kv_groups, h_kv_groups, n_kv16,
+                                 a->proj_cblocks, L.kv16, a->linear_impl, L.ws_proj, L.ws_proj_bytes + 256, stream);
+    if (rc) return rc;
+  }
   if (a->use_rte) {
     if ((rc = hgt_typed_linear(a->emb_weight, din, a->emb_lin_w, a->emb_lin_b, din, din, a->rt_groups, a->h_rt_groups, 1,
                                a->rt_cblocks, L.rt, 1, nullptr, 0, stream)))
       return rc;
-    HGT_CHECK_CUDA(cudaMemsetAsync(L.kvr + (int64_t)P * HGT_RTE_MAX_LEN * 2 * d, 0, sizeof(float) * 2 * d, st));
-    if ((rc = hgt_typed_linear(L.rt, din, L.w_cat, nullptr, din, d, a->rte_groups, a->h_rte_groups, a->n_rte_groups,
-                               a->rte_cblocks, L.kvr, 1, nullptr, 0, stream)))
-      return rc;
+    const int64_t zero_row = (int64_t)P * HGT_RTE_MAX_LEN * 2 * d;
+    if (bf16) {
+      HGT_CHECK_CUDA(cudaMemsetAsync(reinterpret_cast<__nv_bfloat16*>(L.kvr16) + zero_row, 0,
+                                     sizeof(__nv_bfloat16) * 2 * d, st));
+      rc = hgt_typed_linear_bf16(L.rt, din, L.w_cat, nullptr, din, d, a->rte_groups, a->h_rte_groups, a->n_rte_groups,
+                                 a->rte_cblocks, L.kvr16, 1, nullptr, 0, stream);
+    } else {
+      HGT_CHECK_CUDA(cudaMemsetAsync(L.kvr + zero_row, 0, sizeof(float) * 2 * d, st));
+      rc = hgt_typed_linear(L.rt, din, L.w_cat, nullptr, din, d, a->rte_groups, a->h_rte_groups, a->n_rte_groups,
+                            a->rte_cblocks, L.kvr, 1, nullptr, 0, stream);
+    }
+    if (rc) return rc;
   }
-  if ((rc = hgt_edge_forward(L.proj + a->q_off, L.proj + a->kv_off, L.kvr, a->row_ptr, a->kv_row,
-                             a->use_rte ? a->rte_row : nullptr, a->csr_eid, a->tiles, a->n_tiles, a->n_split, a->hubs,
-                             a->n_hubs, N, a->n_edges, d, a->n_heads, 1, L.g_act, a->att, nullptr, L.g_hi, L.g_lo,
-                             L.ws_edge, L.ws_edge_bytes, a->edge_variant, a->d_tile_counts, a->type_row0, T,
-                             a->type_active, stream)))
-    return rc;
+  if (bf16)
+    rc = hgt_edge_forward_bf16kv(L.proj + a->q_off, L.kv16, L.kvr16, a->row_ptr, a->kv_row,
+                                 a->use_rte ? a->rte_row : nullptr, a->csr_eid, a->tiles, a->n_tiles, a->n_split,
+                                 a->hubs, a->n_hubs, N, a->n_edges, d, a->n_heads, 1, L.g_act, a->att, nullptr, L.g_hi,
+                                 L.g_lo, L.ws_edge, L.ws_edge_bytes, a->edge_variant, a->d_tile_counts, a->type_row0, T,
+                                 a->type_active, stream);
+  else
+    rc = hgt_edge_forward(L.proj + a->q_off, L.proj + a->kv_off, L.kvr, a->row_ptr, a->kv_row,
+                          a->use_rte ? a->rte_row : nullptr, a->csr_eid, a->tiles, a->n_tiles, a->n_split, a->hubs,
+                          a->n_hubs, N, a->n_edges, d, a->n_heads, 1, L.g_act, a->att, nullptr, L.g_hi, L.g_lo,
+                          L.ws_edge, L.ws_edge_bytes, a->edge_variant, a->d_tile_counts, a->type_row0, T,
+                          a->type_active, stream);
+  if (rc) return rc;
   if ((rc = hgt_concat_linears(a->wa, a->ba, T, d, d, L.wa_cat, L.ba_cat, stream))) return rc;
   if (L.fuse_split)
     rc = hgt_typed_linear_presplit(L.g_hi, L.g_lo, L.wa_cat, L.ba_cat, d, d, a->upd_groups, a->h_upd_groups,

@@ -8,6 +8,10 @@ int hgt_typed_linear_tc(const float* A, int64_t lda, const float* W, const float
                         int32_t cb_width, const hgt_lin_group* groups, const hgt_lin_group* h_groups,
                         int32_t n_groups, const hgt_lin_cblock* cblocks, float* out, void* workspace,
                         size_t workspace_bytes, cudaStream_t st);
+int hgt_typed_linear_tc(const float* A, int64_t lda, const float* W, const float* bias, int32_t K,
+                        int32_t cb_width, const hgt_lin_group* groups, const hgt_lin_group* h_groups,
+                        int32_t n_groups, const hgt_lin_cblock* cblocks, __nv_bfloat16* out, void* workspace,
+                        size_t workspace_bytes, cudaStream_t st);
 bool hgt_typed_linear_tc_supported(int64_t lda, int32_t K, int32_t cb_width);
 size_t hgt_typed_linear_tc_workspace(const hgt_lin_group* h_groups, int32_t n_groups, int32_t K, int32_t cb_width);
 
@@ -75,11 +79,12 @@ struct TilePrefix {
   int32_t n_tiles_n;   // n-tiles per column block
 };
 
+template <typename OutT>
 __global__ void __launch_bounds__(GEMM_THREADS)
 k_typed_linear_simt(const float* __restrict__ A, int64_t lda, const float* __restrict__ W,
                     const float* __restrict__ bias, int K, int cb_width,
                     const hgt_lin_group* __restrict__ groups, int n_groups,
-                    const hgt_lin_cblock* __restrict__ cblocks, float* __restrict__ out, TilePrefix tp) {
+                    const hgt_lin_cblock* __restrict__ cblocks, OutT* __restrict__ out, TilePrefix tp) {
   __shared__ __align__(16) float As[BK][LDA_S];
   __shared__ __align__(16) float Ws[BK][LDW_S];
   int tile = blockIdx.x;
@@ -150,7 +155,7 @@ k_typed_linear_simt(const float* __restrict__ A, int64_t lda, const float* __res
     for (int j = 0; j < 4; ++j)
       if (tn * 4 + j < cols_here) bj[j] = bias[w_row0 + tn * 4 + j];
   }
-  float* Og = out + cblk.out_off + m0 * cblk.ld + n0;
+  OutT* Og = out + cblk.out_off + m0 * cblk.ld + n0;
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     int r = tm * 8 + i;
@@ -158,9 +163,56 @@ k_typed_linear_simt(const float* __restrict__ A, int64_t lda, const float* __res
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       int c = tn * 4 + j;
-      if (c < cols_here) Og[(int64_t)r * cblk.ld + c] = acc[i][j] + bj[j];
+      if (c < cols_here) hgt_store_out(Og + (int64_t)r * cblk.ld + c, acc[i][j] + bj[j]);
     }
   }
+}
+
+// hgt_typed_linear for either output type: the fp32 and the bf16 entry points share dispatch, kernels and accumulation
+// order, so the bf16 result is the fp32 result rounded to nearest even.
+template <typename OutT>
+int typed_linear(const float* A, int64_t lda, const float* W, const float* bias, int32_t K, int32_t cb_width,
+                 const hgt_lin_group* groups, const hgt_lin_group* h_groups, int32_t n_groups,
+                 const hgt_lin_cblock* cblocks, OutT* out, int32_t impl, void* workspace, size_t workspace_bytes,
+                 cudaStream_t st) {
+  HGT_REQUIRE(n_groups >= 0, "hgt_typed_linear: n_groups=%d", n_groups);
+  HGT_REQUIRE(K > 0 && cb_width > 0, "hgt_typed_linear: K=%d cb_width=%d", K, cb_width);
+  if (n_groups == 0) return 0;
+  if (n_groups > kMaxGroups) {
+    // schemas with many <type, relation> pairs: the per-launch tile prefix holds kMaxGroups entries, so launch in
+    // chunks (same stream, same workspace: launches are ordered)
+    for (int g0 = 0; g0 < n_groups; g0 += kMaxGroups) {
+      const int n = n_groups - g0 < kMaxGroups ? n_groups - g0 : kMaxGroups;
+      int rc = typed_linear<OutT>(A, lda, W, bias, K, cb_width, groups + g0, h_groups + g0, n, cblocks, out, impl,
+                                  workspace, workspace_bytes, st);
+      if (rc) return rc;
+    }
+    return 0;
+  }
+  if (impl == 0) impl = hgt_typed_linear_tc_supported(lda, K, cb_width) ? 2 : 1;
+  if (impl == 2) {
+    HGT_REQUIRE(hgt_typed_linear_tc_supported(lda, K, cb_width),
+                "hgt_typed_linear: tensor-core kernel does not support lda=%lld K=%d cb_width=%d",
+                (long long)lda, K, cb_width);
+    return hgt_typed_linear_tc(A, lda, W, bias, K, cb_width, groups, h_groups, n_groups, cblocks, out, workspace,
+                               workspace_bytes, st);
+  }
+  HGT_REQUIRE(impl == 1, "hgt_typed_linear: unknown impl %d", impl);
+  TilePrefix tp;
+  tp.n_tiles_n = (cb_width + BN - 1) / BN;
+  int64_t total = 0;
+  for (int g = 0; g < n_groups; ++g) {
+    tp.first_tile[g] = (int32_t)total;
+    int64_t mt = (h_groups[g].m + BM - 1) / BM;
+    total += mt * h_groups[g].n_cblocks * tp.n_tiles_n;
+    HGT_REQUIRE(total < 2147483647ll, "hgt_typed_linear: too many tiles");
+  }
+  tp.first_tile[n_groups] = (int32_t)total;
+  if (total == 0) return 0;
+  k_typed_linear_simt<OutT><<<(unsigned)total, GEMM_THREADS, 0, st>>>(A, lda, W, bias, K, cb_width, groups, n_groups,
+                                                                      cblocks, out, tp);
+  HGT_LAUNCH_CHECK();
+  return 0;
 }
 
 }  // namespace
@@ -215,43 +267,21 @@ extern "C" int hgt_typed_linear(const float* A, int64_t lda, const float* W, con
                                 int32_t cb_width, const hgt_lin_group* groups, const hgt_lin_group* h_groups,
                                 int32_t n_groups, const hgt_lin_cblock* cblocks, float* out, int32_t impl,
                                 void* workspace, size_t workspace_bytes, void* stream_) {
-  cudaStream_t st = (cudaStream_t)stream_;
-  HGT_REQUIRE(n_groups >= 0, "hgt_typed_linear: n_groups=%d", n_groups);
-  HGT_REQUIRE(K > 0 && cb_width > 0, "hgt_typed_linear: K=%d cb_width=%d", K, cb_width);
-  if (n_groups == 0) return 0;
-  if (n_groups > kMaxGroups) {
-    // schemas with many <type, relation> pairs: the per-launch tile prefix holds kMaxGroups entries, so launch in
-    // chunks (same stream, same workspace: launches are ordered)
-    for (int g0 = 0; g0 < n_groups; g0 += kMaxGroups) {
-      const int n = n_groups - g0 < kMaxGroups ? n_groups - g0 : kMaxGroups;
-      int rc = hgt_typed_linear(A, lda, W, bias, K, cb_width, groups + g0, h_groups + g0, n, cblocks, out, impl,
-                                workspace, workspace_bytes, stream_);
-      if (rc) return rc;
-    }
-    return 0;
-  }
-  if (impl == 0) impl = hgt_typed_linear_tc_supported(lda, K, cb_width) ? 2 : 1;
-  if (impl == 2) {
-    HGT_REQUIRE(hgt_typed_linear_tc_supported(lda, K, cb_width),
-                "hgt_typed_linear: tensor-core kernel does not support lda=%lld K=%d cb_width=%d",
-                (long long)lda, K, cb_width);
-    return hgt_typed_linear_tc(A, lda, W, bias, K, cb_width, groups, h_groups, n_groups, cblocks, out, workspace,
-                               workspace_bytes, st);
-  }
-  HGT_REQUIRE(impl == 1, "hgt_typed_linear: unknown impl %d", impl);
-  TilePrefix tp;
-  tp.n_tiles_n = (cb_width + BN - 1) / BN;
-  int64_t total = 0;
-  for (int g = 0; g < n_groups; ++g) {
-    tp.first_tile[g] = (int32_t)total;
-    int64_t mt = (h_groups[g].m + BM - 1) / BM;
-    total += mt * h_groups[g].n_cblocks * tp.n_tiles_n;
-    HGT_REQUIRE(total < 2147483647ll, "hgt_typed_linear: too many tiles");
-  }
-  tp.first_tile[n_groups] = (int32_t)total;
-  if (total == 0) return 0;
-  k_typed_linear_simt<<<(unsigned)total, GEMM_THREADS, 0, st>>>(A, lda, W, bias, K, cb_width, groups, n_groups,
-                                                                cblocks, out, tp);
-  HGT_LAUNCH_CHECK();
-  return 0;
+  return typed_linear<float>(A, lda, W, bias, K, cb_width, groups, h_groups, n_groups, cblocks, out, impl, workspace,
+                             workspace_bytes, (cudaStream_t)stream_);
+}
+
+extern "C" int hgt_typed_linear_bf16_workspace_bytes(const hgt_lin_group* h_groups, int32_t n_groups, int32_t K,
+                                                     int32_t cb_width, int32_t impl, size_t* out_bytes) {
+  // every path stores bf16 straight from its epilogue: the same workspace as the fp32 output
+  return hgt_typed_linear_workspace_bytes(h_groups, n_groups, K, cb_width, impl, out_bytes);
+}
+
+extern "C" int hgt_typed_linear_bf16(const float* A, int64_t lda, const float* W, const float* bias, int32_t K,
+                                     int32_t cb_width, const hgt_lin_group* groups, const hgt_lin_group* h_groups,
+                                     int32_t n_groups, const hgt_lin_cblock* cblocks, void* out, int32_t impl,
+                                     void* workspace, size_t workspace_bytes, void* stream_) {
+  return typed_linear<__nv_bfloat16>(A, lda, W, bias, K, cb_width, groups, h_groups, n_groups, cblocks,
+                                     reinterpret_cast<__nv_bfloat16*>(out), impl, workspace, workspace_bytes,
+                                     (cudaStream_t)stream_);
 }

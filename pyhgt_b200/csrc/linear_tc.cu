@@ -15,6 +15,8 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -31,18 +33,25 @@ constexpr int TC_BK = 64;              // 64 bf16 = 128 bytes = one SWIZZLE_128B
 constexpr int TC_THREADS = 192;
 constexpr int UMMA_K = 16;
 
+// Two fp32 values rounded to nearest even as a packed bf16 pair (first value at the lower address).
+__device__ __forceinline__ uint32_t bf16x2_bits(float a, float b) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<const uint32_t*>(&h);
+}
+
 struct TcTilePrefix {
   int32_t first_tile[kMaxGroups + 1];
   int32_t n_tiles_n;
 };
 
 // ---- the GEMM -------------------------------------------------------------------------------------
+template <typename OutT>
 __global__ void __launch_bounds__(TC_THREADS, 2)
 k_typed_linear_tc(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                   const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
                   const float* __restrict__ bias, int Kp, int cb_width, int BN, int stages, int tmem_cols,
                   const hgt_lin_group* __restrict__ groups, int n_groups,
-                  const hgt_lin_cblock* __restrict__ cblocks, float* __restrict__ out, TcTilePrefix tp) {
+                  const hgt_lin_cblock* __restrict__ cblocks, OutT* __restrict__ out, TcTilePrefix tp) {
   extern __shared__ unsigned char smem_dyn[];
   // carve: [stages][A 16 KB | B BN*128 B] (1024-aligned), then barriers, tmem pointer, bias tile
   unsigned char* smem = smem_dyn + ((1024u - (s_u32(smem_dyn) & 1023u)) & 1023u);   // keeps the shared address space
@@ -149,21 +158,32 @@ k_typed_linear_tc(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
     const int row = lg * 32 + lane;
     mbar_wait(s_u32(tmem_full_bar), 0);
     tc_fence_after();
-    float* orow = out + cblk.out_off + (m0 + row) * cblk.ld + n0;
+    OutT* orow = out + cblk.out_off + (m0 + row) * cblk.ld + n0;
     const bool row_ok = row < rows_here;
     for (int c = 0; c < BN; c += 16) {
       uint32_t r[16];
       tmem_ld16(tmem_base + ((uint32_t)(lg * 32) << 16) + (uint32_t)c, r);
       tmem_ld_wait();
       if (row_ok) {
+        if constexpr (std::is_same<OutT, float>::value) {
 #pragma unroll
-        for (int j = 0; j < 16; j += 4) {
-          float4 v;
-          v.x = __uint_as_float(r[j + 0]) + s_bias[c + j + 0];
-          v.y = __uint_as_float(r[j + 1]) + s_bias[c + j + 1];
-          v.z = __uint_as_float(r[j + 2]) + s_bias[c + j + 2];
-          v.w = __uint_as_float(r[j + 3]) + s_bias[c + j + 3];
-          *reinterpret_cast<float4*>(orow + c + j) = v;
+          for (int j = 0; j < 16; j += 4) {
+            float4 v;
+            v.x = __uint_as_float(r[j + 0]) + s_bias[c + j + 0];
+            v.y = __uint_as_float(r[j + 1]) + s_bias[c + j + 1];
+            v.z = __uint_as_float(r[j + 2]) + s_bias[c + j + 2];
+            v.w = __uint_as_float(r[j + 3]) + s_bias[c + j + 3];
+            *reinterpret_cast<float4*>(orow + c + j) = v;
+          }
+        } else {
+          // bf16 row: 16 values = two 16-byte stores
+          uint32_t w[8];
+#pragma unroll
+          for (int j = 0; j < 8; ++j)
+            w[j] = bf16x2_bits(__uint_as_float(r[2 * j]) + s_bias[c + 2 * j],
+                               __uint_as_float(r[2 * j + 1]) + s_bias[c + 2 * j + 1]);
+          *reinterpret_cast<uint4*>(orow + c) = make_uint4(w[0], w[1], w[2], w[3]);
+          *reinterpret_cast<uint4*>(orow + c + 8) = make_uint4(w[4], w[5], w[6], w[7]);
         }
       }
     }
@@ -203,8 +223,9 @@ constexpr int TC2_STAGE_BYTES = TC2_EPI_WARPS * 32 * TC2_STG_LD * 4;
 // has bank conflicts.  Measured at C2 together with the .cta-scope pair barriers: projection 3.90 -> 3.81 ms against the
 // round-1 drain; a drain straight from registers without the transpose ran at the same speed
 // (profiles/r02_gemm_epilogue_ab.md); see DESIGN.md section 9 for what was ruled out as the limiter.
+template <typename OutT>
 __device__ __forceinline__ void tc_epi_chunk(const uint32_t (&r)[16], int c0, float* stg, const float* s_bias,
-                                             float* out_tile, int64_t ld, int64_t rows_left, int lane) {
+                                             OutT* out_tile, int64_t ld, int64_t rows_left, int lane) {
   // staging rows of 64 bytes, the 16-byte piece j of row r kept at position j ^ ((r >> 1) & 3): the row-per-lane writes
   // and the 4-lanes-per-row reads both touch every bank once per quarter warp (no conflicts, 4 wavefronts per access)
   const int sub = lane & 3, rsel = lane >> 2;
@@ -214,25 +235,55 @@ __device__ __forceinline__ void tc_epi_chunk(const uint32_t (&r)[16], int c0, fl
     *reinterpret_cast<uint4*>(stg + lane * 16 + ((j ^ wsw) << 2)) =
         make_uint4(r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
   __syncwarp();
-  const float4 b = *reinterpret_cast<const float4*>(s_bias + c0 + sub * 4);
-  const int rsw = (sub ^ ((rsel >> 1) & 3)) << 2;                     // (8k + rsel) >> 1 & 3 == rsel >> 1 & 3
-  float4 v[4];
+  if constexpr (std::is_same<OutT, float>::value) {
+    const float4 b = *reinterpret_cast<const float4*>(s_bias + c0 + sub * 4);
+    const int rsw = (sub ^ ((rsel >> 1) & 3)) << 2;                   // (8k + rsel) >> 1 & 3 == rsel >> 1 & 3
+    float4 v[4];
 #pragma unroll
-  for (int k = 0; k < 4; ++k) v[k] = *reinterpret_cast<const float4*>(stg + (8 * k + rsel) * 16 + rsw);
-  __syncwarp();
+    for (int k = 0; k < 4; ++k) v[k] = *reinterpret_cast<const float4*>(stg + (8 * k + rsel) * 16 + rsw);
+    __syncwarp();
 #pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const int rr = 8 * k + rsel;
-    if (rr < rows_left) {
-      float4 w = v[k];
-      w.x += b.x; w.y += b.y; w.z += b.z; w.w += b.w;
-      *reinterpret_cast<float4*>(out_tile + (int64_t)rr * ld + c0 + sub * 4) = w;
+    for (int k = 0; k < 4; ++k) {
+      const int rr = 8 * k + rsel;
+      if (rr < rows_left) {
+        float4 w = v[k];
+        w.x += b.x; w.y += b.y; w.z += b.z; w.w += b.w;
+        *reinterpret_cast<float4*>(out_tile + (int64_t)rr * ld + c0 + sub * 4) = w;
+      }
+    }
+  } else {
+    // bf16 rows: the 16 columns of a row are 32 bytes, two lanes of 8 values (one 16-byte store each), 16 rows per
+    // pass.  Lane (row rh, half h) reads pieces 2h and 2h+1 of its staging row; the swizzle keeps each quarter warp on
+    // distinct banks.
+    const int h = lane & 1, rh = lane >> 1;
+    const int sw = (rh >> 1) & 3;                                      // (16k + rh) >> 1 & 3 == rh >> 1 & 3
+    const float4 b0 = *reinterpret_cast<const float4*>(s_bias + c0 + h * 8);
+    const float4 b1 = *reinterpret_cast<const float4*>(s_bias + c0 + h * 8 + 4);
+    float4 v[2][2];
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const float* srow = stg + (16 * k + rh) * 16;
+      v[k][0] = *reinterpret_cast<const float4*>(srow + (((2 * h) ^ sw) << 2));
+      v[k][1] = *reinterpret_cast<const float4*>(srow + (((2 * h + 1) ^ sw) << 2));
+    }
+    __syncwarp();
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int rr = 16 * k + rh;
+      if (rr < rows_left) {
+        const uint4 w = make_uint4(bf16x2_bits(v[k][0].x + b0.x, v[k][0].y + b0.y),
+                                   bf16x2_bits(v[k][0].z + b0.z, v[k][0].w + b0.w),
+                                   bf16x2_bits(v[k][1].x + b1.x, v[k][1].y + b1.y),
+                                   bf16x2_bits(v[k][1].z + b1.z, v[k][1].w + b1.w));
+        *reinterpret_cast<uint4*>(out_tile + (int64_t)rr * ld + c0 + h * 8) = w;
+      }
     }
   }
 }
 
+template <typename OutT>
 __device__ __forceinline__ void tc_epilogue_tile_pf(uint32_t t_row, int n_cols, int chunk0, float* stg,
-                                                    const float* s_bias, float* out_tile, int64_t ld,
+                                                    const float* s_bias, OutT* out_tile, int64_t ld,
                                                     int64_t rows_left, int lane) {
   uint32_t ra[16], rb[16];
   int c0 = 16 * chunk0;
@@ -255,12 +306,13 @@ struct Tc2Sched {
   int32_t n_tiles_n;
 };
 
+template <typename OutT>
 __global__ void __launch_bounds__(TC2_THREADS, 1)
 k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                    const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
                    const float* __restrict__ bias, int Kp, int cb_width, int BN, int stages, int tmem_cols,
                    const hgt_lin_group* __restrict__ groups, int n_groups,
-                   const hgt_lin_cblock* __restrict__ cblocks, float* __restrict__ out, Tc2Sched sc) {
+                   const hgt_lin_cblock* __restrict__ cblocks, OutT* __restrict__ out, Tc2Sched sc) {
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = smem_dyn + ((1024u - (s_u32(smem_dyn) & 1023u)) & 1023u);   // keeps the shared address space
   const int k_blocks = (Kp + TC_BK - 1) / TC_BK;
@@ -452,12 +504,13 @@ k_typed_linear_tc2(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
 // peer-bit-masked address, the leader's producer posts expect_tx for both); a_empty / w_empty / t_full are
 // per-CTA and signalled by multicast tcgen05.commit; t_empty lives in the leader and collects the 8 epilogue
 // warps of the pair.
+template <typename OutT>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC2_THREADS, 1)
 k_typed_linear_tc3(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                    const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
                    const float* __restrict__ bias, int Kp, int cb_width, int stages,
                    const hgt_lin_group* __restrict__ groups, int n_groups,
-                   const hgt_lin_cblock* __restrict__ cblocks, float* __restrict__ out, Tc2Sched sc) {
+                   const hgt_lin_cblock* __restrict__ cblocks, OutT* __restrict__ out, Tc2Sched sc) {
   constexpr int BNH = 128;              // W columns resident per CTA
   constexpr int BNP = 256;              // columns per pair step
   constexpr int BMP = 256;              // rows per pair step
@@ -697,14 +750,22 @@ size_t hgt_typed_linear_tc_workspace(const hgt_lin_group* h_groups, int32_t n_gr
   return 4 * 256 + 2 * hgt_align_up((size_t)a_rows * Kp * 2, 256) + 2 * hgt_align_up((size_t)w_rows * Kp * 2, 256);
 }
 
+template <typename OutT>
 static int tc_run(const float* A, int64_t lda, const __nv_bfloat16* a_hi_in, const __nv_bfloat16* a_lo_in,
                   const float* W, const float* bias, int32_t K, int32_t cb_width, const hgt_lin_group* groups,
-                  const hgt_lin_group* h_groups, int32_t n_groups, const hgt_lin_cblock* cblocks, float* out,
+                  const hgt_lin_group* h_groups, int32_t n_groups, const hgt_lin_cblock* cblocks, OutT* out,
                   void* workspace, size_t workspace_bytes, cudaStream_t st);
 
 int hgt_typed_linear_tc(const float* A, int64_t lda, const float* W, const float* bias, int32_t K, int32_t cb_width,
                         const hgt_lin_group* groups, const hgt_lin_group* h_groups, int32_t n_groups,
                         const hgt_lin_cblock* cblocks, float* out, void* workspace, size_t workspace_bytes,
+                        cudaStream_t st) {
+  return tc_run(A, lda, nullptr, nullptr, W, bias, K, cb_width, groups, h_groups, n_groups, cblocks, out, workspace,
+                workspace_bytes, st);
+}
+int hgt_typed_linear_tc(const float* A, int64_t lda, const float* W, const float* bias, int32_t K, int32_t cb_width,
+                        const hgt_lin_group* groups, const hgt_lin_group* h_groups, int32_t n_groups,
+                        const hgt_lin_cblock* cblocks, __nv_bfloat16* out, void* workspace, size_t workspace_bytes,
                         cudaStream_t st) {
   return tc_run(A, lda, nullptr, nullptr, W, bias, K, cb_width, groups, h_groups, n_groups, cblocks, out, workspace,
                 workspace_bytes, st);
@@ -717,11 +778,10 @@ extern "C" int hgt_typed_linear_presplit_workspace_bytes(const hgt_lin_group* h_
   return 0;
 }
 
-extern "C" int hgt_typed_linear_presplit(const void* a_hi, const void* a_lo, const float* W, const float* bias,
-                                         int32_t K, int32_t cb_width, const hgt_lin_group* groups,
-                                         const hgt_lin_group* h_groups, int32_t n_groups,
-                                         const hgt_lin_cblock* cblocks, float* out, void* workspace,
-                                         size_t workspace_bytes, void* stream_) {
+template <typename OutT>
+static int presplit(const void* a_hi, const void* a_lo, const float* W, const float* bias, int32_t K, int32_t cb_width,
+                    const hgt_lin_group* groups, const hgt_lin_group* h_groups, int32_t n_groups,
+                    const hgt_lin_cblock* cblocks, OutT* out, void* workspace, size_t workspace_bytes, cudaStream_t st) {
   HGT_REQUIRE(a_hi && a_lo, "hgt_typed_linear_presplit: NULL operand");
   HGT_REQUIRE(K % 8 == 0 && hgt_typed_linear_tc_supported(K, K, cb_width),
               "hgt_typed_linear_presplit: unsupported shape K=%d cb_width=%d", K, cb_width);
@@ -729,20 +789,43 @@ extern "C" int hgt_typed_linear_presplit(const void* a_hi, const void* a_lo, con
   if (n_groups > kMaxGroups) {                               // see hgt_typed_linear: chunked launches
     for (int g0 = 0; g0 < n_groups; g0 += kMaxGroups) {
       const int n = n_groups - g0 < kMaxGroups ? n_groups - g0 : kMaxGroups;
-      int rc = hgt_typed_linear_presplit(a_hi, a_lo, W, bias, K, cb_width, groups + g0, h_groups + g0, n, cblocks, out,
-                                         workspace, workspace_bytes, stream_);
+      int rc = presplit(a_hi, a_lo, W, bias, K, cb_width, groups + g0, h_groups + g0, n, cblocks, out, workspace,
+                        workspace_bytes, st);
       if (rc) return rc;
     }
     return 0;
   }
   return tc_run(nullptr, 0, reinterpret_cast<const __nv_bfloat16*>(a_hi), reinterpret_cast<const __nv_bfloat16*>(a_lo),
-                W, bias, K, cb_width, groups, h_groups, n_groups, cblocks, out, workspace, workspace_bytes,
-                (cudaStream_t)stream_);
+                W, bias, K, cb_width, groups, h_groups, n_groups, cblocks, out, workspace, workspace_bytes, st);
 }
 
+extern "C" int hgt_typed_linear_presplit(const void* a_hi, const void* a_lo, const float* W, const float* bias,
+                                         int32_t K, int32_t cb_width, const hgt_lin_group* groups,
+                                         const hgt_lin_group* h_groups, int32_t n_groups,
+                                         const hgt_lin_cblock* cblocks, float* out, void* workspace,
+                                         size_t workspace_bytes, void* stream_) {
+  return presplit(a_hi, a_lo, W, bias, K, cb_width, groups, h_groups, n_groups, cblocks, out, workspace,
+                  workspace_bytes, (cudaStream_t)stream_);
+}
+
+extern "C" int hgt_typed_linear_presplit_bf16_workspace_bytes(const hgt_lin_group* h_groups, int32_t n_groups,
+                                                              int32_t K, int32_t cb_width, size_t* out_bytes) {
+  return hgt_typed_linear_presplit_workspace_bytes(h_groups, n_groups, K, cb_width, out_bytes);
+}
+
+extern "C" int hgt_typed_linear_presplit_bf16(const void* a_hi, const void* a_lo, const float* W, const float* bias,
+                                              int32_t K, int32_t cb_width, const hgt_lin_group* groups,
+                                              const hgt_lin_group* h_groups, int32_t n_groups,
+                                              const hgt_lin_cblock* cblocks, void* out, void* workspace,
+                                              size_t workspace_bytes, void* stream_) {
+  return presplit(a_hi, a_lo, W, bias, K, cb_width, groups, h_groups, n_groups, cblocks,
+                  reinterpret_cast<__nv_bfloat16*>(out), workspace, workspace_bytes, (cudaStream_t)stream_);
+}
+
+template <typename OutT>
 static int tc_run(const float* A, int64_t lda, const __nv_bfloat16* a_hi_in, const __nv_bfloat16* a_lo_in,
                   const float* W, const float* bias, int32_t K, int32_t cb_width, const hgt_lin_group* groups,
-                  const hgt_lin_group* h_groups, int32_t n_groups, const hgt_lin_cblock* cblocks, float* out,
+                  const hgt_lin_group* h_groups, int32_t n_groups, const hgt_lin_cblock* cblocks, OutT* out,
                   void* workspace, size_t workspace_bytes, cudaStream_t st) {
   const int BN = pick_bn(cb_width);
   HGT_REQUIRE(BN > 0, "hgt_typed_linear(tc): cb_width=%d has no multiple-of-16 tile", cb_width);
@@ -787,8 +870,9 @@ static int tc_run(const float* A, int64_t lda, const __nv_bfloat16* a_hi_in, con
                     TC2_STAGE_BYTES;
       int pairs = hgt_sm_count() / 2;
       if (pairs > units) pairs = (int)units;
-      HGT_CHECK_CUDA(cudaFuncSetAttribute(k_typed_linear_tc3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k_typed_linear_tc3<<<2 * pairs, TC2_THREADS, smem, st>>>(m_a_hi, m_a_lo, m_w_hi, m_w_lo, bias, Kp, cb_width,
+      HGT_CHECK_CUDA(cudaFuncSetAttribute(k_typed_linear_tc3<OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)smem));
+      k_typed_linear_tc3<OutT><<<2 * pairs, TC2_THREADS, smem, st>>>(m_a_hi, m_a_lo, m_w_hi, m_w_lo, bias, Kp, cb_width,
                                                                stages, groups, n_groups, cblocks, out, sc);
       HGT_LAUNCH_CHECK();
       return 0;
@@ -812,10 +896,11 @@ static int tc_run(const float* A, int64_t lda, const __nv_bfloat16* a_hi_in, con
     while (tmem_cols < 2 * bn) tmem_cols <<= 1;
     size_t smem = 1024 + w_region + (size_t)stages * a_stage + (2 * stages + 6) * 8 + 16 + (size_t)bn * 4 + 64 +
                   TC2_STAGE_BYTES;
-    HGT_CHECK_CUDA(cudaFuncSetAttribute(k_typed_linear_tc2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    HGT_CHECK_CUDA(cudaFuncSetAttribute(k_typed_linear_tc2<OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)smem));
     int grid = hgt_sm_count();
     if (grid > units) grid = (int)units;
-    k_typed_linear_tc2<<<grid, TC2_THREADS, smem, st>>>(m_a_hi, m_a_lo, m_w_hi, m_w_lo, bias, Kp, cb_width, bn,
+    k_typed_linear_tc2<OutT><<<grid, TC2_THREADS, smem, st>>>(m_a_hi, m_a_lo, m_w_hi, m_w_lo, bias, Kp, cb_width, bn,
                                                         stages, tmem_cols, groups, n_groups, cblocks, out, sc);
     HGT_LAUNCH_CHECK();
     return 0;
@@ -843,8 +928,8 @@ static int tc_run(const float* A, int64_t lda, const __nv_bfloat16* a_hi_in, con
   int tmem_cols = 32;
   while (tmem_cols < BN) tmem_cols <<= 1;
   size_t smem = 1024 + (size_t)stages * stage_bytes + (2 * stages + 1) * 8 + 16 + (size_t)BN * 4 + 64;
-  HGT_CHECK_CUDA(cudaFuncSetAttribute(k_typed_linear_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_typed_linear_tc<<<(unsigned)total, TC_THREADS, smem, st>>>(m_a_hi, m_a_lo, m_w_hi, m_w_lo, bias, Kp, cb_width,
+  HGT_CHECK_CUDA(cudaFuncSetAttribute(k_typed_linear_tc<OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_typed_linear_tc<OutT><<<(unsigned)total, TC_THREADS, smem, st>>>(m_a_hi, m_a_lo, m_w_hi, m_w_lo, bias, Kp, cb_width,
                                                                BN, stages, tmem_cols, groups, n_groups, cblocks, out,
                                                                tp);
   HGT_LAUNCH_CHECK();

@@ -367,6 +367,9 @@ class LayerTables:
     kv_off: int
     proj_elems: int
     type_active_dev: torch.Tensor = None
+    kv_bf16: bool = False         # bf16 [K'|V'] table: proj_groups = n_q_groups Q groups, then the K'/V' groups, whose
+    n_q_groups: int = 0           # cblocks address a separate bf16 table of kv_elems elements (the fp32 projection
+    kv_elems: int = 0             # buffer of proj_elems floats then holds Q only)
 
 
 class GroupTable(tuple):
@@ -387,13 +390,17 @@ def _pack_groups(groups, cblocks, dev):
     return tab
 
 
-def layer_tables(plan, d_in, d_out, active=None, kv_runs=None):
+def layer_tables(plan, d_in, d_out, active=None, kv_runs=None, kv_bf16=False):
     """`active[t]` (sharded runs): only the first active[t] nodes of type t (in rank order) are destinations
     that need Q / a_linear / update; the rest of the type (halo sources) only get K'/V' rows.
     `kv_runs` (sharded runs): (((type, relation), ((row0, row1), ...)), ...) — type-relative row ranges whose K'/V' rows
     some local edge reads; the projection then covers those ranges only (the other rows of the table are never
-    gathered and stay unwritten)."""
-    key = (d_in, d_out, None if active is None else tuple(active), kv_runs)
+    gathered and stay unwritten).
+    `kv_bf16` (inference with bf16 K'/V' tables, HGTConv.kv_dtype): the projection table lists one Q group per type
+    (fp32 output) and then one K'/V' group per type with pairs, whose column blocks address a separate bf16 table."""
+    if kv_bf16 and (active is not None or kv_runs is not None):
+        raise ValueError("bf16 K'/V' tables are not supported on the sharded path")
+    key = (d_in, d_out, None if active is None else tuple(active), kv_runs, bool(kv_bf16))
     hit = plan._layer_tables.get(key)
     if hit is not None:
         return hit
@@ -433,6 +440,26 @@ def layer_tables(plan, d_in, d_out, active=None, kv_runs=None):
                 cblocks.append((base, 2 * d_out))
                 cblocks.append((base + d_out, 2 * d_out))
             groups.append((plan.type_row0[t] + a, m - a, q_row0[t] + d_out, 2 * len(pairs_of_type[t]), first, 1))
+    n_q_groups = kv_elems = 0
+    if kv_bf16:
+        # Q groups (fp32, into a projection buffer of N * d_out floats), then the K'/V' groups (bf16 table from 0)
+        groups, cblocks = [], []
+        for t in range(T):
+            if plan.type_count[t]:
+                groups.append((plan.type_row0[t], plan.type_count[t], q_row0[t], 1, len(cblocks), 1))
+                cblocks.append((q_off + plan.type_row0[t] * d_out, d_out))
+        n_q_groups = len(groups)
+        for t in range(T):
+            if plan.type_count[t] and pairs_of_type[t]:
+                first = len(cblocks)
+                for p in pairs_of_type[t]:
+                    base = plan.pair_row0[p] * 2 * d_out
+                    cblocks.append((base, 2 * d_out))
+                    cblocks.append((base + d_out, 2 * d_out))
+                groups.append((plan.type_row0[t], plan.type_count[t], q_row0[t] + d_out, 2 * len(pairs_of_type[t]),
+                               first, 1))
+        kv_off, proj_elems = 0, N * d_out
+        kv_elems = (plan.kv_rows + 1) * 2 * d_out
     if kv_runs is not None:
         # per-pair compaction: a Q group over the active prefix, and one K'/V' group per needed row range of every pair
         runs = dict(kv_runs)
@@ -486,6 +513,7 @@ def layer_tables(plan, d_in, d_out, active=None, kv_runs=None):
     lt = LayerTables(cat_rows=rows, q_row0=q_row0, cat_row0=cat_row0, q_row0_dev=small[:T],
                      cat_row0_dev=small[T:T + max(P, 1)],
                      type_active_dev=None if active is None else small[T + max(P, 1):], proj_groups=proj, rte_groups=rte, upd_groups=upd, rt_group=rt_group, q_off=q_off,
-                     kv_off=kv_off, proj_elems=proj_elems)
+                     kv_off=kv_off, proj_elems=proj_elems, kv_bf16=bool(kv_bf16), n_q_groups=n_q_groups,
+                     kv_elems=kv_elems)
     plan._layer_tables[key] = lt
     return lt

@@ -16,6 +16,12 @@ import torch
 import torch.distributed as dist
 
 
+def _require_fp32_kv(conv):
+    """The sharded layer has fp32 K'/V' tables only (the bf16 mode of HGTConv.kv_dtype is single-GPU inference)."""
+    if getattr(conv, "kv_dtype", torch.float32) != torch.float32:
+        raise ValueError("the sharded path supports kv_dtype=torch.float32 only, got %r" % (conv.kv_dtype,))
+
+
 def partition_owner(node_type, edge_index, num_types, world):
     """owner[n] in [0, world): contiguous cost-balanced blocks inside every node type (deterministic; runs on the device
     of its inputs)."""
@@ -396,6 +402,7 @@ class ShardedGraph:
         """Differentiable sharded layer (BASELINE config 4): halo exchange with a reverse all-to-all in backward, the
         layer's autograd path on the local graph, owned rows out.  Parameter gradients are PARTIAL per rank (each rank
         sees only its destinations): sum them with `allreduce_grads` (or wrap the model in DistributedDataParallel)."""
+        _require_fp32_kv(conv)
         x_local = _HaloExchange.apply(x_own, self)
         tm = self.edge_time if conv.use_RTE else None
         if x_local.is_cuda and hasattr(conv, "q_linears") and type(conv).__name__ == "HGTConv":
@@ -419,6 +426,7 @@ class ShardedGraph:
         `graph` = (node_type, edge_index, edge_type, edge_time) device tensors holding this rank's LOCAL graph, for
         callers that stream the shard from the host every step (the plan is rebuilt when they change)."""
         from .conv import HGTConv
+        _require_fp32_kv(conv)
         with HGTConv._stage("halo_exchange"):
             x_local, x_split = self.exchange(x_own, split=x_own.is_cuda and conv.linear_impl in (0, 2))
         l_nt, l_ei, l_et, l_tm = (self.node_type, self.edge_index, self.edge_type, self.edge_time) if graph is None else graph
